@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: audio-seconds synthesised per second (22.05 kHz, mel + vocoder) on N x B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch: MatchaTTS.synthesise(x, x_lengths, n_timesteps=10,
 temperature=0.667, spks=emoji ids, length_scale=0.8) followed by vocoder(mel).clamp(-1, 1), on BASELINE.json
@@ -22,6 +22,10 @@ PyTorch path (the unmodified files staged under baseline/_ref, else the oracle p
 bounded sample.  Further blocks: `padded_vocoder` (the reference's literal work list, with its own e2e), `denoiser`,
 `config3` (BASELINE configs[2]: 1024 mixed-length utterances sharded over the N ranks through synthesise_corpus, strong
 scaling, wall clock incl. D2H + crop, cold = never-seen shapes and warm) and `config5` (vocoder only, 60-s segments).
+
+`--dump-outputs DIR` writes what the last timed step returned to its caller (the synthesise dict of the reference and the
+waveform) as DIR/<name>.npy.  The prior noise is drawn from a generator seeded before the timed region, so with the same
+arguments two runs, or two builds, compute the same step and can be compared output for output.
 """
 from __future__ import annotations
 
@@ -43,6 +47,8 @@ SR, HOP = 22050, 256
 N_TIMESTEPS, TEMPERATURE, LENGTH_SCALE = 10, 0.667, 0.8      # feel_me.py:71-77 (the operating point of every app)
 BATCH, P_LO, P_HI = 32, 60, 90                                # SURVEY.md 8d config 2: Tx = 2P+1 in [121, 181]
 CPU_SAMPLE = 8                                                # utterances the `cpu_baseline` leg / reference warm-up synthesise (~4.5 s per pass)
+DUMP_BYTES = 64 * 10**6                                       # cap on what --dump-outputs writes in all
+DUMPED = ("encoder_outputs", "decoder_outputs", "attn", "mel", "mel_lengths")      # the dict the reference's synthesise returns
 
 
 def load_peaks():
@@ -129,6 +135,25 @@ def measured_traffic(kernel_class: str):
 
 def audio_seconds(mel_lengths) -> float:
     return float(mel_lengths.sum()) * HOP / SR
+
+
+def dump_outputs(out_dir, tensors, cap=DUMP_BYTES):
+    """Write each tensor as out_dir/<name>.npy: floating point as float32, integers as float64 (exact).  Should the whole
+    exceed `cap` bytes, every array above 1 MiB keeps the same fraction of its elements, flattened, at ascending positions
+    drawn with a fixed seed (identical positions from run to run as long as the shapes agree); its original shape is then
+    written beside it as <name>.shape.npy."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    arrs = {k: (t.detach().float() if t.is_floating_point() else t.detach().double()).cpu().numpy() for k, t in tensors.items()}
+    big = [k for k, a in arrs.items() if a.nbytes > 2**20]
+    need = sum(arrs[k].nbytes for k in big)
+    room = cap - 8192 * len(arrs) - sum(a.nbytes for k, a in arrs.items() if k not in big)      # (8192: .npy headers, shapes)
+    for name, a in arrs.items():
+        if name in big and need > room:
+            np.save(os.path.join(out_dir, name + ".shape.npy"), np.array(a.shape, dtype=np.float64))
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, a.size * room // need, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 class CpuArm:
@@ -244,7 +269,14 @@ def main():
                          "own length: identical waveform on [: length*256], zero beyond -- what cli.py:307-311 crops away)")
     ap.add_argument("--profile-one-step", action="store_true",
                     help="after warm-up, bracket ONE step with cudaProfilerStart/Stop and exit (for `ncu --profile-from-start off`)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (%s, waveform) as DIR/<name>.npy, float32 "
+                         "(float64 for the lengths), at most 64 MB in all" % ", ".join(DUMPED))
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.profile_one_step):
+        ap.error("--dump-outputs writes the outputs of the timed CUDA path: not with --impl reference or --profile-one-step")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -313,6 +345,7 @@ def main():
         return v(out["mel"], lengths=out["mel_lengths"] if ragged[0] else None).clamp(-1, 1)
 
     lane_done = [None] * n_lanes
+    last_step = [False, None]                                    # [recording, (out, wav) of the last step recorded]
 
     def step_resident():
         lane, m, v, st = next_lane()
@@ -323,6 +356,8 @@ def main():
             wav = vocode(v, out)
             lane_done[lane] = torch.cuda.Event()
             lane_done[lane].record()
+        if last_step[0]:
+            last_step[1] = (out, wav)
         return out, wav
 
     host = [dict(wav=None, len=torch.empty(BATCH, dtype=torch.int64).pin_memory(), done=None) for _ in range(n_lanes)]
@@ -399,6 +434,9 @@ def main():
         return
 
     # ---------------- timed region: K steps, inputs resident in HBM
+    # every step draws its prior noise from the device's generator; the warm-up above runs until the step time settles, so
+    # the generator is seeded here, a fixed number of steps before the last timed one
+    torch.cuda.manual_seed(0)
     sampler = ClockSampler(local_rank)
     sampler.start()
     def count_launches(reset=False):
@@ -407,9 +445,15 @@ def main():
     if n_lanes > 1:
         timed(step_resident, 2 * n_lanes)                        # untimed: brings the lanes into their steady overlap
     count_launches(reset=True)
+    last_step[0] = bool(args.dump_outputs) and rank == 0
     ms = timed(step_resident, args.steps)
     launches = count_launches()
     clocks = sampler.stop()
+    if last_step[0]:
+        out_last, wav_last = last_step[1]
+        dump_outputs(args.dump_outputs, {**{k: out_last[k] for k in DUMPED}, "waveform": wav_last})
+        last_step[:] = [False, None]
+        del out_last, wav_last
     # one step at a time (every step on lane 0): the loop rounds 1 and 2 reported until in-flight lanes existed
     ms_serial = None
     if n_lanes > 1:

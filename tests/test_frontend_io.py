@@ -1,4 +1,5 @@
 """Host-side rows f2/f3 of SURVEY.md 8f: symbol table / id mapping, script formats, PCM_24 WAV + NPY writers."""
+import json
 import os
 import sys
 import wave
@@ -23,15 +24,25 @@ def test_symbol_table_shape_and_mapping_rules():
         tf.cleaned_text_to_sequence("日本")
 
 
-@pytest.mark.skipif(not shim.available(), reason="/root/reference not present")
 def test_symbol_table_equals_the_reference_file():
-    sys.path.insert(0, os.path.join(shim.REFERENCE_ROOT, "Matcha-TTS", "matcha", "text"))
-    try:
-        import symbols as ref_symbols                    # the reference's own symbols.py, imported where it lies
-    finally:
-        sys.path.pop(0)
-    assert tf.SYMBOLS == ref_symbols.symbols and tf.SPACE_ID == ref_symbols.SPACE_ID
-    assert tf.SYMBOL_TO_ID == {s: i for i, s in enumerate(ref_symbols.symbols)}
+    """Against the reference's table as committed (tests/golden/symbols.json) and, where the reference tree is present, against
+    its own symbols.py imported where it lies (EV_WRITE_GOLDEN=1 then rewrites the fixture from it)."""
+    golden = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "symbols.json")
+    if shim.available():
+        sys.path.insert(0, os.path.join(shim.REFERENCE_ROOT, "Matcha-TTS", "matcha", "text"))
+        try:
+            import symbols as ref_symbols
+        finally:
+            sys.path.pop(0)
+        if os.environ.get("EV_WRITE_GOLDEN"):
+            with open(golden, "w", encoding="utf-8") as f:
+                json.dump({"symbols": ref_symbols.symbols, "space_id": ref_symbols.SPACE_ID}, f, ensure_ascii=False, indent=0)
+                f.write("\n")
+        assert tf.SYMBOLS == ref_symbols.symbols and tf.SPACE_ID == ref_symbols.SPACE_ID
+    with open(golden, encoding="utf-8") as f:
+        ref = json.load(f)
+    assert tf.SYMBOLS == ref["symbols"] and tf.SPACE_ID == ref["space_id"]
+    assert tf.SYMBOL_TO_ID == {s: i for i, s in enumerate(ref["symbols"])}
 
 
 def test_process_text_intersperses_blanks_like_the_cli():

@@ -39,17 +39,17 @@ def test_oracle_matches_reference_golden(name):
 
 
 def test_oracle_matches_compiled_reference():
+    """The seeded sweep against the paths the compiled reference wrote (tests/golden/mas_seeded.npz), and against the
+    compiled reference itself where oracle/_ref/ holds it."""
     ref = build_oracle.load_ref()
-    if ref is None:
-        pytest.skip("oracle/_ref/ not built (only the build container holds /root/reference)")
-    for seed in range(20):
-        rng = np.random.default_rng(100 + seed)
-        b, tx = int(rng.integers(1, 5)), int(rng.integers(1, 40))
-        ty = tx + int(rng.integers(0, 60))
-        v, t_xs, t_ys = mg.make_inputs(200 + seed, b, tx, ty, ["ragged", "ties", "full"][seed % 3])
-        want = np.zeros_like(v).astype(np.int32)
-        ref.maximum_path_c(want, v.copy(), t_xs, t_ys)
-        assert np.array_equal(oracle_path(v, t_xs, t_ys), want), seed
+    g = np.load(os.path.join(GOLD, "mas_seeded.npz"))
+    for i, (b, tx, ty, kind, (v, t_xs, t_ys)) in enumerate(mg.seeded_cases()):
+        want = np.unpackbits(g["path_bits_%d" % i], axis=-1)[..., :ty].astype(np.int32)
+        assert np.array_equal(oracle_path(v, t_xs, t_ys), want), i
+        if ref is not None:
+            live = np.zeros_like(v).astype(np.int32)
+            ref.maximum_path_c(live, v.copy(), t_xs, t_ys)
+            assert np.array_equal(live, want), i
 
 
 def test_path_properties():

@@ -39,6 +39,17 @@ def test_hifigan_oracle_matches_reference_fixture(name):
     assert rel_l2(den, torch.from_numpy(g["denoised"])) < 1e-4
 
 
+def test_parameter_counts_match_the_reference():
+    """The state dicts the oracle and the CUDA loaders consume hold exactly the reference's parameters: 18,204,193 for the
+    single-speaker Matcha-TTS (the count its synthesis.ipynb:127 prints; mel_mean / mel_std are buffers) and 13,926,017 for
+    HiFi-GAN v1."""
+    import dataclasses
+
+    lj = synthetic.matcha_state_dict(dataclasses.replace(VCTK, n_spks=1), seed=1)
+    assert sum(v.numel() for k, v in lj.items() if k not in ("mel_mean", "mel_std")) == 18_204_193
+    assert sum(v.numel() for v in synthetic.hifigan_state_dict(HIFIGAN_V1).values()) == 13_926_017
+
+
 def test_weight_norm_checkpoint_form_folds_to_plain_weights():
     plain = synthetic.hifigan_state_dict(HIFIGAN_V1, seed=7)
     wn = synthetic.hifigan_state_dict(HIFIGAN_V1, seed=7, weight_norm=True)
