@@ -73,6 +73,8 @@ SIGNATURES = {
     "ev_test_ff_block": (_I, [_P] * 11 + [_I, _I, _I, _I, _P, _I, C.POINTER(_F), _P]),
     "ev_test_tf_tail": (_I, [_P] * 14 + [_I, _I, _I, _I, _P, _I, C.POINTER(_F), _P]),
     "ev_test_resnet_block": (_I, [_P, C.POINTER(EvTensor), _I, _P, _P, _I, _I, _I, _I, _I, _P, _P, _P, _I, C.POINTER(_F), _P]),
+    "ev_test_resblock": (_I, [_P, C.POINTER(EvTensor), _I, _I, _I, _P, _P, _I, _I, _I, _F, _F, _I, _I, _P, _I, _I, _I, _I,
+                              _P, _P, _P, _P, _P]),
     "ev_test_resnet_trace": (_I, [_P, _P, _I]),
     "ev_test_vocoder_margins": (_I, [C.POINTER(EvHifiganCfg), C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "ev_test_euler_schedule": (_I, [_I, C.POINTER(_F), C.POINTER(_F)]),

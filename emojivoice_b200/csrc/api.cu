@@ -496,6 +496,129 @@ extern "C" int ev_test_resnet_block(ev_ctx* ctx, const ev_tensor* weights, int n
   return EV_OK;
 }
 
+namespace {
+// (B, C, L) channel-first fp32 -> the vocoder's residual stream (B, L, C) fp32 and its operand lrelu(x, 0.1) as ActT
+template <typename ActT>
+__global__ void rb_input_kernel(const float* __restrict__ x, int C, int L, long long n, float* __restrict__ xs, ActT* __restrict__ xa) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const int c = (int)(i % C);
+  const long long bt = i / C, b = bt / L, t = bt - b * L;
+  const float v = x[(b * C + c) * L + t];
+  xs[i] = v;
+  xa[i] = ActT(v > 0.0f ? v : v * 0.1f);
+}
+
+template <typename ActT>
+int test_resblock(ev_ctx* ctx, const ev_tensor* weights, int n_weights, int C, int k, const float* x, const float* sum_in, int B, int L, int mode,
+                  float inv_n, float slope_out, int write_f32, int want_act, const int64_t* lengths, int rows_per_frame, int margin, int impl,
+                  const int32_t* schedule, float* sum, float* act_out, int32_t* report, cudaStream_t s) {
+  const size_t mark = ctx->owned.size();
+  struct Release {   // frees this call's allocations and leaves the context's ragged planner inactive, on every return path
+    ev_ctx* c; cudaStream_t s; size_t mark;
+    ~Release() {
+      cudaStreamSynchronize(s);
+      for (size_t i = mark; i < c->owned.size(); ++i) cudaFree(c->owned[i]);
+      c->owned.resize(mark);
+      c->rag = RaggedPlanner();
+    }
+  } release{ctx, s, mark};
+  WeightStore ws(ctx, weights, n_weights, s);
+  const int dil[3] = {1, 3, 5};
+  ConvWeights c1[3], c2[3];
+  float* bacc[3] = {};
+  EV_TRY(load_resblock(ctx, ws, "", C, k, dil, c1, c2, bacc, s));
+  // outputs live `guard` rows inside NaN-filled buffers: a row written before item 0 or after item B-1 is caught below
+  const long long n = (long long)B * L * C, guard = 1024LL * C;
+  void *xs = nullptr, *xa = nullptr, *sb = nullptr, *ab = nullptr, *xb = nullptr, *xba = nullptr, *mid = nullptr, *li = nullptr, *arena = nullptr;
+  EV_TRY(device_alloc(ctx, n * 4, &xs, false, s));
+  EV_TRY(device_alloc(ctx, n * sizeof(ActT), &xa, false, s));
+  EV_TRY(device_alloc(ctx, (n + 2 * guard) * 4, &sb, false, s));
+  EV_TRY(device_alloc(ctx, (n + 2 * guard) * sizeof(ActT), &ab, false, s));
+  if (!impl) {
+    EV_TRY(device_alloc(ctx, n * 4, &xb, true, s));
+    EV_TRY(device_alloc(ctx, n * sizeof(ActT), &xba, true, s));
+    EV_TRY(device_alloc(ctx, n * sizeof(ActT), &mid, true, s));
+  }
+  float* sum_buf = reinterpret_cast<float*>(sb) + guard;
+  ActT* act_buf = reinterpret_cast<ActT*>(ab) + guard;
+  EV_CUDA(ctx, cudaMemsetAsync(sb, 0xff, (n + 2 * guard) * 4, s));
+  EV_CUDA(ctx, cudaMemsetAsync(ab, 0xff, (n + 2 * guard) * sizeof(ActT), s));
+  if (mode >= 1) EV_CUDA(ctx, cudaMemcpyAsync(sum_buf, sum_in, n * 4, cudaMemcpyDeviceToDevice, s));
+  rb_input_kernel<ActT><<<(unsigned)((n + 255) / 256), 256, 0, s>>>(x, C, L, n, reinterpret_cast<float*>(xs), reinterpret_cast<ActT*>(xa));
+  EV_CUDA(ctx, cudaGetLastError());
+  if (lengths) {   // as ev_vocode_ragged sets it up: item b needs rows [0, (lengths[b] + margin) * rows_per_frame)
+    const size_t arena_ints = 32 * ((size_t)B * ceil_div(L, 128) + 64);
+    EV_TRY(device_alloc(ctx, (size_t)B * 4, &li, false, s));
+    EV_TRY(device_alloc(ctx, arena_ints * 4, &arena, false, s));
+    EV_CUDA(ctx, i64_to_i32(reinterpret_cast<const long long*>(lengths), reinterpret_cast<int*>(li), B, s));
+    RaggedPlanner& r = ctx->rag;
+    r = RaggedPlanner();
+    r.lens = reinterpret_cast<int*>(li); r.B = B; r.margin = margin; r.rows_per_frame = rows_per_frame;
+    r.arena = reinterpret_cast<int*>(arena); r.arena_ints = arena_ints;
+    r.launch_counter = &ctx->launches;
+  }
+  ResBlockArgs<ActT> a;
+  a.C = C; a.k = k;
+  for (int l = 0; l < 3; ++l) { a.c1[l] = &c1[l]; a.c2[l] = &c2[l]; a.bacc[l] = bacc[l]; }
+  a.x = reinterpret_cast<float*>(xs); a.x_act = reinterpret_cast<ActT*>(xa);
+  a.xb = reinterpret_cast<float*>(xb); a.xba = reinterpret_cast<ActT*>(xba); a.mid = reinterpret_cast<ActT*>(mid);
+  a.sum = sum_buf; a.act_out = want_act ? act_buf : nullptr;
+  a.B = B; a.L = L; a.mode = mode; a.write_f32 = write_f32; a.inv_n = inv_n; a.slope_out = slope_out;
+  a.fused = impl == 1;
+  RbSchedule sched;
+  if (schedule) { sched.cluster = schedule[0]; sched.occ2 = schedule[1]; sched.wave = schedule[2]; sched.resident = schedule[3]; }
+  RbLaunchInfo info;
+  a.sched = &sched; a.info = &info;
+  EV_TRY(run_resblock<ActT>(ctx, a, s));
+  if (report) {
+    const int32_t r[9] = {info.cl, info.occ, info.wave, info.resident, info.w_slots, info.n_epi, info.grid, info.Wv, info.total_tiles};
+    memcpy(report, r, sizeof r);
+  }
+  // the rows around the outputs must still hold the fill pattern
+  std::vector<uint8_t> hs(guard * 4), ha(guard * sizeof(ActT));
+  for (int side = 0; side < 2; ++side) {
+    const long long off = side ? guard + n : 0;
+    EV_CUDA(ctx, cudaMemcpyAsync(hs.data(), reinterpret_cast<float*>(sb) + off, hs.size(), cudaMemcpyDeviceToHost, s));
+    EV_CUDA(ctx, cudaMemcpyAsync(ha.data(), reinterpret_cast<ActT*>(ab) + off, ha.size(), cudaMemcpyDeviceToHost, s));
+    EV_CUDA(ctx, cudaStreamSynchronize(s));
+    for (uint8_t v : hs) if (v != 0xff) return fail(ctx, EV_ERR_STATE, "ev_test_resblock: sum written outside its (B, L, C) rows");
+    for (uint8_t v : ha) if (v != 0xff) return fail(ctx, EV_ERR_STATE, "ev_test_resblock: act_out written outside its (B, L, C) rows");
+  }
+  EV_CUDA(ctx, cudaMemcpyAsync(sum, sum_buf, n * 4, cudaMemcpyDeviceToDevice, s));
+  if (act_out) {
+    if constexpr (std::is_same<ActT, bf16>::value) {
+      bf16_to_f32_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(act_buf, act_out, n);
+      EV_CUDA(ctx, cudaGetLastError());
+    } else {
+      EV_CUDA(ctx, cudaMemcpyAsync(act_out, act_buf, n * 4, cudaMemcpyDeviceToDevice, s));
+    }
+  }
+  EV_CUDA(ctx, cudaStreamSynchronize(s));
+  return EV_OK;
+}
+}  // namespace
+
+// One HiFi-GAN ResBlock1 alone, through the code the vocoder runs (run_resblock, hifigan.cu).  See the header.
+extern "C" int ev_test_resblock(ev_ctx* ctx, const ev_tensor* weights, int n_weights, int C, int k, const float* x, const float* sum_in, int B,
+                                int L, int mode, float inv_n, float slope_out, int write_f32, int want_act, const int64_t* lengths,
+                                int rows_per_frame, int margin, int impl, int precision, const int32_t* schedule, float* sum, float* act_out,
+                                int32_t* report, void* stream) {
+  if (!ctx || !weights || !x || !sum || B <= 0 || L <= 0 || C <= 0 || C % 8 || k <= 0 || mode < 0 || mode > 2 || (mode >= 1 && !sum_in) ||
+      (impl != 0 && impl != 1) || (lengths && (rows_per_frame <= 0 || margin < 0)))
+    return EV_ERR_INVALID;
+  cudaStream_t s = as_stream(stream);
+  EV_CUDA(ctx, cudaSetDevice(ctx->device));
+  if (report) memset(report, 0, 9 * sizeof(int32_t));
+  if (precision == EV_PREC_BF16)
+    return test_resblock<bf16>(ctx, weights, n_weights, C, k, x, sum_in, B, L, mode, inv_n, slope_out, write_f32, want_act, lengths, rows_per_frame,
+                               margin, impl, schedule, sum, act_out, report, s);
+  if (precision == EV_PREC_FP32)
+    return test_resblock<float>(ctx, weights, n_weights, C, k, x, sum_in, B, L, mode, inv_n, slope_out, write_f32, want_act, lengths, rows_per_frame,
+                                margin, impl, schedule, sum, act_out, report, s);
+  return fail(ctx, EV_ERR_INVALID, "ev_test_resblock: unknown precision");
+}
+
 extern "C" int ev_test_resnet_trace(ev_ctx* ctx, uint64_t* out_host, int n) {
   if (!ctx || !out_host || n <= 0) return EV_ERR_INVALID;
   EV_CUDA(ctx, cudaSetDevice(ctx->device));

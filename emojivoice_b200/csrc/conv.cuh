@@ -145,10 +145,17 @@ int tc_sm_count();
 cudaError_t conv_tc_read_trace(unsigned long long* host, int n);   // diagnostic: clock stamps of the last traced launch
 
 // resblock_tc.cu: one fused HiFi-GAN ResBlock1 (six convs, residual stream resident in TMEM)
+// Per-call schedule: -1 keeps the EV_RB_* switch (EV_RB_CLUSTER, EV_RB_OCC2, EV_RB_WAVE, EV_RB_RESIDENT, same values); any other value
+// is forced, and a forced choice the kernel cannot honour for this block fails the launch instead of running another variant.
+struct RbSchedule { int cluster = -1, occ2 = -1, wave = -1, resident = -1; };
+// What a launch ran: CTAs per cluster, CTAs per SM, wavefront schedule, resident weights, weight ring slots, epilogue warps, grid,
+// output rows per (cluster) window and windows of the dense batch.
+struct RbLaunchInfo { int cl = 0, occ = 0, wave = 0, resident = 0, w_slots = 0, n_epi = 0, grid = 0, Wv = 0, total_tiles = 0; };
 bool resblock_tc_supported(int C, int k, const int* dil);
 cudaError_t resblock_tc_launch(int C, int k, const ConvWeights* const c1[3], const ConvWeights* const c2[3], const float* const bacc[3],
                                const float* x, float* sum, bf16* act_out, int B, int L, int mode, float inv_n, float slope_out,
-                               int write_f32, cudaStream_t s, std::string* err, RaggedPlanner* ragged = nullptr);
+                               int write_f32, cudaStream_t s, std::string* err, RaggedPlanner* ragged = nullptr,
+                               const RbSchedule* sched = nullptr, RbLaunchInfo* info = nullptr);
 int conv_tc_pick_bn(int N);
 
 // ff_tc.cu: LayerNorm -> Linear(256 -> inner) -> SnakeBeta -> Linear(inner -> 256) -> + residual -> * mask, one kernel

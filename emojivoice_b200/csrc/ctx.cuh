@@ -191,4 +191,33 @@ template <typename ActT>
 int run_conv(ev_ctx* ctx, const ConvWeights& w, const ActT* x, long long x_ld, long long x_bs, int B, int T_in,
              Epilogue e, cudaStream_t s);
 
+// ---- one HiFi-GAN ResBlock1 (hifigan.cu): what the vocoder runs per block, and what ev_test_resblock runs alone
+// Packs `<prefix>convs1.{0,1,2}` / `<prefix>convs2.{0,1,2}` (C x C x k, dilations dil[0..2] and 1) and the cumulative conv2 biases
+// bacc[l] = sum_{i <= l} convs2.i.bias the fused kernel adds to its residual stream.
+int load_resblock(ev_ctx* ctx, WeightStore& ws, const std::string& prefix, int C, int k, const int dil[3], ConvWeights c1[3],
+                  ConvWeights c2[3], float* bacc[3], cudaStream_t s);
+template <typename ActT>
+struct ResBlockArgs {
+  int C = 0, k = 0;
+  const ConvWeights* c1[3] = {};
+  const ConvWeights* c2[3] = {};
+  const float* bacc[3] = {};
+  const float* x = nullptr;        // fp32 (B, L, C) block input
+  const ActT* x_act = nullptr;     // lrelu(x) as the convs' operand (layer path)
+  float* xb = nullptr; ActT* xba = nullptr; ActT* mid = nullptr;   // layer-path scratch, (B, L, C) each
+  float* sum = nullptr;            // fp32 (B, L, C) multi-receptive-field accumulator
+  ActT* act_out = nullptr;         // mode 2: lrelu(mean, slope_out) (the next stage's operand), or nullptr
+  int B = 0, L = 0;
+  // 0: sum = y   1: sum += y   2: sum = (sum + y) * inv_n (written only if write_f32)   3: as 2 without the sum read (a lone branch;
+  // layer path only)
+  int mode = 0, write_f32 = 1;
+  float inv_n = 1.0f, slope_out = 0.1f;
+  bool fused = false;              // resblock_tc (bf16 only) or six conv launches
+  const RbSchedule* sched = nullptr;
+  RbLaunchInfo* info = nullptr;
+};
+// Ragged batches: ctx->rag, as for run_conv.
+template <typename ActT>
+int run_resblock(ev_ctx* ctx, const ResBlockArgs<ActT>& a, cudaStream_t s);
+
 }  // namespace ev

@@ -64,6 +64,81 @@ int resolve_weight(ev_ctx* ctx, WeightStore& ws, const std::string& base, long l
 }
 }  // namespace
 
+namespace ev {
+
+int load_resblock(ev_ctx* ctx, WeightStore& ws, const std::string& prefix, int C, int k, const int dil[3], ConvWeights c1[3],
+                  ConvWeights c2[3], float* bacc[3], cudaStream_t s) {
+  for (int l = 0; l < 3; ++l) {
+    const std::string a = prefix + "convs1." + std::to_string(l), b = prefix + "convs2." + std::to_string(l);
+    // get_padding(k, d) = (k*d - d)/2  (hifigan/xutils.py:37-38)
+    EV_TRY(make_conv(ctx, ws, {a + ".weight"}, {a + ".bias"}, C, C, k, 1, (k * dil[l] - dil[l]) / 2, dil[l], CONV_NORMAL, TC_BF16, &c1[l]));
+    EV_TRY(make_conv(ctx, ws, {b + ".weight"}, {b + ".bias"}, C, C, k, 1, (k - 1) / 2, 1, CONV_NORMAL, TC_BF16, &c2[l]));
+  }
+  for (int l = 0; l < 3; ++l) {
+    void* q;
+    EV_TRY(device_alloc(ctx, (size_t)align_up(C, 4) * sizeof(float), &q, true, s));
+    bacc[l] = reinterpret_cast<float*>(q);
+  }
+  if (c2[0].bias && c2[1].bias && c2[2].bias) {
+    bias_cumsum_kernel<<<ceil_div(C, 128), 128, 0, s>>>(c2[0].bias, c2[1].bias, c2[2].bias, C, bacc[0], bacc[1], bacc[2]);
+    EV_CUDA(ctx, cudaGetLastError());
+  }
+  return 0;
+}
+
+template <typename ActT>
+int run_resblock(ev_ctx* ctx, const ResBlockArgs<ActT>& a, cudaStream_t s) {
+  const int C = a.C;
+  const long long bs = (long long)a.L * C;
+  if (a.fused) {
+    if constexpr (std::is_same<ActT, bf16>::value) {
+      // fused ResBlock: six convs in one kernel, residual stream resident in TMEM (resblock_tc.cu)
+      if (a.mode > 2) return fail(ctx, EV_ERR_INVALID, "resblock_tc: a lone branch (mode 3) runs layer by layer");
+      const double fl = 3 * 2.0 * 2.0 * a.B * (double)a.L * C * (double)C * a.k;
+      std::string msg;
+      cudaError_t ce;
+      {
+        char nm[48];
+        snprintf(nm, sizeof nm, "resblock_tc/voc c%d k%d", C, a.k);
+        LaunchScope ls(ctx, s, ctx->prof_detail ? nm : "resblock_tc/voc", fl, (double)a.B * a.L * C * (4.0 + (a.mode ? 8.0 : 4.0)));
+        ce = resblock_tc_launch(C, a.k, a.c1, a.c2, a.bacc, a.x, a.sum, a.act_out, a.B, a.L, a.mode, a.inv_n, a.slope_out, a.write_f32, s,
+                                &msg, ctx->rag.active() ? &ctx->rag : nullptr, a.sched, a.info);
+      }
+      if (ce == cudaErrorInvalidValue && !msg.empty()) return fail(ctx, EV_ERR_INVALID, msg);
+      if (ce != cudaSuccess) return fail(ctx, EV_ERR_CUDA, "resblock_tc_launch: " + (msg.empty() ? std::string(cudaGetErrorString(ce)) : msg));
+      return 0;
+    } else {
+      return fail(ctx, EV_ERR_INVALID, "resblock_tc: the fused ResBlock runs with bf16 operands only");
+    }
+  }
+  const float* in_f32 = a.x;
+  const ActT* in_act = a.x_act;
+  for (int l = 0; l < 3; ++l) {  // ResBlock1.forward (hifigan/models.py:90-97)
+    Epilogue e1; e1.act = ACT_LRELU; e1.slope = kSlope; e1.out_act = a.mid; e1.act_ld = C; e1.act_bs = bs;
+    EV_TRY(run_conv<ActT>(ctx, *a.c1[l], in_act, C, bs, a.B, a.L, e1, s));
+    Epilogue e2; e2.res = in_f32; e2.res_ld = C; e2.res_bs = bs;
+    if (l < 2) {
+      e2.out_f32 = a.xb; e2.f32_ld = C; e2.f32_bs = bs;
+      e2.act = ACT_LRELU; e2.slope = kSlope; e2.out_act = a.xba; e2.act_ld = C; e2.act_bs = bs;
+    } else {  // branch output joins the MRF sum; the last branch divides by n_kernels (hifigan/models.py:186-192)
+      if (a.mode == 1 || a.mode == 2) { e2.res2 = a.sum; e2.res2_ld = C; e2.res2_bs = bs; }
+      if (a.mode < 2 || a.write_f32) { e2.out_f32 = a.sum; e2.f32_ld = C; e2.f32_bs = bs; }
+      if (a.mode >= 2) {
+        e2.div = 1.0f / a.inv_n;
+        if (a.act_out) { e2.act = ACT_LRELU; e2.slope = a.slope_out; e2.out_act = a.act_out; e2.act_ld = C; e2.act_bs = bs; }
+      }
+    }
+    EV_TRY(run_conv<ActT>(ctx, *a.c2[l], a.mid, C, bs, a.B, a.L, e2, s));
+    in_f32 = a.xb;
+    in_act = a.xba;
+  }
+  return 0;
+}
+template int run_resblock<float>(ev_ctx*, const ResBlockArgs<float>&, cudaStream_t);
+template int run_resblock<bf16>(ev_ctx*, const ResBlockArgs<bf16>&, cudaStream_t);
+
+}  // namespace ev
+
 extern "C" int ev_load_hifigan(ev_ctx* ctx, const ev_tensor* weights, int n_weights, const ev_hifigan_cfg* cfg, void* stream) {
   if (!ctx || !weights || !cfg) return EV_ERR_INVALID;
   cudaStream_t s = as_stream(stream);
@@ -107,27 +182,9 @@ extern "C" int ev_load_hifigan(ev_ctx* ctx, const ev_tensor* weights, int n_weig
     h.total_up *= u;
     const std::string up = "ups." + std::to_string(i);
     EV_TRY(make_conv(ctx, ws, {up + ".weight"}, {up + ".bias"}, ch, cin, k, u, (k - u) / 2, 1, CONV_TRANSPOSED, TC_BF16, &h.ups[i]));
-    for (int j = 0; j < c.n_kernels; ++j) {
-      const int rk = c.resblock_kernel_sizes[j];
-      for (int l = 0; l < 3; ++l) {
-        const int dl = c.resblock_dilation_sizes[j][l];
-        const std::string rb = "resblocks." + std::to_string(i * c.n_kernels + j);
-        const std::string a = rb + ".convs1." + std::to_string(l), b = rb + ".convs2." + std::to_string(l);
-        // get_padding(k, d) = (k*d - d)/2  (hifigan/xutils.py:37-38)
-        EV_TRY(make_conv(ctx, ws, {a + ".weight"}, {a + ".bias"}, ch, ch, rk, 1, (rk * dl - dl) / 2, dl, CONV_NORMAL, TC_BF16, &h.c1[i][j][l]));
-        EV_TRY(make_conv(ctx, ws, {b + ".weight"}, {b + ".bias"}, ch, ch, rk, 1, (rk - 1) / 2, 1, CONV_NORMAL, TC_BF16, &h.c2[i][j][l]));
-      }
-      for (int l = 0; l < 3; ++l) {
-        void* q;
-        EV_TRY(device_alloc(ctx, (size_t)align_up(ch, 4) * sizeof(float), &q, true, s));
-        h.bacc[i][j][l] = reinterpret_cast<float*>(q);
-      }
-      if (h.c2[i][j][0].bias && h.c2[i][j][1].bias && h.c2[i][j][2].bias) {
-        bias_cumsum_kernel<<<ceil_div(ch, 128), 128, 0, s>>>(h.c2[i][j][0].bias, h.c2[i][j][1].bias, h.c2[i][j][2].bias, ch,
-                                                             h.bacc[i][j][0], h.bacc[i][j][1], h.bacc[i][j][2]);
-        EV_CUDA(ctx, cudaGetLastError());
-      }
-    }
+    for (int j = 0; j < c.n_kernels; ++j)
+      EV_TRY(load_resblock(ctx, ws, "resblocks." + std::to_string(i * c.n_kernels + j) + ".", ch, c.resblock_kernel_sizes[j],
+                           c.resblock_dilation_sizes[j], h.c1[i][j], h.c2[i][j], h.bacc[i][j], s));
   }
   h.c_last = c0 >> c.n_ups;
   if (h.c_last != 32 && h.c_last != 16) return fail(ctx, EV_ERR_INVALID, "conv_post supports 16 or 32 input channels");
@@ -270,54 +327,20 @@ int vocode_impl(ev_ctx* ctx, const float* mel, const long long* mel_lengths, int
     const bool last_stage = (i == c.n_ups - 1);
     ctx->rag.rows_per_frame = (int)(L / T);
     ctx->rag.margin = margins.stage[i];
-    for (int j = 0; j < c.n_kernels; ++j) {
-      if constexpr (std::is_same<ActT, bf16>::value) {
-        // fused ResBlock: six convs in one kernel, residual stream resident in TMEM (resblock_tc.cu)
-        if (h.fuse_resblocks && c.n_kernels >= 2 && L >= 1024 &&
-            resblock_tc_supported(C, c.resblock_kernel_sizes[j], c.resblock_dilation_sizes[j])) {
-          const ConvWeights* c1p[3] = {&h.c1[i][j][0], &h.c1[i][j][1], &h.c1[i][j][2]};
-          const ConvWeights* c2p[3] = {&h.c2[i][j][0], &h.c2[i][j][1], &h.c2[i][j][2]};
-          const float* bp[3] = {h.bacc[i][j][0], h.bacc[i][j][1], h.bacc[i][j][2]};
-          const bool last_branch = j == c.n_kernels - 1;
-          const int mode = last_branch ? 2 : (j == 0 ? 0 : 1);
-          const int rk = c.resblock_kernel_sizes[j];
-          double fl = 0.0;
-          for (int l = 0; l < 3; ++l) fl += 2.0 * 2.0 * B * (double)L * C * (double)C * rk;
-          std::string msg;
-          cudaError_t ce;
-          {
-            char nm[48];
-            snprintf(nm, sizeof nm, "resblock_tc/voc c%d k%d", C, rk);
-            LaunchScope ls(ctx, s, ctx->prof_detail ? nm : "resblock_tc/voc", fl, (double)B * L * C * (4.0 + (mode ? 8.0 : 4.0)));
-            ce = resblock_tc_launch(C, rk, c1p, c2p, bp, v.x0, v.sum, (last_branch && !last_stage) ? v.stage_in : nullptr, B, (int)L, mode,
-                                    1.0f / (float)c.n_kernels, kSlope, last_stage ? 1 : 0, s, &msg,
-                                    ctx->rag.active() ? &ctx->rag : nullptr);
-          }
-          if (ce != cudaSuccess) return fail(ctx, EV_ERR_CUDA, "resblock_tc_launch: " + (msg.empty() ? std::string(cudaGetErrorString(ce)) : msg));
-          continue;
-        }
-      }
-      const float* in_f32 = v.x0;
-      const ActT* in_act = v.x0a;
-      for (int l = 0; l < 3; ++l) {  // ResBlock1.forward (hifigan/models.py:90-97)
-        Epilogue e1; e1.act = ACT_LRELU; e1.slope = kSlope; e1.out_act = v.mid; e1.act_ld = C; e1.act_bs = bs;
-        EV_TRY(run_conv<ActT>(ctx, h.c1[i][j][l], in_act, C, bs, B, (int)L, e1, s));
-        Epilogue e2; e2.res = in_f32; e2.res_ld = C; e2.res_bs = bs;
-        if (l < 2) {
-          e2.out_f32 = v.xb; e2.f32_ld = C; e2.f32_bs = bs;
-          e2.act = ACT_LRELU; e2.slope = kSlope; e2.out_act = v.xba; e2.act_ld = C; e2.act_bs = bs;
-        } else {  // branch output joins the MRF sum; the last branch divides by n_kernels (hifigan/models.py:186-192)
-          if (j > 0) { e2.res2 = v.sum; e2.res2_ld = C; e2.res2_bs = bs; }
-          e2.out_f32 = v.sum; e2.f32_ld = C; e2.f32_bs = bs;
-          if (j == c.n_kernels - 1) {
-            e2.div = (float)c.n_kernels;
-            if (!last_stage) { e2.act = ACT_LRELU; e2.slope = kSlope; e2.out_act = v.stage_in; e2.act_ld = C; e2.act_bs = bs; }
-          }
-        }
-        EV_TRY(run_conv<ActT>(ctx, h.c2[i][j][l], v.mid, C, bs, B, (int)L, e2, s));
-        in_f32 = v.xb;
-        in_act = v.xba;
-      }
+    for (int j = 0; j < c.n_kernels; ++j) {   // the MRF branches: sum = mean_j ResBlock_j(x), lrelu(sum) -> next stage's operand
+      ResBlockArgs<ActT> a;
+      a.C = C; a.k = c.resblock_kernel_sizes[j];
+      for (int l = 0; l < 3; ++l) { a.c1[l] = &h.c1[i][j][l]; a.c2[l] = &h.c2[i][j][l]; a.bacc[l] = h.bacc[i][j][l]; }
+      a.x = v.x0; a.x_act = v.x0a; a.xb = v.xb; a.xba = v.xba; a.mid = v.mid; a.sum = v.sum;
+      a.B = B; a.L = (int)L;
+      const bool last_branch = j == c.n_kernels - 1;
+      a.mode = last_branch ? (j == 0 ? 3 : 2) : (j == 0 ? 0 : 1);
+      a.write_f32 = last_stage ? 1 : 0;   // only conv_post reads the mean in fp32
+      a.act_out = (last_branch && !last_stage) ? v.stage_in : nullptr;
+      a.inv_n = 1.0f / (float)c.n_kernels; a.slope_out = kSlope;
+      a.fused = std::is_same<ActT, bf16>::value && h.fuse_resblocks && c.n_kernels >= 2 && L >= 1024 &&
+                resblock_tc_supported(C, a.k, c.resblock_dilation_sizes[j]);
+      EV_TRY(run_resblock<ActT>(ctx, a, s));
     }
   }
   if (ctx->rag.side) {   // join the side branch whatever happened on it (a captured graph must not end with unjoined work)

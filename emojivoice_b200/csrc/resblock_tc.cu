@@ -749,8 +749,14 @@ cudaError_t launch_rb_kernel(void (*kernel)(KArgs...), int grid, int block, size
 }
 
 template <int C>
-cudaError_t launch_rb(const RbMaps& maps, RbParams& p, int B, cudaStream_t s, RaggedPlanner* ragged) {
+cudaError_t launch_rb(const RbMaps& maps, RbParams& p, int B, cudaStream_t s, RaggedPlanner* ragged, const RbSchedule& sched,
+                      RbLaunchInfo* info, std::string* err) {
   using G = RbCfg<C>;
+  // the EV_RB_* switches, unless this call overrides them
+  const int cluster = sched.cluster >= 0 ? sched.cluster : g_rb_cluster;
+  const bool occ2_on = sched.occ2 >= 0 ? sched.occ2 != 0 : g_rb_occ2 != 0;
+  const bool wave_on = sched.wave >= 0 ? sched.wave != 0 : g_rb_wave != 0;
+  const bool resident_on = sched.resident >= 0 ? sched.resident != 0 : g_rb_resident != 0;
   // CTAs per cluster window: 2 halves the recomputed halo (the wavefront schedule keeps single CTAs)
   // Measured on B200 (profiles/r02_resblock_clusters.txt, us per ResBlock on the ragged config-2 batch, single / paired windows):
   //   C=128: k3 797/855  k7 1658/1546  k11 2849/2194     C=64: k3 633/662  k7 1189/1172  k11 1641/1509
@@ -758,57 +764,80 @@ cudaError_t launch_rb(const RbMaps& maps, RbParams& p, int B, cudaStream_t s, Ra
   // Launching the SAME code as clusters of two costs 2-3 % by itself (CTA placement) and the paired kernel another ~5 %, so pairs pay
   // where the halo is a large part of a window: k >= 7 at C >= 64, k = 11 at C = 32.  EV_RB_CLUSTER=3 pairs everything, =1 nothing.
   const bool pair_pays = (p.k >= 7 && C >= 64) || p.k >= 11;
-  const int cl = ((g_rb_cluster >= 3 || (g_rb_cluster == 2 && pair_pays)) && !g_rb_wave) ? 2 : 1;
+  const int cl = ((cluster >= 3 || (cluster == 2 && pair_pays)) && !wave_on) ? 2 : 1;
   { static const int dbg = []() { const char* v = getenv("EV_RB_DEBUG"); return v ? atoi(v) : 0; }(); p.debug = dbg; }
   p.H = 6 * (p.k - 1);                    // sum over the three pairs of (k-1)/2 * (d_l + 1), d = 1, 3, 5
   p.Wv = cl * G::W - 2 * p.H;             // output rows per (cluster) window
   p.tiles_per_item = ceil_div(p.L, p.Wv);
   p.total_tiles = p.tiles_per_item * B;
-  p.rag = ragged ? ragged->table(p.Wv, p.L, s) : nullptr;
+  // plan: CTAs per SM, all weights resident in shared memory or a ring of w_slots tiles, epilogue warps, shared memory per CTA
+  int occ = 1, n_epi = 16, smem = 0;
+  p.resident = 0;
+  p.w_slots = 0;
   if constexpr (C == 32) {
-    if (g_rb_occ2) {
+    if (occ2_on) {
       const int per_cta = (228 * 1024) / 2 - 2048;
       const int fixed8 = 1024 + G::KC * G::A_PLANE + 8 * G::STAGE_WARP + G::EXTRA;
       const int res_bytes = 6 * p.k * G::W_TILE;
-      int smem;
-      if (g_rb_resident && fixed8 + res_bytes <= per_cta) { p.resident = 1; p.w_slots = 1; smem = fixed8 + res_bytes; }
+      if (resident_on && fixed8 + res_bytes <= per_cta) { p.resident = 1; p.w_slots = 1; smem = fixed8 + res_bytes; }
       else {
         p.resident = 0;
         p.w_slots = std::min((per_cta - fixed8) / G::W_TILE, RB_MAX_SLOTS);
         smem = fixed8 + p.w_slots * G::W_TILE;
       }
-      if (p.w_slots >= 1 && (p.resident || p.w_slots >= 4)) {
-        static DeviceOnce once2;
-        cudaError_t ce2 = once2.run([&]() {
-          cudaError_t ce = cudaFuncSetAttribute(resblock_tc_kernel<C, 2, false, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, per_cta);
-          if (ce == cudaSuccess) ce = cudaFuncSetAttribute(resblock_tc_kernel<C, 2, false, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, per_cta);
-          if (ce == cudaSuccess) ce = cudaFuncSetAttribute(resblock_tc_kernel<C, 2, true, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, per_cta);
-          return ce;
-        });
-        if (ce2 != cudaSuccess) return ce2;
-        const int grid = cl * std::min(p.total_tiles, 2 * tc_sm_count() / cl);
-        // at least a third of the SM's shared memory: a third CTA would not find TMEM columns (2 x 256 are taken)
-        const size_t sm = (size_t)std::max(smem, 80 * 1024);
-        if (p.resident && g_rb_wave) return launch_rb_kernel(resblock_tc_kernel<C, 2, true, 1>, grid, 96 + 32 * 8, sm, 1, s, maps, p);
-        if (cl == 2) return launch_rb_kernel(resblock_tc_kernel<C, 2, false, 2>, grid, 96 + 32 * 8, sm, 2, s, maps, p);
-        return launch_rb_kernel(resblock_tc_kernel<C, 2, false, 1>, grid, 96 + 32 * 8, sm, 1, s, maps, p);
-      }
+      if (p.w_slots >= 1 && (p.resident || p.w_slots >= 4)) { occ = 2; n_epi = 8; }
     }
   }
   const int limit = 224 * 1024;
-  const int fixed16 = 1024 + G::KC * G::A_PLANE + 16 * G::STAGE_WARP + G::EXTRA, fixed8 = 1024 + G::KC * G::A_PLANE + 8 * G::STAGE_WARP + G::EXTRA;
-  const int res_bytes = 6 * p.k * G::W_TILE;
-  int n_epi = 16, smem;
-  p.resident = 0;
-  if (G::KC == 1 && g_rb_resident && fixed16 + res_bytes <= limit) { p.resident = 1; smem = fixed16 + res_bytes; }
-  else if (G::KC == 1 && g_rb_resident && fixed8 + res_bytes <= limit) { p.resident = 1; n_epi = 8; smem = fixed8 + res_bytes; }
-  else {
-    int slots = std::min((limit - fixed16) / G::W_TILE, RB_MAX_SLOTS);
-    if (slots < 3) return cudaErrorInvalidConfiguration;
-    p.w_slots = slots;
-    smem = fixed16 + slots * G::W_TILE;
+  if (occ == 1) {
+    const int fixed16 = 1024 + G::KC * G::A_PLANE + 16 * G::STAGE_WARP + G::EXTRA, fixed8 = 1024 + G::KC * G::A_PLANE + 8 * G::STAGE_WARP + G::EXTRA;
+    const int res_bytes = 6 * p.k * G::W_TILE;
+    p.resident = 0;
+    if (G::KC == 1 && resident_on && fixed16 + res_bytes <= limit) { p.resident = 1; smem = fixed16 + res_bytes; }
+    else if (G::KC == 1 && resident_on && fixed8 + res_bytes <= limit) { p.resident = 1; n_epi = 8; smem = fixed8 + res_bytes; }
+    else {
+      int slots = std::min((limit - fixed16) / G::W_TILE, RB_MAX_SLOTS);
+      if (slots < 3) return cudaErrorInvalidConfiguration;
+      p.w_slots = slots;
+      smem = fixed16 + slots * G::W_TILE;
+    }
+    if (p.resident) p.w_slots = 1;
   }
-  if (p.resident) p.w_slots = 1;
+  const bool wave = wave_on && p.resident && G::BIAS_MMA && G::KC == 1;   // the wavefront issuer needs every weight tile resident
+  // a schedule the caller forces is launched as asked or not at all
+  const char* refuse = nullptr;
+  if (sched.wave == 1 && !wave) refuse = "the wavefront schedule needs resident weights (C = 32, one CTA per SM)";
+  else if (sched.cluster >= 3 && cl != 2) refuse = "paired windows are not combined with the wavefront schedule";
+  else if (sched.occ2 == 1 && occ != 2) refuse = "two CTAs per SM run at C = 32 only";
+  else if (sched.resident == 1 && !p.resident) refuse = "the weights of this block do not fit in shared memory at this occupancy";
+  if (refuse) {
+    if (err) *err = std::string("resblock_tc: forced schedule cannot run: ") + refuse;
+    return cudaErrorInvalidValue;
+  }
+  const int grid = cl * std::min(p.total_tiles, occ * tc_sm_count() / cl);
+  if (info) {
+    info->cl = cl; info->occ = occ; info->wave = wave ? 1 : 0; info->resident = p.resident; info->w_slots = p.w_slots;
+    info->n_epi = n_epi; info->grid = grid; info->Wv = p.Wv; info->total_tiles = p.total_tiles;
+  }
+  p.rag = ragged ? ragged->table(p.Wv, p.L, s) : nullptr;
+  if constexpr (C == 32) {
+    if (occ == 2) {
+      const int per_cta = (228 * 1024) / 2 - 2048;
+      static DeviceOnce once2;
+      cudaError_t ce2 = once2.run([&]() {
+        cudaError_t ce = cudaFuncSetAttribute(resblock_tc_kernel<C, 2, false, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, per_cta);
+        if (ce == cudaSuccess) ce = cudaFuncSetAttribute(resblock_tc_kernel<C, 2, false, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, per_cta);
+        if (ce == cudaSuccess) ce = cudaFuncSetAttribute(resblock_tc_kernel<C, 2, true, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, per_cta);
+        return ce;
+      });
+      if (ce2 != cudaSuccess) return ce2;
+      // at least a third of the SM's shared memory: a third CTA would not find TMEM columns (2 x 256 are taken)
+      const size_t sm = (size_t)std::max(smem, 80 * 1024);
+      if (wave) return launch_rb_kernel(resblock_tc_kernel<C, 2, true, 1>, grid, 96 + 32 * 8, sm, 1, s, maps, p);
+      if (cl == 2) return launch_rb_kernel(resblock_tc_kernel<C, 2, false, 2>, grid, 96 + 32 * 8, sm, 2, s, maps, p);
+      return launch_rb_kernel(resblock_tc_kernel<C, 2, false, 1>, grid, 96 + 32 * 8, sm, 1, s, maps, p);
+    }
+  }
   static DeviceOnce once;
   cudaError_t ce1 = once.run([&]() {
     cudaError_t ce = cudaFuncSetAttribute(resblock_tc_kernel<C, 1, false, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, limit);
@@ -817,7 +846,6 @@ cudaError_t launch_rb(const RbMaps& maps, RbParams& p, int B, cudaStream_t s, Ra
     return ce;
   });
   if (ce1 != cudaSuccess) return ce1;
-  const int grid = cl * std::min(p.total_tiles, tc_sm_count() / cl);
   if (p.debug & 8) {     // how many clusters the device holds at once
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(grid); cfg.blockDim = dim3(96 + 32 * n_epi); cfg.dynamicSmemBytes = (size_t)std::max(smem, 120 * 1024);
@@ -831,7 +859,7 @@ cudaError_t launch_rb(const RbMaps& maps, RbParams& p, int B, cudaStream_t s, Ra
   }
   // shared memory above half an SM keeps a second CTA (and its TMEM allocation) off the SM
   const size_t sm = (size_t)std::max(smem, 120 * 1024);
-  if (G::BIAS_MMA && G::KC == 1 && p.resident && g_rb_wave)
+  if (wave)
     return launch_rb_kernel(resblock_tc_kernel<C, 1, G::BIAS_MMA && G::KC == 1, 1>, grid, 96 + 32 * n_epi, sm, 1, s, maps, p);
   if (cl == 2) return launch_rb_kernel(resblock_tc_kernel<C, 1, false, 2>, grid, 96 + 32 * n_epi, sm, 2, s, maps, p);
   return launch_rb_kernel(resblock_tc_kernel<C, 1, false, 1>, (p.debug & 16) ? grid / 2 * 2 : grid, 96 + 32 * n_epi, sm, (p.debug & 16) ? 2 : 1, s, maps, p);
@@ -875,11 +903,23 @@ bool resblock_tc_supported(int C, int k, const int* dil) {
 }
 
 // One fused ResBlock1.  c1[l] / c2[l]: packed conv weights (bf16 K-major, as conv_tc uses); bacc[l] = cumulative conv2
-// biases (device, [C]).  x, sum: fp32 (B, L, C); act_out: bf16 (B, L, C) or nullptr.
+// biases (device, [C]).  x, sum: fp32 (B, L, C); act_out: bf16 (B, L, C) or nullptr.  A shape the kernel does not take is
+// rejected (cudaErrorInvalidValue and a message in *err).
 cudaError_t resblock_tc_launch(int C, int k, const ConvWeights* const c1[3], const ConvWeights* const c2[3], const float* const bacc[3],
                                const float* x, float* sum, bf16* act_out, int B, int L, int mode, float inv_n, float slope_out,
-                               int write_f32, cudaStream_t s, std::string* err, RaggedPlanner* ragged) {
+                               int write_f32, cudaStream_t s, std::string* err, RaggedPlanner* ragged, const RbSchedule* sched,
+                               RbLaunchInfo* info) {
   rb_read_env();
+  const char* bad = nullptr;
+  if (C != 32 && C != 64 && C != 128) bad = "C must be 32, 64 or 128";
+  else if (k != 3 && k != 7 && k != 11) bad = "k must be 3, 7 or 11";
+  else if (c1[0]->dilation != 1 || c1[1]->dilation != 3 || c1[2]->dilation != 5) bad = "dilations must be (1, 3, 5)";
+  else if (B <= 0 || L <= 0) bad = "empty batch";
+  else if (mode < 0 || mode > 2) bad = "mode must be 0, 1 or 2";
+  if (bad) {
+    if (err) *err = std::string("resblock_tc: ") + bad;
+    return cudaErrorInvalidValue;
+  }
   RbMaps maps;
   RbParams p{};
   const int rb = C == 32 ? 64 : 128;
@@ -904,10 +944,11 @@ cudaError_t resblock_tc_launch(int C, int k, const ConvWeights* const c1[3], con
   p.sum = sum; p.sum_bs = (long long)L * C;
   p.act_out = act_out; p.act_bs = (long long)L * C;
   p.L = L; p.k = k; p.mode = mode; p.inv_n = inv_n; p.slope_out = slope_out; p.write_f32 = write_f32;
+  const RbSchedule sc = sched ? *sched : RbSchedule{};
   switch (C) {
-    case 32: return launch_rb<32>(maps, p, B, s, ragged);
-    case 64: return launch_rb<64>(maps, p, B, s, ragged);
-    default: return launch_rb<128>(maps, p, B, s, ragged);
+    case 32: return launch_rb<32>(maps, p, B, s, ragged, sc, info, err);
+    case 64: return launch_rb<64>(maps, p, B, s, ragged, sc, info, err);
+    default: return launch_rb<128>(maps, p, B, s, ragged, sc, info, err);
   }
 }
 

@@ -237,6 +237,22 @@ EV_API int ev_test_tf_tail(ev_ctx* ctx, const float* xr_cf, const float* att, co
 EV_API int ev_test_resnet_block(ev_ctx* ctx, const ev_tensor* weights, int n_weights, const float* x, const int64_t* y_lengths,
               int B, int T, int C_in, int len_shift, int full, float* out_a, float* out_xr, float* out_n, int repeat,
               float* avg_us_host, void* stream);
+/* One HiFi-GAN ResBlock1 (hifigan/models.py:90-97, dilations 1, 3, 5) and its share of the multi-receptive-field mean
+ * (:186-192), through the code the vocoder runs for each block.  weights: ev_tensor list named convs1.{0,1,2}.weight (C,C,k),
+ * convs1.{0,1,2}.bias, convs2.{0,1,2}.weight, convs2.{0,1,2}.bias.  x (B,C,L) channel-first fp32; sum_in (B,L,C) fp32, read when
+ * mode >= 1.  mode 0: sum = y; 1: sum = sum_in + y; 2: v = (sum_in + y) * inv_n, sum = v if write_f32 (else sum = sum_in),
+ * act = lrelu(v, slope_out) if want_act.  lengths (B) int64 frames or NULL: a ragged batch as ev_vocode_ragged plans it (item b
+ * needs rows [0, (lengths[b] + margin) * rows_per_frame)).  impl 0: six conv launches, 1: the fused kernel (resblock_tc.cu; bf16 only).
+ * precision: EV_PREC_FP32 (impl 0 only) / EV_PREC_BF16.  schedule: NULL or int32[4] {EV_RB_CLUSTER, EV_RB_OCC2, EV_RB_WAVE,
+ * EV_RB_RESIDENT} for this call, -1 = the environment's; a forced value the kernel cannot honour is EV_ERR_INVALID.
+ * Outputs (B,L,C) channel-last fp32: sum, and act (bf16 widened; may be NULL).  A row the call does not write holds NaN (all bits
+ * set); a write outside the B*L rows fails the call.  report: NULL or int32[9] of what the fused kernel launched: CTAs per cluster,
+ * CTAs per SM, wavefront schedule, resident weights, weight ring slots, epilogue warps, grid, output rows per window, windows
+ * (zeros for impl 0). */
+EV_API int ev_test_resblock(ev_ctx* ctx, const ev_tensor* weights, int n_weights, int C, int k, const float* x, const float* sum_in,
+              int B, int L, int mode, float inv_n, float slope_out, int write_f32, int want_act, const int64_t* lengths,
+              int rows_per_frame, int margin, int impl, int precision, const int32_t* schedule, float* sum, float* act,
+              int32_t* report, void* stream);
 /* EV_RN_TRACE=1: clock64 stamps [32] of CTA 0 of the most recent fused ResNet-block launch (host buffer). */
 EV_API int ev_test_resnet_trace(ev_ctx* ctx, uint64_t* out_host, int n);
 /* Host-only: how many mel frames past an utterance's end ev_vocode_ragged still computes in front of conv_pre (pre), of
