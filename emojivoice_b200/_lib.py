@@ -32,6 +32,19 @@ class EvHifiganCfg(C.Structure):
                 ("resblock_kernel_sizes", C.c_int32 * 4), ("resblock_dilation_sizes", (C.c_int32 * 3) * 4)]
 
 
+class EvConvEpilogueTest(C.Structure):
+    _fields_ = ([(n, C.c_int32) for n in ("B", "C_in", "T", "C_out", "K", "stride", "pad", "dilation", "transposed", "precision")] +
+                [("w", C.c_void_p), ("bias", C.c_void_p), ("x", C.c_void_p), ("x_ld", C.c_int64), ("x_bs", C.c_int64),
+                 ("res", C.c_void_p), ("res_ld", C.c_int64), ("res_bs", C.c_int64),
+                 ("res2", C.c_void_p), ("res2_ld", C.c_int64), ("res2_bs", C.c_int64),
+                 ("out_f32", C.c_void_p), ("f32_ld", C.c_int64), ("f32_bs", C.c_int64),
+                 ("out_act", C.c_void_p), ("act_ld", C.c_int64), ("act_bs", C.c_int64),
+                 ("gn_sum", C.c_void_p), ("lengths", C.c_void_p), ("snake_a", C.c_void_p), ("snake_invb", C.c_void_p)] +
+                [(n, C.c_int32) for n in ("gn_groups", "len_shift", "mask_pre", "mask_act", "act", "f32_is_act")] +
+                [("slope", C.c_float), ("alpha", C.c_float), ("div", C.c_float), ("ragged_margin", C.c_int32), ("rows_per_frame", C.c_int32),
+                 ("ragged_lengths", C.c_void_p), ("schedule_host", C.c_void_p), ("report_host", C.c_void_p)])
+
+
 class EvKernelStat(C.Structure):
     _fields_ = [("name", C.c_char * 48), ("launches", C.c_int64), ("total_ms", C.c_double), ("flops", C.c_double),
                 ("bytes", C.c_double)]
@@ -75,6 +88,7 @@ SIGNATURES = {
     "ev_test_resnet_block": (_I, [_P, C.POINTER(EvTensor), _I, _P, _P, _I, _I, _I, _I, _I, _P, _P, _P, _I, C.POINTER(_F), _P]),
     "ev_test_resblock": (_I, [_P, C.POINTER(EvTensor), _I, _I, _I, _P, _P, _I, _I, _I, _F, _F, _I, _I, _P, _I, _I, _I, _I,
                               _P, _P, _P, _P, _P]),
+    "ev_test_conv_epilogue": (_I, [_P, C.POINTER(EvConvEpilogueTest), _P]),
     "ev_test_resnet_trace": (_I, [_P, _P, _I]),
     "ev_test_vocoder_margins": (_I, [C.POINTER(EvHifiganCfg), C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "ev_test_euler_schedule": (_I, [_I, C.POINTER(_F), C.POINTER(_F)]),

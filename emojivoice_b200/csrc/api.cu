@@ -619,6 +619,87 @@ extern "C" int ev_test_resblock(ev_ctx* ctx, const ev_tensor* weights, int n_wei
   return fail(ctx, EV_ERR_INVALID, "ev_test_resblock: unknown precision");
 }
 
+// One tensor-core conv with its fused epilogue, through run_conv / run_conv_tf32 (see the header).
+extern "C" int ev_test_conv_epilogue(ev_ctx* ctx, const ev_conv_epilogue_test* a, void* stream) {
+  static_assert(sizeof(TcSchedule) == 8 * sizeof(int32_t) && sizeof(TcLaunchInfo) == 19 * sizeof(int32_t), "the header's int32 arrays");
+  if (!ctx || !a) return EV_ERR_INVALID;
+  if (a->report_host) memset(a->report_host, 0, sizeof(TcLaunchInfo));
+  if (!a->w || !a->x || a->B <= 0 || a->C_in <= 0 || a->T <= 0 || a->C_out <= 0 || a->K <= 0 || a->precision < 1 || a->precision > 3 ||
+      (a->ragged_lengths && (a->precision != 1 || a->rows_per_frame <= 0 || a->ragged_margin < 0)))
+    return fail(ctx, EV_ERR_INVALID, "ev_test_conv_epilogue: bad arguments");
+  cudaStream_t s = as_stream(stream);
+  EV_CUDA(ctx, cudaSetDevice(ctx->device));
+  const size_t mark = ctx->owned.size();
+  struct Release {   // frees this call's allocations and leaves the context's ragged planner inactive, on every return path
+    ev_ctx* c; cudaStream_t s; size_t mark;
+    ~Release() {
+      cudaStreamSynchronize(s);
+      for (size_t i = mark; i < c->owned.size(); ++i) cudaFree(c->owned[i]);
+      c->owned.resize(mark);
+      c->rag = RaggedPlanner();
+    }
+  } release{ctx, s, mark};
+  ev_tensor tw{}, tb{};
+  tw.name = "w"; tw.data = a->w; tw.ndim = 3;
+  tw.shape[0] = a->transposed ? a->C_in : a->C_out; tw.shape[1] = a->transposed ? a->C_out : a->C_in; tw.shape[2] = a->K;
+  tb.name = "b"; tb.data = a->bias; tb.ndim = 1; tb.shape[0] = a->C_out;
+  ev_tensor list[2] = {tw, tb};
+  WeightStore ws(ctx, list, a->bias ? 2 : 1, s);
+  ConvWeights cw;
+  EV_TRY(make_conv(ctx, ws, {"w"}, a->bias ? std::vector<std::string>{"b"} : std::vector<std::string>{}, a->C_out, a->C_in, a->K, a->stride,
+                   a->pad, a->dilation, a->transposed ? CONV_TRANSPOSED : CONV_NORMAL, a->precision == 1 ? TC_BF16 : TC_TF32X3, &cw));
+  if (a->precision >= 2 && !cw.w_tf32) return fail(ctx, EV_ERR_INVALID, "ev_test_conv_epilogue: this layer has no split tensor-core path");
+  if (a->precision == 2) cw.w_f16x3 = nullptr;   // the 3xTF32 products (what EV_ENC_SPLIT=tf32 selects)
+  if (a->precision == 3 && !cw.w_f16x3) return fail(ctx, EV_ERR_INVALID, "ev_test_conv_epilogue: the 3xFP16 path needs C_in % 64 == 0");
+  Epilogue e;
+  e.res = a->res; e.res_ld = a->res_ld; e.res_bs = a->res_bs;
+  e.res2 = a->res2; e.res2_ld = a->res2_ld; e.res2_bs = a->res2_bs;
+  e.out_f32 = a->out_f32; e.f32_ld = a->f32_ld; e.f32_bs = a->f32_bs;
+  e.out_act = a->out_act; e.act_ld = a->act_ld; e.act_bs = a->act_bs;
+  e.mask_pre = a->mask_pre; e.mask_act = a->mask_act; e.alpha = a->alpha; e.div = a->div; e.f32_is_act = a->f32_is_act;
+  e.act = a->act; e.slope = a->slope; e.snake_a = a->snake_a; e.snake_invb = a->snake_invb;
+  e.gn_sum = a->gn_sum; e.gn_groups = a->gn_groups;
+  if (a->lengths) {
+    void* li = nullptr;
+    EV_TRY(device_alloc(ctx, (size_t)a->B * 4, &li, false, s));
+    EV_CUDA(ctx, i64_to_i32(reinterpret_cast<const long long*>(a->lengths), reinterpret_cast<int*>(li), a->B, s));
+    e.mask = RowMask{reinterpret_cast<int*>(li), a->len_shift};
+  }
+  if (a->ragged_lengths) {   // as ev_vocode_ragged sets it up: item b needs rows [0, (lengths[b] + margin) * rows_per_frame)
+    const size_t arena_ints = 32 * ((size_t)a->B * ceil_div(a->T + 1, 128) + 64);
+    void *li = nullptr, *arena = nullptr;
+    EV_TRY(device_alloc(ctx, (size_t)a->B * 4, &li, false, s));
+    EV_TRY(device_alloc(ctx, arena_ints * 4, &arena, false, s));
+    EV_CUDA(ctx, i64_to_i32(reinterpret_cast<const long long*>(a->ragged_lengths), reinterpret_cast<int*>(li), a->B, s));
+    RaggedPlanner& r = ctx->rag;
+    r = RaggedPlanner();
+    r.lens = reinterpret_cast<int*>(li); r.B = a->B; r.margin = a->ragged_margin; r.rows_per_frame = a->rows_per_frame;
+    r.arena = reinterpret_cast<int*>(arena); r.arena_ints = arena_ints;
+    r.launch_counter = &ctx->launches;
+  }
+  TcSchedule sched;
+  if (a->schedule_host) memcpy(&sched, a->schedule_host, sizeof sched);
+  TcLaunchInfo info;
+  if (a->precision == 1) {
+    EV_TRY(run_conv<bf16>(ctx, cw, reinterpret_cast<const bf16*>(a->x), a->x_ld, a->x_bs, a->B, a->T, e, s, &sched, &info));
+  } else {
+    void* scratch = nullptr;
+    EV_TRY(device_alloc(ctx, (size_t)a->B * a->T * a->C_in * 8, &scratch, false, s));
+    const bool keep = ctx->enc_tc;
+    ctx->enc_tc = true;
+    const int rc = run_conv_tf32(ctx, cw, reinterpret_cast<const float*>(a->x), a->x_ld, a->x_bs, a->B, a->T, e, reinterpret_cast<float*>(scratch), s,
+                                 false, &sched, &info);
+    ctx->enc_tc = keep;
+    EV_TRY(rc);
+    if (info.grid > 0 && info.split != a->precision - 1)
+      return fail(ctx, EV_ERR_INVALID, "ev_test_conv_epilogue: EV_ENC_SPLIT selects the other split path");
+  }
+  if (info.grid == 0) return fail(ctx, EV_ERR_INVALID, "ev_test_conv_epilogue: the layer ran on the CUDA-core kernel, not conv_tc");
+  EV_CUDA(ctx, cudaStreamSynchronize(s));
+  if (a->report_host) memcpy(a->report_host, &info, sizeof info);
+  return EV_OK;
+}
+
 extern "C" int ev_test_resnet_trace(ev_ctx* ctx, uint64_t* out_host, int n) {
   if (!ctx || !out_host || n <= 0) return EV_ERR_INVALID;
   EV_CUDA(ctx, cudaSetDevice(ctx->device));

@@ -132,11 +132,24 @@ cudaError_t ragged_build_table(const int* lens, int B, int margin, int rows_per_
 cudaError_t conv_simt_launch(const ConvGeom& g, const float* x, long long x_ld, long long x_bs, const ConvWeights& w,
                              const Epilogue& e, cudaStream_t stream);
 // conv_tc.cu
+// Per-call schedule: -1 keeps what the EV_TC_* switch chooses (EV_TC_LEAN, EV_TC_MB, EV_TC_CTA2, EV_TC_WIDE, EV_TC_RESIDENT,
+// EV_TC_BK32, EV_TC_HALO, EV_TF32_SHARE); lean / resident / bk32 / halo / share 0 or 1, mb 1 or 2, ctas_per_sm 1 or 2, epi_warps 8 or
+// 16 force that choice.  A forced choice the launch cannot honour fails it (cudaErrorInvalidValue and a message in *err); it is
+// never swapped for another variant.  Forcing only picks among plans that pass the launcher's shared-memory and TMEM guards.
+struct TcSchedule { int lean = -1, mb = -1, ctas_per_sm = -1, epi_warps = -1, resident = -1, bk32 = -1, halo = -1, share = -1; };
+// What a launch ran: tile width BN, m-blocks per tile, CTAs per SM, epilogue warps, MMA issuer warps, resident weights, activation /
+// weight ring slots, K-chunk width, halo reuse (one activation tile serves several taps), TMA boxes per activation tile, lean
+// activation-only epilogue, vector epilogue (else the scalar one), split mode (0 bf16, 1 3xTF32, 2 3xFP16), accumulation groups per
+// tile (> 1: the two-level flush), 3xTF32 operand sharing, compact (ragged) tile list, grid, tiles of the dense batch.
+struct TcLaunchInfo {
+  int bn = 0, mb = 0, ctas_per_sm = 0, epi_warps = 0, issuers = 0, resident = 0, a_slots = 0, b_slots = 0, bk = 0, halo = 0, a_boxes = 0,
+      act_only = 0, vec_ok = 0, split = 0, flush_groups = 0, tf32_share = 0, ragged = 0, grid = 0, total_tiles = 0;
+};
 // x: bf16 activations, or (tf32x3 != 0) the split fp32 pair [hi | lo] of width 2*C_in per row (x_ld, x_bs in elements)
 // split: 0 = bf16 operands; 1 = 3xTF32 (x: the fp32 pair [hi | lo], 2*C_in floats per row); 2 = 3xFP16 (x: [hi | lo] halves, 2*C_in per row)
 cudaError_t conv_tc_launch(const ConvGeom& g, const void* x, long long x_ld, long long x_bs, int tf32x3,
                            const ConvWeights& w, const Epilogue& e, cudaStream_t stream, std::string* err,
-                           RaggedPlanner* ragged = nullptr);
+                           RaggedPlanner* ragged = nullptr, const TcSchedule* sched = nullptr, TcLaunchInfo* info = nullptr);
 bool conv_tc_init(std::string* err);
 // 3-D bf16 tensor map (dims d0 fastest; strides in bytes for d1, d2; box b0 x b1 x 1; swizzle 128 or 64 bytes)
 bool tc_encode_bf16_map(::CUtensorMap_st* map, const void* base, uint64_t d0, uint64_t d1, uint64_t d2, uint64_t s1_bytes,

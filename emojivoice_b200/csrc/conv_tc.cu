@@ -461,6 +461,9 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             if (lane == 0) mbar_arrive(&acc_empty[buf]);
           }
           const int nb = n0 + cb * 32;                 // first output channel of the block (N % 32 == 0 on this path)
+          // the last n-tile of a layer with N % BN != 0 holds blocks past C_out: their accumulator columns are read and released
+          // above like any other, but they have no bias, no SnakeBeta parameters and no output columns
+          if (nb >= N) continue;
           const int row = m0 + mb * BM + q * 32 + lane;
           const float mv = (mask_act && !((row << e.mask.shift) < len_b)) ? 0.0f : 1.0f;
           uint8_t* brow = reinterpret_cast<uint8_t*>(wstage) + lane * ACT_PITCH;
@@ -617,7 +620,8 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
               }
             }
           }
-          if (e.gn_sum) {   // the block's 32 columns are one GroupNorm group: one fp64 atomic pair per warp and block
+          if (e.gn_sum && n0 + cb * 32 < N) {   // the block's 32 columns are one GroupNorm group: one fp64 atomic pair per warp and block
+                                                // (a block past C_out has no group)
             gs = warp_sum(gs); gq = warp_sum(gq);
             if (lane == 0) {
               double* dst = e.gn_sum + ((long long)b * e.gn_groups + ((n0 + cb * 32) >> 5)) * 2;
@@ -697,15 +701,19 @@ int g_tf32_share = 1;      // EV_TF32_SHARE=0: every one of the three products l
 int g_tf32_flush = 1;      // EV_TF32_FLUSH=0: 3xTF32 without two-level accumulation (shows the tensor core's truncation error)
 
 // Shared-memory plan of one launch for `k` CTAs per SM with `epi_warps` epilogue warps; false when the rings do not fit.
+// resident: -1 = EV_TC_RESIDENT and the tile-count heuristic; 0 / 1 = streamed / resident weights (1: false when they cannot stay)
 template <int BN>
-bool plan_smem(TcParams& p, int k, int epi_warps, int* smem_out) {
+bool plan_smem(TcParams& p, int k, int epi_warps, int* smem_out, int resident) {
   const int staging = epi_warps * STAGING_WARP_BYTES;
   const int per_cta = std::min(SMEM_LIMIT, (228 * 1024) / k - 2048);   // 1 KiB driver reserve + static barriers per CTA
   const int budget = per_cta - 1024 - staging;
   const int w_tiles = p.kchunks * p.g.taps;
   int a_slots, b_slots;
-  p.resident = (g_resident_mode != 0) && p.n_tiles == 1 && p.total_tiles >= 2 * k * g_sm_count &&
-               (w_tiles * p.b_tile_bytes + 2 * p.a_slot_bytes <= budget);
+  // resident weights need one n-tile (the producer loads them at n0 = 0) and room beside two activation slots; enough tiles to
+  // amortise the up-front load is a preference only, which a forced choice skips
+  const bool want = resident >= 0 ? resident != 0 : (g_resident_mode != 0 && p.total_tiles >= 2 * k * g_sm_count);
+  p.resident = want && p.n_tiles == 1 && (w_tiles * p.b_tile_bytes + 2 * p.a_slot_bytes <= budget);
+  if (resident == 1 && !p.resident) return false;
   if (p.resident) {
     b_slots = w_tiles;
     a_slots = std::min(MAX_A_SLOTS, (budget - w_tiles * p.b_tile_bytes) / p.a_slot_bytes);
@@ -724,8 +732,14 @@ bool plan_smem(TcParams& p, int k, int epi_warps, int* smem_out) {
   return true;
 }
 
+cudaError_t refuse(std::string* err, const char* why) {
+  if (err) *err = std::string("conv_tc: forced schedule cannot run: ") + why;
+  return cudaErrorInvalidValue;
+}
+
 template <int BN>
-cudaError_t launch_bn(const CUtensorMap& tmA, const CUtensorMap& tmB, TcParams& p, cudaStream_t stream, RaggedPlanner* ragged) {
+cudaError_t launch_bn(const CUtensorMap& tmA, const CUtensorMap& tmB, TcParams& p, cudaStream_t stream, RaggedPlanner* ragged,
+                      const TcSchedule& sc, int split, TcLaunchInfo* info, std::string* err) {
   p.m_tiles = ceil_div(p.g.M, BM * p.mb);
   p.rag = (ragged && !p.tf32) ? ragged->table(BM * p.mb, p.g.M, stream) : nullptr;
   p.n_tiles = ceil_div(p.g.N, BN);
@@ -743,14 +757,25 @@ cudaError_t launch_bn(const CUtensorMap& tmA, const CUtensorMap& tmB, TcParams& 
   bool ok = false;
   const bool flush = p.flush_kc < p.kchunks;
   if (flush && (BN != 128 || p.mb != 1)) return cudaErrorInvalidConfiguration;   // one block per epilogue warp
-  if (!flush && g_cta2_mode && k_tmem >= 2 && (p.total_tiles > g_sm_count || g_cta2_mode == 2) && p.mb * (BN / 32) <= 4 && plan_smem<BN>(p, 2, 8, &smem)) {
+  if (sc.ctas_per_sm == 2 && sc.epi_warps == 16) return refuse(err, "two CTAs per SM run 8 epilogue warps each");
+  // the EV_TC_CTA2 / EV_TC_WIDE switches, unless this call forces CTAs per SM or epilogue warps; a forced pair of CTAs skips
+  // the "more tiles than SMs" preference as EV_TC_CTA2=2 does, never the TMEM and shared-memory conditions
+  const bool two_on = sc.ctas_per_sm >= 0 ? sc.ctas_per_sm == 2
+                                          : sc.epi_warps != 16 && g_cta2_mode && (p.total_tiles > g_sm_count || g_cta2_mode == 2);
+  const bool wide_on = sc.epi_warps >= 0 ? sc.epi_warps == 16 : (g_wide_mode || flush);
+  if (!flush && two_on && k_tmem >= 2 && p.mb * (BN / 32) <= 4 && plan_smem<BN>(p, 2, 8, &smem, sc.resident)) {
     k = 2; threads = NUM_THREADS; ok = true;
   }
-  if (!ok && (g_wide_mode || flush) && plan_smem<BN>(p, 1, 16, &smem)) ok = true;
-  if (!ok && flush) return cudaErrorInvalidConfiguration;
+  if (!ok && sc.ctas_per_sm != 2 && wide_on && plan_smem<BN>(p, 1, 16, &smem, sc.resident)) ok = true;
+  if (!ok && sc.ctas_per_sm != 2 && sc.epi_warps != 16 && !flush && plan_smem<BN>(p, 1, 8, &smem, sc.resident)) {
+    threads = NUM_THREADS; ok = true;
+  }
   if (!ok) {
-    threads = NUM_THREADS;
-    if (!plan_smem<BN>(p, 1, 8, &smem)) return cudaErrorInvalidConfiguration;
+    if (sc.ctas_per_sm == 2) return refuse(err, "two CTAs per SM need 2*mb*BN <= 256 TMEM columns, no split flush and rings that fit");
+    if (sc.epi_warps == 8 && flush) return refuse(err, "the two-level flush of the split paths needs 16 epilogue warps");
+    if (sc.resident == 1) return refuse(err, "resident weights need one n-tile and a weight set that fits in shared memory");
+    if (sc.epi_warps == 16) return refuse(err, "16 epilogue warps leave no room for the rings");
+    return cudaErrorInvalidConfiguration;
   }
   // never let more CTAs become co-resident than TMEM can serve (tcgen05.alloc would spin forever)
   const int min_smem = (228 * 1024) / (k_tmem + 1) + 1;
@@ -760,8 +785,19 @@ cudaError_t launch_bn(const CUtensorMap& tmA, const CUtensorMap& tmB, TcParams& 
   if (ce_attr != cudaSuccess) return ce_attr;
   p.n_issuers = threads == NUM_THREADS_WIDE ? 2 : 1;
   // the sharing walk needs one tap group (haloed tile or a 1x1 conv), streamed weights and room for a step's weight tiles
-  if (p.tf32_share && (p.n_groups != 1 || p.resident || p.b_slots < p.g.taps + 1 || p.a_slots < 2 || p.kchunks % 3 != 0)) p.tf32_share = 0;
+  if (p.tf32_share && (p.n_groups != 1 || p.resident || p.b_slots < p.g.taps + 1 || p.a_slots < 2 || p.kchunks % 3 != 0)) {
+    if (sc.share == 1) return refuse(err, "operand sharing needs one tap group, streamed weights and a weight slot per tap and one more");
+    p.tf32_share = 0;
+  }
   const int grid = std::min(p.total_tiles, k * g_sm_count);
+  if (info) {
+    TcLaunchInfo& r = *info;
+    r.bn = BN; r.mb = p.mb; r.ctas_per_sm = k; r.epi_warps = threads / 32 - 1 - p.n_issuers; r.issuers = p.n_issuers;
+    r.resident = p.resident; r.a_slots = p.a_slots; r.b_slots = p.b_slots; r.bk = p.bk; r.halo = p.n_groups == 1 && p.g.taps > 1;
+    r.a_boxes = p.a_boxes; r.act_only = p.act_only; r.vec_ok = p.vec_ok; r.split = split;
+    r.flush_groups = (p.kchunks + p.flush_kc - 1) / p.flush_kc; r.tf32_share = p.tf32_share; r.ragged = p.rag != nullptr;
+    r.grid = grid; r.total_tiles = p.total_tiles;
+  }
   return launch_pdl(conv_tc_kernel<BN>, dim3(grid), dim3(threads), (size_t)smem, stream, tmA, tmB, p);
 }
 
@@ -800,8 +836,20 @@ bool conv_tc_init(std::string* err) {
 
 // x: channel-last bf16 activations (b, t, c) at x + b*x_bs + t*x_ld + c, `x_rows` addressable rows per item.
 cudaError_t conv_tc_launch(const ConvGeom& g, const void* x, long long x_ld, long long x_bs, int tf32x3,
-                           const ConvWeights& w, const Epilogue& e, cudaStream_t stream, std::string* err, RaggedPlanner* ragged) {
+                           const ConvWeights& w, const Epilogue& e, cudaStream_t stream, std::string* err, RaggedPlanner* ragged,
+                           const TcSchedule* sched, TcLaunchInfo* info) {
   if (!g_encode && !conv_tc_init(err)) return cudaErrorNotSupported;
+  const TcSchedule sc = sched ? *sched : TcSchedule{};
+  {
+    auto flag = [](int v) { return v >= -1 && v <= 1; };
+    if (!flag(sc.lean) || !flag(sc.resident) || !flag(sc.bk32) || !flag(sc.halo) || !flag(sc.share) || (sc.mb != -1 && sc.mb != 1 && sc.mb != 2) ||
+        (sc.ctas_per_sm != -1 && sc.ctas_per_sm != 1 && sc.ctas_per_sm != 2) || (sc.epi_warps != -1 && sc.epi_warps != 8 && sc.epi_warps != 16))
+      return refuse(err, "a value outside its choices");
+    if (tf32x3 && sc.bk32 >= 0) return refuse(err, "the split paths have a fixed K-chunk width");
+    if (tf32x3 && sc.mb == 2) return refuse(err, "the split paths run one m-block per tile (one 32 x 32 block per epilogue warp)");
+    if (!tf32x3 && sc.share == 1) return refuse(err, "operand sharing is a walk of the split paths");
+    if (sc.bk32 == 1 && g.C_in > 32) return refuse(err, "BK = 32 serves C_in <= 32 only");
+  }
   const int esz = tf32x3 == 1 ? 4 : 2;
   if ((x_ld * esz & 15) || (x_bs * esz & 15) || (reinterpret_cast<uintptr_t>(x) & 15)) {
     if (err) *err = "conv_tc: activation tensor is not 16-byte aligned / strided";
@@ -840,7 +888,7 @@ cudaError_t conv_tc_launch(const ConvGeom& g, const void* x, long long x_ld, lon
     p.idesc = make_idesc(BM, BN) & ~((7u << 7) | (7u << 10));      // kind::f16 with F16 (format 0) operands instead of BF16
     p.flush_kc = std::max(1, 16 / (g.taps * p.ksteps));
     if (g_tf32_flush == 0) p.flush_kc = p.kchunks;
-    p.tf32_share = g_tf32_share;
+    p.tf32_share = sc.share >= 0 ? sc.share : g_tf32_share;
     p.descale = w.f16_scale;
   } else if (tf32x3) {      // 32 fp32 channels per 128-byte row, UMMA K = 8; K-chunks walk [x_hi | x_hi | x_lo] x [w_hi | w_lo | w_hi]
     if (g.conv_stride != 1 || !w.w_tf32) { if (err) *err = "conv_tc: the 3xTF32 path needs stride 1 and split weights"; return cudaErrorInvalidValue; }
@@ -853,10 +901,10 @@ cudaError_t conv_tc_launch(const ConvGeom& g, const void* x, long long x_ld, lon
     p.idesc = make_idesc_tf32(BM, BN);
     p.flush_kc = std::max(1, 16 / (g.taps * p.ksteps));    // <= 16 truncating tensor-core accumulations per partial sum
     if (g_tf32_flush == 0) p.flush_kc = p.kchunks;
-    p.tf32_share = g_tf32_share;
+    p.tf32_share = sc.share >= 0 ? sc.share : g_tf32_share;
   } else {
     p.tf32_share = 0;
-    p.bk = (g_bk32_mode && g.C_in <= 32) ? 32 : 64;
+    p.bk = ((sc.bk32 >= 0 ? sc.bk32 : g_bk32_mode) && g.C_in <= 32) ? 32 : 64;
     p.row_bytes = p.bk * 2;
     p.ksteps = p.bk / UMMA_K;
     p.kchunks = ceil_div(g.C_in, p.bk);
@@ -897,6 +945,7 @@ cudaError_t conv_tc_launch(const ConvGeom& g, const void* x, long long x_ld, lon
     };
     p.mb = (g.M > BM && cost(2) <= cost(1)) ? 2 : 1;
     if (g_mb_mode == 1 || g_mb_mode == 2) p.mb = g_mb_mode;
+    if (sc.mb > 0) p.mb = sc.mb;
     if (tf32x3) p.mb = 1;            // two-level accumulation: one 32 x 32 block per epilogue warp (16 warps, 128 x 128 tile)
     if (p.mb > MB_MAX) p.mb = MB_MAX;
   }
@@ -904,7 +953,9 @@ cudaError_t conv_tc_launch(const ConvGeom& g, const void* x, long long x_ld, lon
   int lo = tap_row[0], hi = tap_row[0];
   bool same_col = true;
   for (int j = 1; j < g.taps; ++j) { lo = std::min(lo, tap_row[j]); hi = std::max(hi, tap_row[j]); same_col &= tap_col[j] == tap_col[0]; }
-  const bool halo = g_halo_mode != 0 && g.taps > 1 && same_col && (hi - lo) <= 128;
+  const bool halo_ok = g.taps > 1 && same_col && (hi - lo) <= 128;
+  if (sc.halo == 1 && !halo_ok) return refuse(err, "halo reuse needs several taps that read the same columns within 128 rows");
+  const bool halo = (sc.halo >= 0 ? sc.halo != 0 : g_halo_mode != 0) && halo_ok;
   int a_rows;
   if (halo) {
     p.n_groups = 1;
@@ -959,9 +1010,11 @@ cudaError_t conv_tc_launch(const ConvGeom& g, const void* x, long long x_ld, lon
              ((reinterpret_cast<uintptr_t>(e.res) | reinterpret_cast<uintptr_t>(e.res2) |
                reinterpret_cast<uintptr_t>(e.out_f32) | reinterpret_cast<uintptr_t>(e.bias)) & 15) == 0 &&
              (reinterpret_cast<uintptr_t>(e.out_act) & 7) == 0;
-  p.act_only = g_lean_mode && p.vec_ok && e.out_act && !e.out_f32 && !e.res && !e.res2 && e.alpha == 1.0f && e.div == 1.0f &&
-               !e.mask_pre && e.phase_cout == g.N && g.N % 32 == 0 && (e.act_ld % 8) == 0 && (e.act_bs % 8) == 0 &&
-               (reinterpret_cast<uintptr_t>(e.out_act) & 15) == 0;
+  const bool lean_ok = p.vec_ok && e.out_act && !e.out_f32 && !e.res && !e.res2 && e.alpha == 1.0f && e.div == 1.0f &&
+                       !e.mask_pre && e.phase_cout == g.N && g.N % 32 == 0 && (e.act_ld % 8) == 0 && (e.act_bs % 8) == 0 &&
+                       (reinterpret_cast<uintptr_t>(e.out_act) & 15) == 0;
+  if (sc.lean == 1 && !lean_ok) return refuse(err, "the lean epilogue serves a bf16-only output of an ordinary conv with N % 32 == 0 and aligned rows");
+  p.act_only = (sc.lean >= 0 ? sc.lean != 0 : g_lean_mode != 0) && lean_ok;
   if (e.gn_sum && (!p.vec_ok || !e.out_f32 || e.phase_cout != g.N || g.N % 32 != 0 || g.N / 32 != e.gn_groups)) {
     if (err) *err = "conv_tc: fused GroupNorm statistics need 32 channels per group on the vector path";
     return cudaErrorInvalidValue;
@@ -970,9 +1023,9 @@ cudaError_t conv_tc_launch(const ConvGeom& g, const void* x, long long x_ld, lon
   { static const int ia = []() { const char* v = getenv("EV_TC_IDLE_ARRIVE"); return v ? atoi(v) : 1; }(); p.idle_arrive = ia; }
   { static const int tr = []() { const char* v = getenv("EV_TC_TRACE"); return v ? atoi(v) : 0; }(); p.trace = tr; }
   switch (BN) {
-    case 32: return launch_bn<32>(tmA, tmB, p, stream, ragged);
-    case 64: return launch_bn<64>(tmA, tmB, p, stream, ragged);
-    default: return launch_bn<128>(tmA, tmB, p, stream, ragged);
+    case 32: return launch_bn<32>(tmA, tmB, p, stream, ragged, sc, tf32x3, info, err);
+    case 64: return launch_bn<64>(tmA, tmB, p, stream, ragged, sc, tf32x3, info, err);
+    default: return launch_bn<128>(tmA, tmB, p, stream, ragged, sc, tf32x3, info, err);
   }
 }
 

@@ -183,13 +183,14 @@ int conv_geometry(const ConvWeights& w, int B, int T_in, ConvGeom* g);
 // fp32-accurate tensor-core convolution (3xTF32 split); `scratch` holds B*T_in*2*C_in floats
 // presplit: `scratch` already holds the 3xFP16 [hi | lo] operand of x (written by the producer: LnArgs::split / AttnArgs::split);
 // honoured only when the 3xFP16 path runs (enc_split_f16()), otherwise x is split here as usual
+// sched / info: conv_tc_launch's per-call schedule and launch report (conv.cuh); left untouched when the CUDA-core kernel runs
 int run_conv_tf32(ev_ctx* ctx, const ConvWeights& w, const float* x, long long x_ld, long long x_bs, int B, int T_in, Epilogue e,
-                  float* scratch, cudaStream_t s, bool presplit = false);
+                  float* scratch, cudaStream_t s, bool presplit = false, const TcSchedule* sched = nullptr, TcLaunchInfo* info = nullptr);
 bool enc_split_f16();   // EV_ENC_SPLIT=tf32 selects the round-1 3xTF32 products (their operand has another layout)
 
 template <typename ActT>
 int run_conv(ev_ctx* ctx, const ConvWeights& w, const ActT* x, long long x_ld, long long x_bs, int B, int T_in,
-             Epilogue e, cudaStream_t s);
+             Epilogue e, cudaStream_t s, const TcSchedule* sched = nullptr, TcLaunchInfo* info = nullptr);
 
 // ---- one HiFi-GAN ResBlock1 (hifigan.cu): what the vocoder runs per block, and what ev_test_resblock runs alone
 // Packs `<prefix>convs1.{0,1,2}` / `<prefix>convs2.{0,1,2}` (C x C x k, dilations dil[0..2] and 1) and the cumulative conv2 biases

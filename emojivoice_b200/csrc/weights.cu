@@ -303,7 +303,7 @@ int conv_geometry(const ConvWeights& w, int B, int T_in, ConvGeom* g) {
 
 template <typename ActT>
 int run_conv(ev_ctx* ctx, const ConvWeights& w, const ActT* x, long long x_ld, long long x_bs, int B, int T_in, Epilogue e,
-             cudaStream_t s) {
+             cudaStream_t s, const TcSchedule* sched, TcLaunchInfo* info) {
   ConvGeom g;
   const int T_out = conv_geometry(w, B, T_in, &g);
   e.bias = w.bias;
@@ -336,7 +336,8 @@ int run_conv(ev_ctx* ctx, const ConvWeights& w, const ActT* x, long long x_ld, l
       snprintf(buf, sizeof buf, " c%d n%d k%d d%d m%d", w.C_in, w.N, w.taps, w.dilation, g.M);
       nm += buf;
     }
-    { LaunchScope ls(ctx, s, nm.c_str(), flops, bytes); ce = conv_tc_launch(g, x, x_ld, x_bs, 0, w, e, s, &msg, ctx->rag.active() ? &ctx->rag : nullptr); }
+    { LaunchScope ls(ctx, s, nm.c_str(), flops, bytes); ce = conv_tc_launch(g, x, x_ld, x_bs, 0, w, e, s, &msg, ctx->rag.active() ? &ctx->rag : nullptr, sched, info); }
+    if (ce == cudaErrorInvalidValue && !msg.empty()) return fail(ctx, EV_ERR_INVALID, msg);
     if (ce != cudaSuccess) return fail(ctx, EV_ERR_CUDA, "conv_tc_launch: " + (msg.empty() ? std::string(cudaGetErrorString(ce)) : msg));
   }
   return 0;
@@ -350,7 +351,7 @@ bool enc_split_f16() {
 }
 
 int run_conv_tf32(ev_ctx* ctx, const ConvWeights& w, const float* x, long long x_ld, long long x_bs, int B, int T_in, Epilogue e,
-                  float* scratch, cudaStream_t s, bool presplit) {
+                  float* scratch, cudaStream_t s, bool presplit, const TcSchedule* sched, TcLaunchInfo* info) {
   const bool aligned = (e.f32_ld % 4 == 0) && (e.f32_bs % 4 == 0) && (e.act_ld % 4 == 0) && (e.res_ld % 4 == 0) && w.N % 4 == 0;
   const bool act_ok = e.act == ACT_NONE || e.act == ACT_RELU || e.act == ACT_LRELU;
   if (!w.w_tf32 || !scratch || x_bs != (long long)T_in * x_ld || !aligned || !act_ok || (e.out_act && e.out_f32) || !ctx->enc_tc ||
@@ -392,12 +393,15 @@ int run_conv_tf32(ev_ctx* ctx, const ConvWeights& w, const float* x, long long x
     snprintf(buf, sizeof buf, " c%d n%d k%d m%d", w.C_in, w.N, w.taps, g.M);
     nm += buf;
   }
-  { LaunchScope ls(ctx, s, nm.c_str(), flops, bytes); ce = conv_tc_launch(g, scratch, 2LL * w.C_in, (long long)T_in * 2 * w.C_in, split, w, e, s, &msg); }
+  { LaunchScope ls(ctx, s, nm.c_str(), flops, bytes); ce = conv_tc_launch(g, scratch, 2LL * w.C_in, (long long)T_in * 2 * w.C_in, split, w, e, s, &msg, nullptr, sched, info); }
+  if (ce == cudaErrorInvalidValue && !msg.empty()) return fail(ctx, EV_ERR_INVALID, msg);
   if (ce != cudaSuccess) return fail(ctx, EV_ERR_CUDA, "conv_tc_launch(tf32x3): " + (msg.empty() ? std::string(cudaGetErrorString(ce)) : msg));
   return 0;
 }
 
-template int run_conv<float>(ev_ctx*, const ConvWeights&, const float*, long long, long long, int, int, Epilogue, cudaStream_t);
-template int run_conv<bf16>(ev_ctx*, const ConvWeights&, const bf16*, long long, long long, int, int, Epilogue, cudaStream_t);
+template int run_conv<float>(ev_ctx*, const ConvWeights&, const float*, long long, long long, int, int, Epilogue, cudaStream_t, const TcSchedule*,
+                             TcLaunchInfo*);
+template int run_conv<bf16>(ev_ctx*, const ConvWeights&, const bf16*, long long, long long, int, int, Epilogue, cudaStream_t, const TcSchedule*,
+                            TcLaunchInfo*);
 
 }  // namespace ev

@@ -253,6 +253,50 @@ EV_API int ev_test_resblock(ev_ctx* ctx, const ev_tensor* weights, int n_weights
               int B, int L, int mode, float inv_n, float slope_out, int write_f32, int want_act, const int64_t* lengths,
               int rows_per_frame, int margin, int impl, int precision, const int32_t* schedule, float* sum, float* act,
               int32_t* report, void* stream);
+/* One tensor-core convolution (conv_tc.cu) with its fused epilogue, through the dispatch the models use (bf16 operands, or the
+ * text encoder's split fp32 paths).  Every tensor is the caller's: outputs are written in place and nothing else is touched, so
+ * the caller can surround them with guard rows and padding columns and check those afterwards.
+ *   w (C_out,C_in,K) or, transposed, (C_in,C_out,K) fp32 and bias (C_out) fp32 or NULL: packed like every layer.
+ *   precision 1: bf16 operands, x bf16; 2: 3xTF32, 3: 3xFP16 (C_in % 64 == 0), x fp32 dense (x_bs == T*x_ld); outputs fp32 only.
+ *   x (B,T,C_in) channel-last at x + b*x_bs + t*x_ld + c.  res, res2, out_f32 fp32 and out_act bf16 (B,T_out,C_out) channel-last
+ *   with their own ld / bs, each NULL when unused.  Per output element, on rows t < T_out (mask m = (t << len_shift) < lengths[b]):
+ *     v = (acc + bias), 0 where !m if mask_pre;  v = v*alpha + res + res2;  v = v * (1/div)
+ *     out_f32 = v, or a if f32_is_act;  out_act = bf16(a);  a = act(v), 0 where !m if mask_act
+ *   act 0 identity, 1 ReLU, 2 LeakyReLU(slope), 4 SnakeBeta with snake_a = exp(alpha_c), snake_invb = 1/(exp(beta_c) + 1e-9).
+ *   gn_sum (B,gn_groups,2) fp64 or NULL: the sum and sum of squares of out_f32 per 32-channel group are added in.
+ *   lengths (B) int64 or NULL = no mask.  ragged_lengths (B) int64 frames or NULL: a compact tile list as ev_vocode_ragged plans it
+ *   (rows [0, (ragged_lengths[b] + ragged_margin) * rows_per_frame) are needed; precision 1 only).
+ *   schedule_host: NULL or int32[8] {lean, mb, ctas_per_sm, epi_warps, resident, bk32, halo, share}, -1 = the environment's
+ *   EV_TC_* choice; a forced choice the launch cannot honour is EV_ERR_INVALID.  report_host: NULL or int32[19] of what ran: BN,
+ *   m-blocks, CTAs per SM, epilogue warps, MMA issuers, resident weights, activation / weight ring slots, K-chunk width, halo reuse,
+ *   TMA boxes per activation tile, lean epilogue, vector epilogue, split mode (0 bf16, 1 3xTF32, 2 3xFP16), accumulation groups
+ *   per tile, operand sharing, compact tile list, grid, tiles.  Synchronises `stream`. */
+typedef struct {
+  int32_t B, C_in, T, C_out, K, stride, pad, dilation, transposed, precision;
+  const float* w;
+  const float* bias;
+  const void* x;
+  int64_t x_ld, x_bs;
+  const float* res;
+  int64_t res_ld, res_bs;
+  const float* res2;
+  int64_t res2_ld, res2_bs;
+  float* out_f32;
+  int64_t f32_ld, f32_bs;
+  void* out_act;
+  int64_t act_ld, act_bs;
+  double* gn_sum;
+  const int64_t* lengths;
+  const float* snake_a;
+  const float* snake_invb;
+  int32_t gn_groups, len_shift, mask_pre, mask_act, act, f32_is_act;
+  float slope, alpha, div;
+  int32_t ragged_margin, rows_per_frame;
+  const int64_t* ragged_lengths;
+  const int32_t* schedule_host;
+  int32_t* report_host;
+} ev_conv_epilogue_test;
+EV_API int ev_test_conv_epilogue(ev_ctx* ctx, const ev_conv_epilogue_test* args, void* stream);
 /* EV_RN_TRACE=1: clock64 stamps [32] of CTA 0 of the most recent fused ResNet-block launch (host buffer). */
 EV_API int ev_test_resnet_trace(ev_ctx* ctx, uint64_t* out_host, int n);
 /* Host-only: how many mel frames past an utterance's end ev_vocode_ragged still computes in front of conv_pre (pre), of
