@@ -83,6 +83,7 @@ SIGNATURES = {
     "ev_test_conv1d": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P, _P]),
     "ev_test_attention": (_I, [_P, _P, _P, _I, _I, _I, _I, _I, _P, _P]),
     "ev_test_encoder_attention": (_I, [_P, _P, _P, _I, _I, _I, _I, _P, _I, C.POINTER(_F), _P]),
+    "ev_test_encoder_attention_hd": (_I, [_P, _P, _P, _I, _I, _I, _I, _I, _P, _I, C.POINTER(_F), _P]),
     "ev_test_ff_block": (_I, [_P] * 11 + [_I, _I, _I, _I, _P, _I, C.POINTER(_F), _P]),
     "ev_test_tf_tail": (_I, [_P] * 14 + [_I, _I, _I, _I, _P, _I, C.POINTER(_F), _P]),
     "ev_test_resnet_block": (_I, [_P, C.POINTER(EvTensor), _I, _P, _P, _I, _I, _I, _I, _I, _P, _P, _P, _I, C.POINTER(_F), _P]),

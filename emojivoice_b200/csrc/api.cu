@@ -244,15 +244,18 @@ extern "C" int ev_test_attention(ev_ctx* ctx, const float* qkv, const int64_t* y
   return EV_OK;
 }
 
-// Text-encoder attention alone (text_encoder.py:223-246, head width 128, RoPE on the first 64 features): qkv (B, T, 3*H*128)
-// CHANNEL-LAST fp32 [q | k | v], x_lengths (B) int64 or NULL, out (B, T, H*128).  impl 0: fp32 CUDA cores (attention.cu),
-// 1: tcgen05 with 3xFP16 split operands (attention_enc_tc.cu).  repeat / avg_us_host as ev_test_ff_block.
-extern "C" int ev_test_encoder_attention(ev_ctx* ctx, const float* qkv, const int64_t* x_lengths, int B, int T, int H, int impl,
-                                         float* out, int repeat, float* avg_us_host, void* stream) {
+// Text-encoder attention alone (text_encoder.py:223-246, head width hd, RoPE on the first hd / 2 features): qkv (B, T, 3*H*hd)
+// CHANNEL-LAST fp32 [q | k | v], x_lengths (B) int64 or NULL, out (B, T, H*hd).  impl 0: fp32 CUDA cores (attention.cu,
+// hd 64 / 96 / 128), 1: tcgen05 with 3xFP16 split operands (attention_enc_tc.cu, hd 96 / 128).  repeat / avg_us_host as
+// ev_test_ff_block.
+extern "C" int ev_test_encoder_attention_hd(ev_ctx* ctx, const float* qkv, const int64_t* x_lengths, int B, int T, int H, int hd,
+                                            int impl, float* out, int repeat, float* avg_us_host, void* stream) {
   if (!ctx || !qkv || !out || B <= 0 || T <= 0 || H <= 0) return EV_ERR_INVALID;
+  if (hd != 96 && hd != 128 && (impl == 1 || hd != 64))
+    return fail(ctx, EV_ERR_INVALID, "ev_test_encoder_attention_hd: no kernel for this head width / impl");
   cudaStream_t s = as_stream(stream);
   EV_CUDA(ctx, cudaSetDevice(ctx->device));
-  const int hd = 128, inner = H * hd, rope_dim = hd / 2;
+  const int inner = H * hd, rope_dim = hd / 2;
   const size_t mark = ctx->owned.size();
   auto release = [&]() {
     cudaStreamSynchronize(s);
@@ -291,6 +294,11 @@ extern "C" int ev_test_encoder_attention(ev_ctx* ctx, const float* qkv, const in
   release();
   if (ce != cudaSuccess) return cuda_fail(ctx, ce, "ev_test_encoder_attention");
   return EV_OK;
+}
+
+extern "C" int ev_test_encoder_attention(ev_ctx* ctx, const float* qkv, const int64_t* x_lengths, int B, int T, int H, int impl,
+                                         float* out, int repeat, float* avg_us_host, void* stream) {
+  return ev_test_encoder_attention_hd(ctx, qkv, x_lengths, B, T, H, 128, impl, out, repeat, avg_us_host, stream);
 }
 
 // Fused transformer feed-forward alone (ff_tc.cu): x (B, T, 256) CHANNEL-LAST fp32; w1 (inner, 256), w2 (256, inner) as

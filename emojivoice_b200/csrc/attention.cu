@@ -190,6 +190,7 @@ cudaError_t launch_attn(const AttnArgs& a, cudaStream_t s) {
 template <typename ActT>
 cudaError_t attention_rows(const AttnArgs& a, cudaStream_t s) {
   if (a.D == 64) return launch_attn<ActT, 64>(a, s);
+  if (a.D == 96) return launch_attn<ActT, 96>(a, s);
   if (a.D == 128) return launch_attn<ActT, 128>(a, s);
   return cudaErrorInvalidValue;
 }

@@ -61,7 +61,7 @@ struct AttnArgs {
   void* split = nullptr;   // attention_enc_tc only: optional [B*T][2*H*D] fp16 [hi | lo] halves of out * kF16ActScale (see LnArgs::split)
 };
 template <typename ActT> cudaError_t attention_rows(const AttnArgs& a, cudaStream_t s);
-// Text-encoder attention (mode 0, head width 128, T <= 384) on tcgen05 with 3xFP16 split operands, fp32 output
+// Text-encoder attention (mode 0, head width 96 or 128 with RoPE on half the head, T <= 384) on tcgen05 with 3xFP16 split operands, fp32 output
 // (attention_enc_tc.cu); any other shape stays on attention_rows<float>.
 bool attention_enc_tc_supported(const AttnArgs& a);
 cudaError_t attention_enc_tc(const AttnArgs& a, cudaStream_t s);

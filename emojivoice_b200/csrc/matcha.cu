@@ -72,8 +72,9 @@ extern "C" int ev_load_matcha(ev_ctx* ctx, const ev_tensor* weights, int n_weigh
   const int D = c.dec_channels;
   const int inner = c.dec_heads * c.dec_head_dim;
   const int dec_in = 2 * c.n_feats + (c.n_spks > 1 ? c.spk_emb_dim : 0);
-  if (c.enc_heads <= 0 || H % c.enc_heads || (H / c.enc_heads != 128 && H / c.enc_heads != 64))
-    return fail(ctx, EV_ERR_INVALID, "text-encoder head width must be 64 or 128");
+  // head widths with an encoder attention kernel (attention.cu; 96 and 128 also attention_enc_tc.cu)
+  if (c.enc_heads <= 0 || H % c.enc_heads || (H / c.enc_heads != 64 && H / c.enc_heads != 96 && H / c.enc_heads != 128))
+    return fail(ctx, EV_ERR_INVALID, "text-encoder head width must be 64, 96 or 128");
   if (c.dec_head_dim != 64 || D % 32 || D > 256 || (D / 8) > 32 || c.dec_mid_blocks != 2)
     return fail(ctx, EV_ERR_INVALID, "decoder must be the (c,c) U-Net with head_dim 64, <=256 channels, 2 mid blocks");
   if ((c.enc_channels & 3) || (H & 3) || (dec_in & 7) || (c.n_feats & 7) || c.enc_kernel > kMaxTaps)
@@ -271,7 +272,7 @@ extern "C" int ev_encode(ev_ctx* ctx, const int64_t* x, const int64_t* x_lengths
     at.lens = e.xlen32; at.len_shift = 0; at.mode = 0;
     at.rope_cos = m.rope_cos; at.rope_sin = m.rope_sin; at.rope_dim = hd / 2;
     at.out = e.att; at.out_ld = H; at.out_bs = bsH;
-    // tcgen05 with split fp16 operands where the shape allows (head width 128, Tx <= 384; EV_ENC_ATTN=f32 keeps the CUDA-core
+    // tcgen05 with split fp16 operands where the shape allows (head width 96 or 128; EV_ENC_ATTN=f32 keeps the CUDA-core
     // kernel); both are fp32-accurate
     static const bool enc_attn_tc = []() { const char* v = getenv("EV_ENC_ATTN"); return !(v && std::string(v) == "f32"); }();
     const bool att_tc = enc_attn_tc && attention_enc_tc_supported(at);

@@ -212,6 +212,11 @@ EV_API int ev_test_attention(ev_ctx* ctx, const float* qkv, const int64_t* y_len
  * repeat / avg_us_host as ev_test_ff_block. */
 EV_API int ev_test_encoder_attention(ev_ctx* ctx, const float* qkv, const int64_t* x_lengths, int B, int T, int H, int impl,
                               float* out, int repeat, float* avg_us_host, void* stream);
+/* The same at head width hd (RoPE on the first hd / 2 features, scores / sqrt(hd)): qkv (B, T, 3*H*hd), out (B, T, H*hd).
+ * impl 0 takes hd = 64, 96 or 128, impl 1 hd = 96 or 128; any other pair is refused with EV_ERR_INVALID.
+ * ev_test_encoder_attention is this call with hd = 128. */
+EV_API int ev_test_encoder_attention_hd(ev_ctx* ctx, const float* qkv, const int64_t* x_lengths, int B, int T, int H, int hd,
+                                 int impl, float* out, int repeat, float* avg_us_host, void* stream);
 /* The float32 Euler times/steps of flow_matching.py:52,68-83 as the library computes them (pure host code). */
 /* Fused LayerNorm + feed-forward of one decoder transformer block (transformer.py:296-316): x (B,T,256) CHANNEL-LAST,
  * w1 (inner,256), w2 (256,inner), snake_a = exp(alpha), snake_invb = 1/(exp(beta)+1e-9); out (B,T,256) channel-last,
