@@ -64,8 +64,10 @@ def synthesise_corpus(model, vocoder, utterances, batch_size=32, n_timesteps=10,
     -> (results, stats): results maps utterance index -> dict(waveform (L,) cpu float32, mel_length, [mel]), stats is a
     sharding.ShardStats with this rank's device time.  `z_fn(mb, model, x, x_lengths, spks)` may supply the prior noise per
     micro-batch (parity runs share it with the oracle).  ragged: the vocoder skips the time tiles past each utterance's own length
-    (identical cropped waveforms, see Generator.__call__); ignored with a denoiser, whose STFT windows at an utterance's
-    end reach into the padded region.  cuda_graphs: a corpus hardly ever repeats a (B, Tx, T_pad) shape, so by default the
+    (identical cropped waveforms, see Generator.__call__); with a denoiser, vocoder and denoiser run as one ragged call that
+    vocodes 4 frames past each end, which the denoiser's STFT windows reach, and transforms only each utterance's own frames
+    (identical cropped waveforms, see Generator.vocode_denoised; a denoiser built on another generator than `vocoder` runs
+    the dense path).  ragged=False vocodes and denoises the whole padded batch.  cuda_graphs: a corpus hardly ever repeats a (B, Tx, T_pad) shape, so by default the
     stages are launched eagerly -- measured within 2 % of a graph replay (the host enqueues a step in 5 ms of the GPU's 29),
     whereas capturing costs ~250 ms per new shape (profiles/r02_host_cost.txt); True restores capture-on-second-sight.
     in_flight / lanes: micro-batches in flight at once (see `Lanes`; `lanes` passes a prebuilt set, else `lanes_for` builds and
@@ -121,10 +123,13 @@ def synthesise_corpus(model, vocoder, utterances, batch_size=32, n_timesteps=10,
                 if z_fn is not None:
                     kw["z"] = z_fn(mb, m, x, xl, spks)
                 out = m.synthesise(x, xl, n_timesteps, temperature, spks if m.n_spks > 1 else None, length_scale, **kw)
-                use_ragged = ragged and denoiser is None
-                wav = v(out["mel"], lengths=out["mel_lengths"] if use_ragged else None).clamp(-1, 1)   # to_waveform, cli.py:121-126
-                if denoiser is not None:
-                    wav = lanes.denoiser(lane, denoiser)(wav.squeeze(1), strength=denoiser_strength).unsqueeze(1)
+                d = lanes.denoiser(lane, denoiser)
+                if ragged and d is not None and d.vocoder is v:
+                    wav = v.vocode_denoised(out["mel"], out["mel_lengths"], denoiser_strength)
+                else:
+                    wav = v(out["mel"], lengths=out["mel_lengths"] if ragged and d is None else None).clamp(-1, 1)   # to_waveform, cli.py:121-126
+                    if d is not None:
+                        wav = d(wav.squeeze(1), strength=denoiser_strength).unsqueeze(1)
                 e1.record()
                 # read-back on a copy stream into pinned memory (the `.cpu()` of to_waveform): the host crops an EARLIER micro-batch
                 # while this one's copy -- and the next ones' kernels -- are in flight

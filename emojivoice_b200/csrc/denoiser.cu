@@ -83,12 +83,14 @@ __global__ void spectral_subtract_kernel(float* __restrict__ spec, int frames, c
   }
 }
 
-// torch.istft: overlap-add of the windowed frames divided by the overlap-added squared window, centre padding trimmed
+// torch.istft: overlap-add of the windowed frames divided by the overlap-added squared window, centre padding trimmed.
+// lens (ragged batch, or nullptr): item b is written on [0, lens[b] * HOP) and zero beyond, where its frames were not computed
 __global__ void overlap_add_kernel(const float* __restrict__ y, int frames, const float* __restrict__ win_sq, int L_out,
-                                   float* __restrict__ out) {
+                                   const int* __restrict__ lens, float* __restrict__ out) {
   const int b = blockIdx.y;
   const int t = blockIdx.x * blockDim.x + threadIdx.x;
   if (t >= L_out) return;
+  if (lens && t >= __ldg(lens + b) * HOP) { out[(long long)b * L_out + t] = 0.0f; return; }
   const int tt = t + NFFT / 2;
   int f_lo = (tt - (NFFT - 1) + HOP - 1) / HOP;
   if (f_lo < 0) f_lo = 0;
@@ -144,13 +146,24 @@ __device__ __forceinline__ float2* fft1024(float2* a, float2* b, const float2* t
   return b;
 }
 
-// grid (ceil(frames / 2), B), 256 threads.  audio (B, L); y (B, frames, 1024) windowed inverse frames (bias != nullptr);
-// mag0_out (B, 513): magnitude of frame 0 (the bias spectrum of ev_denoiser_init)
-__global__ void __launch_bounds__(256) denoise_fft_kernel(const float* __restrict__ audio, int L, int frames, const float2* __restrict__ tw,
+// One block per pair of frames (f0, f0 + 1), f0 even, 256 threads.  audio (B, L); y (B, frames, 1024) windowed inverse frames
+// (bias != nullptr); mag0_out (B, 513): magnitude of frame 0 (the bias spectrum of ev_denoiser_init).
+//   RAGGED = false: grid (ceil(frames / 2), B), every pair of every item.
+//   RAGGED = true: grid B * ceil(frames / 2), block i computes entry i of the compact (item, pair) list of ragged_build_table
+//   (pairs[0] = its length, pairs[1 + i] = b << 16 | pair index) and blocks past its end exit.
+// Both variants run the same per-pair code, so a pair's result does not depend on which of them computed it.
+template <bool RAGGED>
+__global__ void __launch_bounds__(256, RAGGED ? 3 : 0) denoise_fft_kernel(const float* __restrict__ audio, int L, int frames, const float2* __restrict__ tw,
                                                           const float* __restrict__ bias, float strength, float* __restrict__ y,
-                                                          float* __restrict__ mag0_out) {
+                                                          float* __restrict__ mag0_out, const int* __restrict__ pairs) {
   __shared__ float2 buf0[NFFT], buf1[NFFT];
-  const int b = blockIdx.y, f0 = blockIdx.x * 2, f1 = f0 + 1, j = threadIdx.x;
+  int b = blockIdx.y, f0 = blockIdx.x * 2;
+  if (RAGGED) {
+    if ((int)blockIdx.x >= __ldg(pairs)) return;
+    const int e = __ldg(pairs + 1 + blockIdx.x);
+    b = e >> 16; f0 = (e & 0xffff) * 2;
+  }
+  const int f1 = f0 + 1, j = threadIdx.x;
   const float* xb = audio + (long long)b * L;
   const bool has1 = f1 < frames;
   float win[4];
@@ -201,6 +214,16 @@ __global__ void __launch_bounds__(256) denoise_fft_kernel(const float* __restric
   }
 }
 
+// lens32[b] = clamp(lengths[b], 0, max_len); wide (optional) = min(lens32[b] + extra, max_len) as int64
+__global__ void ragged_lengths_kernel(const long long* __restrict__ lengths, int B, int max_len, int extra, int* __restrict__ lens32,
+                                      long long* __restrict__ wide) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  const int n = (int)min(max(lengths[b], 0LL), (long long)max_len);
+  lens32[b] = n;
+  if (wide) wide[b] = min(n + extra, max_len);
+}
+
 int ensure_basis(ev_ctx* ctx, cudaStream_t s) {
   DenoiseBasis& d = ctx->hifigan.dn;
   if (d.ready) return 0;
@@ -226,7 +249,7 @@ int ensure_basis(ev_ctx* ctx, cudaStream_t s) {
   return 0;
 }
 
-struct DnBuffers { float* padded; float* spec; float* frames_t; long long pad_ld; int frames; };
+struct DnBuffers { float* padded; float* spec; float* frames_t; int* lens32; int* pairs; long long pad_ld; int frames; };
 
 void plan(int B, int L, Workspace& w, DnBuffers* d) {
   d->frames = L / HOP + 1;
@@ -234,23 +257,48 @@ void plan(int B, int L, Workspace& w, DnBuffers* d) {
   d->padded = w.take<float>((size_t)B * d->pad_ld);
   d->spec = w.take<float>((size_t)B * d->frames * SPEC_LD);
   d->frames_t = w.take<float>((size_t)B * d->frames * NFFT);
+  d->lens32 = w.take<int>((size_t)B);                           // ragged batch: lengths and the compact pair list
+  d->pairs = w.take<int>((size_t)B * ceil_div(d->frames, 2) + 1);
 }
 
-// STFT of `audio` (B, L) into d.spec (re|im); when bias != nullptr also denoise + ISTFT into out (B, HOP*(L/HOP))
+// Mel frames past len_b that the denoised samples [0, len_b * HOP) depend on (DESIGN.md §4, ragged batches): sample t < len*HOP
+// is an overlap-add of frames f <= len + 1; frame f shares its FFT with its pair partner, so pairs (f0, f0 + 1), f0 <= len + 1,
+// are computed, and their windows read audio below (len + 2) * HOP + NFFT / 2 = (len + 4) * HOP.
+constexpr int kDenoiseReach = 4;
+
+// STFT of `audio` (B, L) into d.spec (re|im); when bias != nullptr also denoise + ISTFT into out (B, HOP*(L/HOP)).
+// lens32 (ragged batch, bias != nullptr, or nullptr): only the pairs that item b's samples [0, lens32[b] * HOP) read are
+// computed, and out is zero beyond; what is written equals the dense result bit for bit.
 int stft_pipeline(ev_ctx* ctx, const float* audio, int B, int L, const float* bias, float strength, float* mag0, float* out,
-                  DnBuffers& d, cudaStream_t s) {
+                  const int* lens32, DnBuffers& d, cudaStream_t s) {
   DenoiseBasis& bs = ctx->hifigan.dn;
   const int frames = d.frames;
   static const bool use_fft = []() { const char* v = getenv("EV_DN_FFT"); return !(v && atoi(v) == 0); }();
-  if (use_fft) {
-    const double fft_flops = 2.0 * 5.0 * NFFT * 10.0 * ceil_div(frames, 2) * B;
+  const double pair_flops = 2.0 * 5.0 * NFFT * 10.0;
+  if (use_fft && lens32 && bias) {
+    // frames [0, lens32[b] + 2) in pairs: ceil((len + 2) / 2) = floor((len + 1) / 2) + 1 pairs, all of them when len = frames - 1
+    EV_LAUNCH(ctx, s, "ragged_table", 0, 8.0 * B, ragged_build_table(lens32, B, kDenoiseReach - 2, 1, 0, 2, frames, d.pairs, s));
+    double n_pairs = (double)B * ceil_div(frames, 2);
+    if (ctx->profiling) {   // algorithmic work = the listed pairs (instrumented eager run: a host copy is fine here)
+      int n = 0;
+      EV_CUDA(ctx, cudaMemcpyAsync(&n, d.pairs, sizeof(int), cudaMemcpyDeviceToHost, s));
+      EV_CUDA(ctx, cudaStreamSynchronize(s));
+      n_pairs = n;
+    }
+    EV_LAUNCH(ctx, s, "denoise_fft_ragged", pair_flops * n_pairs, 4.0 * n_pairs * 2.0 * (HOP + NFFT),
+              (denoise_fft_kernel<true><<<B * ceil_div(frames, 2), 256, 0, s>>>(audio, L, frames, reinterpret_cast<const float2*>(bs.twiddle), bias,
+                                                                                strength, d.frames_t, nullptr, d.pairs), cudaGetLastError()));
+  } else if (use_fft) {
+    const double fft_flops = pair_flops * ceil_div(frames, 2) * B;
     EV_LAUNCH(ctx, s, "denoise_fft", fft_flops, 4.0 * B * ((double)L + (bias ? (double)frames * NFFT : NBIN)),
-              (denoise_fft_kernel<<<dim3(ceil_div(frames, 2), B), 256, 0, s>>>(audio, L, frames, reinterpret_cast<const float2*>(bs.twiddle), bias,
-                                                                              strength, d.frames_t, mag0), cudaGetLastError()));
+              (denoise_fft_kernel<false><<<dim3(ceil_div(frames, 2), B), 256, 0, s>>>(audio, L, frames, reinterpret_cast<const float2*>(bs.twiddle), bias,
+                                                                                     strength, d.frames_t, mag0, nullptr), cudaGetLastError()));
+  }
+  if (use_fft) {
     if (!bias) return 0;
     const int L_out = HOP * (frames - 1);
     EV_LAUNCH(ctx, s, "overlap_add", 0, 4.0 * B * (4.0 * L_out + L_out),
-              (overlap_add_kernel<<<dim3(ceil_div(L_out, 256), B), 256, 0, s>>>(d.frames_t, frames, bs.win_sq, L_out, out), cudaGetLastError()));
+              (overlap_add_kernel<<<dim3(ceil_div(L_out, 256), B), 256, 0, s>>>(d.frames_t, frames, bs.win_sq, L_out, lens32, out), cudaGetLastError()));
     return 0;
   }
   EV_LAUNCH(ctx, s, "reflect_pad", 0, 8.0 * B * d.pad_ld,
@@ -278,9 +326,22 @@ int stft_pipeline(ev_ctx* ctx, const float* audio, int B, int L, const float* bi
     if (ce != cudaSuccess) return cuda_fail(ctx, ce, "istft gemm"); }
   const int L_out = HOP * (frames - 1);
   EV_LAUNCH(ctx, s, "overlap_add", 0, 4.0 * B * (4.0 * L_out + L_out),
-            (overlap_add_kernel<<<dim3(ceil_div(L_out, 256), B), 256, 0, s>>>(d.frames_t, frames, bs.win_sq, L_out, out), cudaGetLastError()));
+            (overlap_add_kernel<<<dim3(ceil_div(L_out, 256), B), 256, 0, s>>>(d.frames_t, frames, bs.win_sq, L_out, lens32, out), cudaGetLastError()));
   return 0;
 }
+
+// ev_to_waveform_ragged's workspace: widened lengths, the vocoded batch, the denoiser's buffers, the vocoder's workspace
+struct WavBuffers { long long* wide; float* audio; DnBuffers d; char* voc_ws; size_t voc_bytes; };
+
+void plan_to_waveform(const ev_ctx* ctx, int B, int T, Workspace& w, WavBuffers* t) {
+  t->wide = w.take<long long>((size_t)B);
+  t->audio = w.take<float>((size_t)B * T * HOP);
+  plan(B, T * HOP, w, &t->d);
+  t->voc_bytes = ev_vocode_workspace_bytes(ctx, B, T);
+  t->voc_ws = w.take<char>(t->voc_bytes);
+}
+
+bool ragged_lists_fit(int B, int frames) { return B <= kRaggedMaxB && ceil_div(frames, 2) < 65536; }
 }  // namespace
 
 extern "C" size_t ev_denoise_workspace_bytes(const ev_ctx* ctx, int B, int L) {
@@ -314,16 +375,17 @@ extern "C" int ev_denoiser_init(ev_ctx* ctx, float* bias_spec_out, void* workspa
   }
   EV_CUDA(ctx, cudaMemsetAsync(mel, 0, (size_t)h.cfg.num_mels * T * sizeof(float), s));
   EV_TRY(ev_vocode(ctx, mel, 1, T, EV_PREC_FP32, wav, voc_ws, voc_bytes, stream));
-  EV_TRY(stft_pipeline(ctx, wav, 1, L, nullptr, 0.0f, h.denoise_bias, nullptr, d, s));   // bias_spec[:, :, 0]
+  EV_TRY(stft_pipeline(ctx, wav, 1, L, nullptr, 0.0f, h.denoise_bias, nullptr, nullptr, d, s));   // bias_spec[:, :, 0]
   if (bias_spec_out) EV_CUDA(ctx, cudaMemcpyAsync(bias_spec_out, h.denoise_bias, NBIN * sizeof(float), cudaMemcpyDeviceToDevice, s));
   return 0;
 }
 
-extern "C" int ev_denoise(ev_ctx* ctx, const float* audio, int B, int L, float strength, float* out, void* workspace,
-                          size_t workspace_bytes, void* stream) {
+extern "C" int ev_denoise_ragged(ev_ctx* ctx, const float* audio, const int64_t* lengths, int B, int L, float strength, float* out,
+                                 void* workspace, size_t workspace_bytes, void* stream) {
   if (!ctx) return EV_ERR_INVALID;
   if (!ctx->hifigan.denoise_bias) return fail(ctx, EV_ERR_STATE, "ev_denoise: call ev_denoiser_init first");
   if (!audio || !out || B <= 0 || L < NFFT / 2 + 1) return fail(ctx, EV_ERR_INVALID, "ev_denoise: null argument or audio shorter than the reflect padding");
+  if (lengths && !ragged_lists_fit(B, L / HOP + 1)) return fail(ctx, EV_ERR_INVALID, "ev_denoise_ragged: batch or audio too long for the ragged pair list");
   cudaStream_t s = as_stream(stream);
   EV_CUDA(ctx, cudaSetDevice(ctx->device));
   EV_TRY(ensure_basis(ctx, s));
@@ -331,5 +393,48 @@ extern "C" int ev_denoise(ev_ctx* ctx, const float* audio, int B, int L, float s
   DnBuffers d;
   plan(B, L, w, &d);
   if (w.overflow || !workspace) return fail(ctx, EV_ERR_STATE, "ev_denoise: workspace too small");
-  return stft_pipeline(ctx, audio, B, L, ctx->hifigan.denoise_bias, strength, nullptr, out, d, s);
+  if (lengths)
+    EV_LAUNCH(ctx, s, "ragged_lengths", 0, 12.0 * B,
+              (ragged_lengths_kernel<<<ceil_div(B, 256), 256, 0, s>>>(reinterpret_cast<const long long*>(lengths), B, L / HOP, 0, d.lens32, nullptr),
+               cudaGetLastError()));
+  return stft_pipeline(ctx, audio, B, L, ctx->hifigan.denoise_bias, strength, nullptr, out, lengths ? d.lens32 : nullptr, d, s);
+}
+
+extern "C" int ev_denoise(ev_ctx* ctx, const float* audio, int B, int L, float strength, float* out, void* workspace,
+                          size_t workspace_bytes, void* stream) {
+  return ev_denoise_ragged(ctx, audio, nullptr, B, L, strength, out, workspace, workspace_bytes, stream);
+}
+
+extern "C" size_t ev_to_waveform_ragged_workspace_bytes(const ev_ctx* ctx, int B, int T) {
+  if (!ctx || !ctx->hifigan.loaded || B <= 0 || T <= 0) return 0;
+  Workspace w(nullptr, 0);
+  WavBuffers t;
+  plan_to_waveform(ctx, B, T, w, &t);
+  return w.off + 256;
+}
+
+extern "C" int ev_to_waveform_ragged(ev_ctx* ctx, const float* mel, const int64_t* mel_lengths, int B, int T, int precision, float strength,
+                                     float* wav, void* workspace, size_t workspace_bytes, void* stream) {
+  if (!ctx) return EV_ERR_INVALID;
+  const HifiganW& h = ctx->hifigan;
+  if (!h.loaded) return fail(ctx, EV_ERR_STATE, "ev_to_waveform_ragged: hifigan weights not loaded");
+  if (!h.denoise_bias) return fail(ctx, EV_ERR_STATE, "ev_to_waveform_ragged: call ev_denoiser_init first");
+  if (!mel || !mel_lengths || !wav || B <= 0 || T <= 0) return fail(ctx, EV_ERR_INVALID, "ev_to_waveform_ragged: null argument or empty shape");
+  if (h.total_up != HOP) return fail(ctx, EV_ERR_INVALID, "ev_to_waveform_ragged: the generator's hop must equal the denoiser's (256)");
+  if (T * HOP < NFFT / 2 + 1) return fail(ctx, EV_ERR_INVALID, "ev_to_waveform_ragged: T < 3 frames is shorter than the reflect padding");
+  if (!ragged_lists_fit(B, T + 1)) return fail(ctx, EV_ERR_INVALID, "ev_to_waveform_ragged: batch or T too large for the ragged pair list");
+  if (precision != EV_PREC_FP32 && precision != EV_PREC_BF16) return fail(ctx, EV_ERR_INVALID, "ev_to_waveform_ragged: unknown precision");
+  cudaStream_t s = as_stream(stream);
+  EV_CUDA(ctx, cudaSetDevice(ctx->device));
+  EV_TRY(ensure_basis(ctx, s));
+  Workspace w(workspace, workspace_bytes);
+  WavBuffers t;
+  plan_to_waveform(ctx, B, T, w, &t);
+  if (w.overflow || !workspace) return fail(ctx, EV_ERR_STATE, "ev_to_waveform_ragged: workspace too small");
+  // the vocoder is exact on [0, min(len + reach, T) * HOP), which holds every sample the denoised [0, len * HOP) reads
+  EV_LAUNCH(ctx, s, "ragged_lengths", 0, 20.0 * B,
+            (ragged_lengths_kernel<<<ceil_div(B, 256), 256, 0, s>>>(reinterpret_cast<const long long*>(mel_lengths), B, T, kDenoiseReach,
+                                                                     t.d.lens32, t.wide), cudaGetLastError()));
+  EV_TRY(ev_vocode_ragged(ctx, mel, reinterpret_cast<const int64_t*>(t.wide), B, T, precision, t.audio, t.voc_ws, t.voc_bytes, stream));
+  return stft_pipeline(ctx, t.audio, B, T * HOP, h.denoise_bias, strength, nullptr, wav, t.d.lens32, t.d, s);
 }

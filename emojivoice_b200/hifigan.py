@@ -95,26 +95,51 @@ class Generator:
         waveform of item b is then bit-identical on [: lengths[b]*hop] -- all the reference's batched caller keeps
         (cli.py:307-311) -- and zero beyond; time tiles further than the generator's receptive field past an utterance's
         end are never computed (ev_vocode_ragged)."""
+        return self._run(mel, dtype, lengths, None)
+
+    forward = __call__
+
+    @torch.inference_mode()
+    def vocode_denoised(self, mel, lengths, strength=0.00025, dtype=None):
+        """The batched reply path in one call: `Denoiser(self)(self(mel).clamp(-1, 1).squeeze(1), strength)` followed by the
+        per-utterance crop `[: lengths[b]*hop]` (feel_me.py:181-187, cli.py:300,307-311) -> wav (B, 1, T*hop).
+
+        wav[b] is bit-identical to that dense path on [: lengths[b]*hop] and zero beyond: the generator runs ragged on
+        lengths[b] + 4 frames (all the denoised samples read) and the denoiser transforms only the STFT frames of each
+        utterance's own samples (ev_to_waveform_ragged).  A Denoiser built on this generator must exist (it holds the bias
+        spectrum).  lengths (B,) valid mel frames per item; lengths given on the host must lie in [1, T] (device tensors are
+        clamped to [0, T] on the device, as checking them would synchronise)."""
+        return self._run(mel, dtype, lengths, float(strength))
+
+    def _run(self, mel, dtype, lengths, strength):
+        """ev_vocode_ragged (strength None) or ev_to_waveform_ragged, replayed as a CUDA graph once a call shape repeats."""
         self._materialise()
         ctx, L = self._ctx, _lib.lib()
         dev = ctx.device
+        denoise = strength is not None
         if mel.dim() == 2:
             mel = mel.unsqueeze(0)
         with torch.cuda.device(dev):
             mel = mel.to(device=dev, dtype=torch.float32).contiguous()
             B, _, T = mel.shape
             prec = _lib.PREC[dtype if dtype is not None else self.precision]
-            nb = L.ev_vocode_workspace_bytes(ctx.handle, B, T)
+            nb = (L.ev_to_waveform_ragged_workspace_bytes if denoise else L.ev_vocode_workspace_bytes)(ctx.handle, B, T)
+            if denoise:
+                check_lengths(lengths, T)
             if lengths is not None:
                 lengths = torch.as_tensor(lengths).reshape(-1).to(device=dev, dtype=torch.int64).contiguous()
                 if lengths.numel() != B:
                     raise ValueError(f"lengths has {lengths.numel()} entries for a batch of {B}")
 
             def call(mel_, wav_, ws_, len_=None):
+                if denoise:
+                    ctx.check(L.ev_to_waveform_ragged(ctx.handle, _lib.ptr(mel_), _lib.ptr(len_), B, T, prec, strength, _lib.ptr(wav_),
+                                                      _lib.ptr(ws_), ws_.numel(), _lib.stream_ptr()), "ev_to_waveform_ragged")
+                    return
                 ctx.check(L.ev_vocode_ragged(ctx.handle, _lib.ptr(mel_), _lib.ptr(len_) if len_ is not None else None, B, T, prec,
                                              _lib.ptr(wav_), _lib.ptr(ws_), ws_.numel(), _lib.stream_ptr()), "ev_vocode")
 
-            key = (B, T, prec, lengths is not None)
+            key = (B, T, prec, lengths is not None) + ((strength,) if denoise else ())
             ws_shared = ctx.workspace(nb)                   # (may grow the workspace: do it before looking graphs up)
             ent = self._graphs.get(key, ctx.ws_version) if self.cuda_graphs else None
             if ent is None and self.cuda_graphs and self._graphs.should_capture(key):
@@ -134,14 +159,23 @@ class Generator:
                 wav = ent["wav"].clone()
         return wav
 
-    forward = __call__
-
     def launch_count(self, reset=False):
         """Kernels launched by this generator's context, graph replays included."""
         n = self._ctx.launch_count(reset) + self._replayed_launches
         if reset:
             self._replayed_launches = 0
         return n
+
+
+def check_lengths(lengths, max_len):
+    """Lengths the caller holds on the host must lie in [1, max_len]; a CUDA tensor is not read back (that would synchronise)."""
+    if lengths is None:
+        raise ValueError("lengths are required")
+    if isinstance(lengths, torch.Tensor) and lengths.is_cuda:
+        return
+    t = torch.as_tensor(lengths).reshape(-1)
+    if t.numel() and (int(t.min()) < 1 or int(t.max()) > max_len):
+        raise ValueError(f"lengths must lie in [1, {max_len}] frames, got [{int(t.min())}, {int(t.max())}]")
 
 
 class Denoiser:
@@ -164,16 +198,24 @@ class Denoiser:
                       "ev_denoiser_init")
 
     @torch.inference_mode()
-    def __call__(self, audio, strength=0.0005):
+    def __call__(self, audio, strength=0.0005, lengths=None):
+        """lengths (B,) optional: valid mel frames per item of a padded batch, as `mel_lengths`.  Item b is then bit-identical
+        to the call without lengths on [: lengths[b]*256] and zero beyond, and only the STFT frames those samples reach are
+        transformed (ev_denoise_ragged).  Lengths given on the host must lie in [1, n // 256]."""
         ctx, L = self.vocoder._ctx, _lib.lib()
         squeeze = audio.dim() == 1
         a = audio.reshape(-1, audio.shape[-1]).to(device=self.device, dtype=torch.float32).contiguous()
         B, n = a.shape
         out = torch.empty(B, (n // 256) * 256, device=self.device)
         with torch.cuda.device(self.device):
+            if lengths is not None:
+                check_lengths(lengths, n // 256)
+                lengths = torch.as_tensor(lengths).reshape(-1).to(device=self.device, dtype=torch.int64).contiguous()
+                if lengths.numel() != B:
+                    raise ValueError(f"lengths has {lengths.numel()} entries for a batch of {B}")
             ws = ctx.workspace(L.ev_denoise_workspace_bytes(ctx.handle, B, n))
-            ctx.check(L.ev_denoise(ctx.handle, _lib.ptr(a), B, n, float(strength), _lib.ptr(out), _lib.ptr(ws), ws.numel(),
-                                   _lib.stream_ptr()), "ev_denoise")
+            ctx.check(L.ev_denoise_ragged(ctx.handle, _lib.ptr(a), _lib.ptr(lengths), B, n, float(strength), _lib.ptr(out), _lib.ptr(ws),
+                                          ws.numel(), _lib.stream_ptr()), "ev_denoise")
         return out[0] if squeeze else out
 
     forward = __call__
@@ -183,7 +225,9 @@ class Denoiser:
 def to_waveform(mel, vocoder, denoiser=None, strength=0.00025, lengths=None):
     """feel_me.py:181-187: vocoder(mel).clamp(-1, 1) -> optional denoiser -> .cpu().squeeze().
 
-    lengths: optional valid frames per item of a padded batch (see Generator.__call__)."""
+    lengths: optional valid frames per item of a padded batch (see Generator.__call__).  With a denoiser, the denoiser still
+    transforms the whole padded waveform here (the ragged vocoder leaves zeros past each utterance's end, so the last samples
+    differ from the dense path); `vocoder.vocode_denoised` is the padded batch's exact form."""
     audio = (vocoder(mel, lengths=lengths) if lengths is not None else vocoder(mel)).clamp(-1, 1)
     if denoiser is not None:
         audio = denoiser(audio.squeeze(1), strength=strength)

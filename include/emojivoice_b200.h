@@ -146,6 +146,25 @@ EV_API size_t ev_denoise_workspace_bytes(const ev_ctx* ctx, int B, int L);
 EV_API int ev_denoiser_init(ev_ctx* ctx, float* bias_spec_out, void* workspace, size_t workspace_bytes, void* stream);
 EV_API int ev_denoise(ev_ctx* ctx, const float* audio, int B, int L, float strength, float* out, void* workspace,
                size_t workspace_bytes, void* stream);
+/* Ragged batch: the same denoiser for a padded batch whose item b holds lengths[b] valid mel frames (device int64, samples
+ * [0, lengths[b]*256); NULL = ev_denoise).  out[b] is bit-identical to ev_denoise's on [0, lengths[b]*256) and ZERO beyond.
+ * Only the STFT frames those samples reach are transformed: frames f <= lengths[b] + 1, computed in pairs (f0, f0 + 1), f0
+ * even, so at most floor((lengths[b] + 1) / 2) + 1 pairs per item.  Lengths are clamped to [0, L/256] on the device (a value
+ * there cannot be checked without a host synchronisation).  Uses ev_denoise_workspace_bytes; B <= 2048. */
+EV_API int ev_denoise_ragged(ev_ctx* ctx, const float* audio, const int64_t* lengths, int B, int L, float strength, float* out,
+              void* workspace, size_t workspace_bytes, void* stream);
+
+/* ---- vocoder + denoiser on a padded batch -------------------------------------------------------------------
+ * Replaces the reference's reply path  audio = vocoder(mel).clamp(-1, 1); audio = denoiser(audio, strength)  (feel_me.py:181-187)
+ * in the batched form of Matcha-TTS/matcha/cli.py:300,307-311, which then crops each waveform to [: length * 256].
+ *   mel (B,num_mels,T), mel_lengths (B) device int64 (synthesise's mel_lengths) -> wav (B,1,T*256).
+ * wav[b] is bit-identical to "ev_vocode, then ev_denoise" on [0, mel_lengths[b]*256) and ZERO beyond.  The generator runs as
+ * ev_vocode_ragged on min(mel_lengths[b] + 4, T) frames (the denoised samples read no audio at or past (len + 4) * 256) and
+ * the denoiser as ev_denoise_ragged on mel_lengths[b].  Needs ev_denoiser_init (EV_ERR_STATE before it); lengths are clamped
+ * to [0, T] on the device; T >= 3, B <= 2048, a generator hop of 256.  No host synchronisation: capturable in a CUDA graph. */
+EV_API size_t ev_to_waveform_ragged_workspace_bytes(const ev_ctx* ctx, int B, int T);
+EV_API int ev_to_waveform_ragged(ev_ctx* ctx, const float* mel, const int64_t* mel_lengths, int B, int T, int precision,
+              float strength, float* wav, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- monotonic alignment search (SURVEY 8 f4; training-side, the reference's only native component) ------------
  * replaces  maximum_path_c(paths, values, t_xs, t_ys, max_neg_val)   Matcha-TTS/matcha/utils/monotonic_align/core.pyx:42-47
