@@ -61,10 +61,13 @@ SIGNATURES = {
     "ev_load_hifigan": (_I, [_P, C.POINTER(EvTensor), _I, C.POINTER(EvHifiganCfg), _P]),
     "ev_encode_workspace_bytes": (_SZ, [_P, _I, _I]),
     "ev_encode": (_I, [_P, _P, _P, _P, _I, _I, _F, _P, _P, _P, _P, _P, _P, _P, _SZ, _P]),
+    "ev_encode_items": (_I, [_P, _P, _P, _P, _I, _I, _P, _P, _P, _P, _P, _P, _P, _P, _SZ, _P]),
     "ev_align_workspace_bytes": (_SZ, [_P, _I, _I, _I]),
     "ev_align": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _P, _P, _P, _P, _SZ, _P]),
     "ev_decode_workspace_bytes": (_SZ, [_P, _I, _I, _I]),
     "ev_decode": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _F, _I, _P, _P, _P, _SZ, _P]),
+    "ev_decode_items_workspace_bytes": (_SZ, [_P, _I, _I, _I]),
+    "ev_decode_items": (_I, [_P, _P, _P, _P, _P, _I, _I, _P, _P, _I, _P, _P, _P, _SZ, _P]),
     "ev_vocode_workspace_bytes": (_SZ, [_P, _I, _I]),
     "ev_vocode": (_I, [_P, _P, _I, _I, _I, _P, _P, _SZ, _P]),
     "ev_vocode_ragged": (_I, [_P, _P, _P, _I, _I, _I, _P, _P, _SZ, _P]),
@@ -96,6 +99,7 @@ SIGNATURES = {
     "ev_test_resnet_trace": (_I, [_P, _P, _I]),
     "ev_test_vocoder_margins": (_I, [C.POINTER(EvHifiganCfg), C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "ev_test_euler_schedule": (_I, [_I, C.POINTER(_F), C.POINTER(_F)]),
+    "ev_test_euler_tables": (_I, [C.POINTER(C.c_int32), _I, C.POINTER(_F), C.POINTER(_F)]),
     "ev_test_row_sum": (_I, [_P, _P, _I, _I, _P, _P]),
     "ev_test_conv_trace": (_I, [_P, _P, _I]),
     "ev_test_ff_trace": (_I, [_P, _P, _I]),

@@ -8,8 +8,11 @@ import torch
 from . import sharding
 
 
+SETTINGS = ("length_scale", "temperature", "n_timesteps")
+
+
 def collate(utterances, items):
-    """cli.py:109-120 batched_collate_fn: right-pad the id sequences with 0.  utterances[i] = (ids, speaker_id)."""
+    """cli.py:109-120 batched_collate_fn: right-pad the id sequences with 0.  utterances[i] = (ids, speaker_id[, settings])."""
     seqs = [torch.as_tensor(utterances[i][0], dtype=torch.long).reshape(-1) for i in items]
     x = torch.nn.utils.rnn.pad_sequence(seqs, batch_first=True)
     x_lengths = torch.tensor([s.numel() for s in seqs], dtype=torch.long)
@@ -55,11 +58,31 @@ def lanes_for(model, vocoder, n: int) -> Lanes:
     return cache[-1]
 
 
+def utterance_settings(utterances, defaults):
+    """Each utterance's (length_scale, temperature, n_timesteps): an utterance is (ids, speaker_id) or (ids, speaker_id,
+    settings) with a dict holding any of those keys; a missing key takes its value from `defaults`.
+    -> (per-utterance dicts, True when some utterance has its own settings)"""
+    out, own = [], False
+    for u in utterances:
+        s = dict(defaults)
+        if len(u) > 2 and u[2]:
+            extra = set(u[2]) - set(SETTINGS)
+            if extra:
+                raise ValueError(f"unknown per-utterance settings {sorted(extra)}; expected keys among {SETTINGS}")
+            s.update(u[2])
+            own = True
+        out.append(s)
+    return out, own
+
+
 @torch.inference_mode()
 def synthesise_corpus(model, vocoder, utterances, batch_size=32, n_timesteps=10, temperature=0.667, length_scale=1.0,
                       rank=0, world_size=1, denoiser=None, denoiser_strength=0.00025, sort=True, keep_mel=False, z_fn=None,
                       ragged=True, cuda_graphs=False, in_flight=1, lanes=None):
-    """Synthesise this rank's share of `utterances` (list of (phoneme ids, speaker id)).
+    """Synthesise this rank's share of `utterances`: a list of (phoneme ids, speaker id) or (phoneme ids, speaker id, settings),
+    where settings is a dict with any of "length_scale", "temperature", "n_timesteps" for that utterance (a missing key takes
+    the keyword's value).  Utterances with different settings share micro-batches (MatchaTTS.synthesise with per-utterance
+    values); the micro-batch plan does not depend on them, only its cost estimate uses each utterance's own step count.
 
     -> (results, stats): results maps utterance index -> dict(waveform (L,) cpu float32, mel_length, [mel]), stats is a
     sharding.ShardStats with this rank's device time.  `z_fn(mb, model, x, x_lengths, spks)` may supply the prior noise per
@@ -74,7 +97,9 @@ def synthesise_corpus(model, vocoder, utterances, batch_size=32, n_timesteps=10,
     caches one); the waveforms do not depend on it.  stats.seconds is the sum of the micro-batches' device times for one
     lane and the device span from the first launch to the last kernel's end for several."""
     lens = [len(u[0]) for u in utterances]
-    plan = sharding.shard(lens, batch_size, rank, world_size, n_timesteps=n_timesteps, sort=sort)
+    settings, own = utterance_settings(utterances, dict(length_scale=length_scale, temperature=temperature, n_timesteps=n_timesteps))
+    steps = [int(s["n_timesteps"]) for s in settings] if own else n_timesteps
+    plan = sharding.shard(lens, batch_size, rank, world_size, n_timesteps=steps, sort=sort)
     results, stats = {}, sharding.ShardStats()
     if lanes is None:
         lanes = lanes_for(model, vocoder, in_flight)
@@ -88,7 +113,8 @@ def synthesise_corpus(model, vocoder, utterances, batch_size=32, n_timesteps=10,
     def finish(p):
         p["done"].synchronize()
         mel_len = p["len_host"].tolist()
-        stats.add(mel_len, p["xl"], n_timesteps, p["e0"].elapsed_time(p["e1"]) / 1e3 if n_lanes == 1 else 0.0)
+        stats.add(mel_len, p["xl"], [steps[i] for i in p["items"]] if own else n_timesteps,
+                  p["e0"].elapsed_time(p["e1"]) / 1e3 if n_lanes == 1 else 0.0)
         for j, i in enumerate(p["items"]):
             n = int(mel_len[j])
             rec = {"waveform": p["wav_host"][j, 0, : n * 256].clone(), "mel_length": n}     # cli.py:308-309 crop
@@ -122,7 +148,11 @@ def synthesise_corpus(model, vocoder, utterances, batch_size=32, n_timesteps=10,
                 kw = {}
                 if z_fn is not None:
                     kw["z"] = z_fn(mb, m, x, xl, spks)
-                out = m.synthesise(x, xl, n_timesteps, temperature, spks if m.n_spks > 1 else None, length_scale, **kw)
+                if own:      # one value per utterance of the micro-batch
+                    n_b, temp_b, ls_b = ([settings[i][k] for i in mb.items] for k in ("n_timesteps", "temperature", "length_scale"))
+                else:
+                    n_b, temp_b, ls_b = n_timesteps, temperature, length_scale
+                out = m.synthesise(x, xl, n_b, temp_b, spks if m.n_spks > 1 else None, ls_b, **kw)
                 d = lanes.denoiser(lane, denoiser)
                 if ragged and d is not None and d.vocoder is v:
                     wav = v.vocode_denoised(out["mel"], out["mel_lengths"], denoiser_strength)

@@ -6,12 +6,14 @@
 namespace ev {
 namespace {
 
-// one thread per utterance: the row is short (Tx tokens) and the summation ORDER is the contract
+// one thread per utterance: the row is short (Tx tokens) and the summation ORDER is the contract.  length_scales (device, B)
+// or nullptr = length_scale for every row: a row's arithmetic is the same either way.
 __global__ void durations_kernel(const float* __restrict__ logw, const int* __restrict__ x_lens, int B, int Tx,
-                                 float length_scale, float* __restrict__ w_ceil, long long* __restrict__ y_lengths,
-                                 long long* __restrict__ y_max) {
+                                 float length_scale, const float* __restrict__ length_scales, float* __restrict__ w_ceil,
+                                 long long* __restrict__ y_lengths, long long* __restrict__ y_max) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
+  if (length_scales) length_scale = length_scales[b];
   const float* lw = logw + (long long)b * Tx;
   float* wc = w_ceil + (long long)b * Tx;
   const int len = x_lens[b];
@@ -79,9 +81,9 @@ __global__ void gather_mu_kernel(const float* __restrict__ mu_x, const int* __re
 
 }  // namespace
 
-cudaError_t durations(const float* logw, const int* x_lens, int B, int Tx, float length_scale, float* w_ceil,
-                      long long* y_lengths, long long* y_max, cudaStream_t s) {
-  durations_kernel<<<ceil_div(B, 32), 32, 0, s>>>(logw, x_lens, B, Tx, length_scale, w_ceil, y_lengths, y_max);
+cudaError_t durations(const float* logw, const int* x_lens, int B, int Tx, float length_scale, const float* length_scales,
+                      float* w_ceil, long long* y_lengths, long long* y_max, cudaStream_t s) {
+  durations_kernel<<<ceil_div(B, 32), 32, 0, s>>>(logw, x_lens, B, Tx, length_scale, length_scales, w_ceil, y_lengths, y_max);
   return cudaGetLastError();
 }
 cudaError_t row_sum_aten(const float* x, int B, int Tx, float* out, cudaStream_t s) {

@@ -52,6 +52,12 @@ struct Epilogue {
   // sum and sum of squares over ALL rows are accumulated into gn_sum[(b*G + g)*2 + {0,1}] (zeroed by the caller)
   double* gn_sum = nullptr;
   int gn_groups = 0;
+  // optional per-item Euler step (ev_decode_items; needs res, no res2, div == 1): item b's step is item_dt[b] in place of alpha,
+  // and an item whose step count item_n[b] is <= item_k is HELD: v = res, a select (x + 0*v would turn -0.0 into +0.0 and an
+  // infinite v into NaN).  nullptr: the scalar epilogue, whose kernels are separate instantiations that never read these fields.
+  const float* item_dt = nullptr;
+  const int* item_n = nullptr;
+  int item_k = 0;
 };
 
 // (GEMM row r, GEMM column n) -> (output time t, output channel co); returns false when the slot is outside the output.
@@ -62,9 +68,18 @@ __device__ __forceinline__ bool ep_coord(const Epilogue& e, int r, int n, int& t
   return t >= 0 && t < e.T_out;
 }
 
+// ITEM: the per-item Euler step of Epilogue::item_dt (the caller has checked res != nullptr, res2 == nullptr, div == 1).  The
+// scalar epilogue multiplies and adds in separate branches, which are never contracted into one FMA; the explicit roundings
+// keep the per-item update on the same two roundings, so that an item gets the bits of a scalar call with its own step.
+template <bool ITEM = false>
 __device__ __forceinline__ float ep_value(const Epilogue& e, int b, int t, int co, float acc, float maskv) {
   float v = acc + (e.bias ? __ldg(e.bias + co) : 0.0f);
   if (e.mask_pre && maskv == 0.0f) v = 0.0f;   // select: a padded row may hold a non-finite value
+  if constexpr (ITEM) {
+    const float r = e.res[b * e.res_bs + (long long)t * e.res_ld + co];
+    v = __fadd_rn(__fmul_rn(v, __ldg(e.item_dt + b)), r);
+    return e.item_k >= __ldg(e.item_n + b) ? r : v;
+  }
   v *= e.alpha;
   if (e.res) v += e.res[b * e.res_bs + (long long)t * e.res_ld + co];
   if (e.res2) v += e.res2[b * e.res2_bs + (long long)t * e.res2_ld + co];

@@ -12,7 +12,7 @@ constexpr int BM = 64, BK = 16, THREADS = 256;
 // global loads in flight during the FMAs.  TN = 8 halves the shared-memory bytes read per FMA (the binding resource of
 // a 4x4 register tile); TN = 4 serves narrow layers.  The per-output summation order is unchanged: taps outer,
 // channels ascending, one fmaf chain.
-template <int TN>
+template <int TN, bool ITEM>
 __global__ void __launch_bounds__(THREADS)
 conv_simt_kernel(ConvGeom g, const float* __restrict__ x, long long x_ld, long long x_bs,
                  const float* __restrict__ w, int N_pad, Epilogue e) {
@@ -86,7 +86,7 @@ conv_simt_kernel(ConvGeom g, const float* __restrict__ x, long long x_ld, long l
       int t, co;
       if (!ep_coord(e, r, n, t, co)) continue;
       const float mv = e.mask.at(b, t);
-      const float v = ep_value(e, b, t, co, acc[i][j], mv);
+      const float v = ep_value<ITEM>(e, b, t, co, acc[i][j], mv);
       if (e.out_f32) e.out_f32[b * e.f32_bs + (long long)t * e.f32_ld + co] = v;
       if (out_act) out_act[b * e.act_bs + (long long)t * e.act_ld + co] = ep_act(e, co, v, mv);
     }
@@ -97,13 +97,17 @@ conv_simt_kernel(ConvGeom g, const float* __restrict__ x, long long x_ld, long l
 cudaError_t conv_simt_launch(const ConvGeom& g, const float* x, long long x_ld, long long x_bs, const ConvWeights& w,
                              const Epilogue& e, cudaStream_t stream) {
   if ((g.C_in & 3) || (x_ld & 3) || (w.N_pad & 3)) return cudaErrorInvalidValue;
+  const bool item = e.item_dt != nullptr;
+  if (item && (!e.item_n || !e.res || e.res2 || e.div != 1.0f)) return cudaErrorInvalidValue;
   // the wide tile only pays when it still fills the machine a few times over (the text encoder's GEMMs are small)
   if (g.N > 64 && (long long)ceil_div(g.M, BM) * ceil_div(g.N, 128) * g.B >= 6 * 148) {
     dim3 grid(ceil_div(g.M, BM), ceil_div(g.N, 128), g.B);
-    conv_simt_kernel<8><<<grid, THREADS, 0, stream>>>(g, x, x_ld, x_bs, w.w_f32, w.N_pad, e);
+    if (item) conv_simt_kernel<8, true><<<grid, THREADS, 0, stream>>>(g, x, x_ld, x_bs, w.w_f32, w.N_pad, e);
+    else conv_simt_kernel<8, false><<<grid, THREADS, 0, stream>>>(g, x, x_ld, x_bs, w.w_f32, w.N_pad, e);
   } else {
     dim3 grid(ceil_div(g.M, BM), ceil_div(g.N, 64), g.B);
-    conv_simt_kernel<4><<<grid, THREADS, 0, stream>>>(g, x, x_ld, x_bs, w.w_f32, w.N_pad, e);
+    if (item) conv_simt_kernel<4, true><<<grid, THREADS, 0, stream>>>(g, x, x_ld, x_bs, w.w_f32, w.N_pad, e);
+    else conv_simt_kernel<4, false><<<grid, THREADS, 0, stream>>>(g, x, x_ld, x_bs, w.w_f32, w.N_pad, e);
   }
   return cudaGetLastError();
 }

@@ -136,6 +136,7 @@ constexpr int ACT_PITCH = 80;                                  // bytes per stag
 
 // generic scalar epilogue of one staged 32 x 32 block (unaligned strides / channel counts that are not multiples of 4);
 // kept out of line so the hot vector path stays compact in the instruction cache
+template <bool ITEM>
 __device__ __noinline__ void scalar_block(const TcParams& p, const float* wstage, int b, int r0, int c0, int lane) {
   const Epilogue& e = p.e;
   bf16* out_act = reinterpret_cast<bf16*>(e.out_act);
@@ -146,14 +147,15 @@ __device__ __noinline__ void scalar_block(const TcParams& p, const float* wstage
     int t, cc;
     if (!ep_coord(e, r, nn, t, cc)) continue;
     const float mv = e.mask.at(b, t);
-    const float v = ep_value(e, b, t, cc, wstage[rl * STAGE_LD + nl], mv);
+    const float v = ep_value<ITEM>(e, b, t, cc, wstage[rl * STAGE_LD + nl], mv);
     if (e.out_f32) e.out_f32[b * e.f32_bs + (long long)t * e.f32_ld + cc] = e.f32_is_act ? ep_act(e, cc, v, mv) : v;
     if (out_act) out_act[b * e.act_bs + (long long)t * e.act_ld + cc] = __float2bfloat16_rn(ep_act(e, cc, v, mv));
   }
 }
 
 // ------------------------------------------------------------------------------------------------ the kernel
-template <int BN>
+// ITEM: the per-item Euler step of Epilogue::item_dt (final_proj of ev_decode_items); false is the scalar epilogue
+template <int BN, bool ITEM>
 __global__ void __launch_bounds__(NUM_THREADS_WIDE, 1)
 conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const __grid_constant__ TcParams p) {
   extern __shared__ uint8_t smem_raw[];
@@ -441,6 +443,13 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       const int vmb = min(p.mb, (M - m0 + BM - 1) / BM);
       const int buf = ti & 1;
       const int len_b = e.mask.lens ? __ldg(e.mask.lens + b) : 0x7fffffff;
+      // this item's Euler step, and whether it is held (ep_value in conv.cuh: same roundings, a select for held items)
+      float t_alpha = 0.0f;
+      bool held = false;
+      if constexpr (ITEM) {
+        t_alpha = __ldg(e.item_dt + b);
+        held = e.item_k >= __ldg(e.item_n + b);
+      }
       const int n_blk = vmb * NBLK;                    // this quadrant's blocks; the warp takes slot, slot+n_slots, ...
       bool waited = false;
 #pragma unroll 1
@@ -596,8 +605,14 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             float v0 = a4.x + bias4.x, v1 = a4.y + bias4.y, v2 = a4.z + bias4.z, v3 = a4.w + bias4.w;
             const float mv = ((t << e.mask.shift) < len_b) ? 1.0f : 0.0f;
             if (mask_pre && mv == 0.0f) { v0 = v1 = v2 = v3 = 0.0f; }   // a select, not a multiply: a padded row may hold anything
-            if (use_alpha) { v0 *= alpha; v1 *= alpha; v2 *= alpha; v3 *= alpha; }
-            if (has_res || has_res2) { v0 += rr[u].x; v1 += rr[u].y; v2 += rr[u].z; v3 += rr[u].w; }
+            if constexpr (ITEM) {
+              v0 = __fadd_rn(__fmul_rn(v0, t_alpha), rr[u].x); v1 = __fadd_rn(__fmul_rn(v1, t_alpha), rr[u].y);
+              v2 = __fadd_rn(__fmul_rn(v2, t_alpha), rr[u].z); v3 = __fadd_rn(__fmul_rn(v3, t_alpha), rr[u].w);
+              if (held) { v0 = rr[u].x; v1 = rr[u].y; v2 = rr[u].z; v3 = rr[u].w; }
+            } else {
+              if (use_alpha) { v0 *= alpha; v1 *= alpha; v2 *= alpha; v3 *= alpha; }
+              if (has_res || has_res2) { v0 += rr[u].x; v1 += rr[u].y; v2 += rr[u].z; v3 += rr[u].w; }
+            }
             if (use_div) { v0 *= inv_div; v1 *= inv_div; v2 *= inv_div; v3 *= inv_div; }
             if (has_f32 && !f32_act) *reinterpret_cast<float4*>(f32_p + (long long)t * e.f32_ld) = make_float4(v0, v1, v2, v3);
             if (e.gn_sum) { gs += (v0 + v1) + (v2 + v3); gq += (v0 * v0 + v1 * v1) + (v2 * v2 + v3 * v3); }
@@ -630,7 +645,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             }
           }
         } else {
-          scalar_block(p, wstage, b, m0 + mb * BM + q * 32, n0 + cb * 32, lane);
+          scalar_block<ITEM>(p, wstage, b, m0 + mb * BM + q * 32, n0 + cb * 32, lane);
         }
         __syncwarp();                // the transpose buffer may be overwritten by the next block
         if (ew == 0 && tile == (int)blockIdx.x && blk == slot) EV_TR(15);
@@ -781,7 +796,10 @@ cudaError_t launch_bn(const CUtensorMap& tmA, const CUtensorMap& tmB, TcParams& 
   const int min_smem = (228 * 1024) / (k_tmem + 1) + 1;
   if (smem < min_smem && k_tmem < 8) smem = std::min(min_smem, SMEM_LIMIT);
   static DeviceOnce once;
-  cudaError_t ce_attr = once.run([&]() { return cudaFuncSetAttribute(conv_tc_kernel<BN>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT); });
+  cudaError_t ce_attr = once.run([&]() {
+    const cudaError_t ce = cudaFuncSetAttribute(conv_tc_kernel<BN, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT);
+    return ce != cudaSuccess ? ce : cudaFuncSetAttribute(conv_tc_kernel<BN, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT);
+  });
   if (ce_attr != cudaSuccess) return ce_attr;
   p.n_issuers = threads == NUM_THREADS_WIDE ? 2 : 1;
   // the sharing walk needs one tap group (haloed tile or a 1x1 conv), streamed weights and room for a step's weight tiles
@@ -798,7 +816,8 @@ cudaError_t launch_bn(const CUtensorMap& tmA, const CUtensorMap& tmB, TcParams& 
     r.flush_groups = (p.kchunks + p.flush_kc - 1) / p.flush_kc; r.tf32_share = p.tf32_share; r.ragged = p.rag != nullptr;
     r.grid = grid; r.total_tiles = p.total_tiles;
   }
-  return launch_pdl(conv_tc_kernel<BN>, dim3(grid), dim3(threads), (size_t)smem, stream, tmA, tmB, p);
+  if (p.e.item_dt) return launch_pdl(conv_tc_kernel<BN, true>, dim3(grid), dim3(threads), (size_t)smem, stream, tmA, tmB, p);
+  return launch_pdl(conv_tc_kernel<BN, false>, dim3(grid), dim3(threads), (size_t)smem, stream, tmA, tmB, p);
 }
 
 }  // namespace
@@ -1000,6 +1019,10 @@ cudaError_t conv_tc_launch(const ConvGeom& g, const void* x, long long x_ld, lon
   }
   if (!ok) return cudaErrorInvalidValue;
   if (tf32x3 && e.out_act) { if (err) *err = "conv_tc: the split-operand paths write fp32 outputs only"; return cudaErrorInvalidValue; }
+  if (e.item_dt && (tf32x3 || !e.item_n || !e.res || e.res2 || e.div != 1.0f || e.gn_sum)) {
+    if (err) *err = "conv_tc: the per-item Euler step needs bf16 operands, item_n, a residual and no res2 / div / GroupNorm statistics";
+    return cudaErrorInvalidValue;
+  }
   if (e.act != ACT_NONE && e.act != ACT_RELU && e.act != ACT_LRELU && e.act != ACT_SNAKE) {
     if (err) *err = "conv_tc: the tensor-core epilogue implements identity / (leaky) ReLU / SnakeBeta only";
     return cudaErrorInvalidValue;

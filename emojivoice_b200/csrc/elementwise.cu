@@ -51,6 +51,10 @@ struct Vals32 { float v[32]; };
 __global__ void upload_kernel(float* dst, Vals32 vals, int n) {
   if ((int)threadIdx.x < n) dst[threadIdx.x] = vals.v[threadIdx.x];
 }
+struct Words { uint32_t w[kUploadWords]; };
+__global__ void upload_words_kernel(uint32_t* dst, Words words, int n) {
+  for (int i = threadIdx.x; i < n; i += blockDim.x) dst[i] = words.w[i];
+}
 
 // ---------------------------------------------------------------------------------------------- embeddings
 __global__ void embed_tokens_kernel(const long long* __restrict__ ids, const float* __restrict__ emb, int Tx, int C,
@@ -152,11 +156,12 @@ __global__ void time_sinusoid_kernel(const float* t_steps, int n, int dim, float
 
 template <typename ActT>
 __global__ void decoder_pack_kernel(const float* __restrict__ z, const float* __restrict__ mu, const float* __restrict__ spk,
-                                    int F, int S, int T, float temperature, RowMask mask, float* __restrict__ x_state,
-                                    ActT* __restrict__ xin, long long xin_ld) {
+                                    int F, int S, int T, float temperature, const float* __restrict__ temperatures,
+                                    RowMask mask, float* __restrict__ x_state, ActT* __restrict__ xin, long long xin_ld) {
   // one block per (b, 32-frame tile): transposes z and mu through shared memory
   extern __shared__ float sh[];  // [2][F][33]
   const int b = blockIdx.y, t0 = blockIdx.x * 32;
+  if (temperatures) temperature = temperatures[b];
   float* zs = sh;
   float* ms = sh + F * 33;
   for (int idx = threadIdx.x; idx < F * 32; idx += blockDim.x) {
@@ -549,6 +554,17 @@ cudaError_t upload_floats(float* dst, const float* vals_host, int n, cudaStream_
   return cudaGetLastError();
 }
 
+cudaError_t upload_words(void* dst, const void* words_host, int n, cudaStream_t s) {
+  const uint32_t* src = reinterpret_cast<const uint32_t*>(words_host);
+  for (int off = 0; off < n; off += kUploadWords) {
+    Words v;
+    const int m = n - off < kUploadWords ? n - off : kUploadWords;
+    for (int i = 0; i < kUploadWords; ++i) v.w[i] = i < m ? src[off + i] : 0u;
+    upload_words_kernel<<<1, 256, 0, s>>>(reinterpret_cast<uint32_t*>(dst) + off, v, m);
+  }
+  return cudaGetLastError();
+}
+
 cudaError_t embed_tokens(const long long* ids, const float* emb, int B, int Tx, int C, int n_vocab, float scale,
                          RowMask mask, float* out, long long out_ld, long long* flags, cudaStream_t s) {
   embed_tokens_kernel<<<B * Tx, 64, 0, s>>>(ids, emb, Tx, C, n_vocab, scale, mask, out, out_ld, flags);
@@ -584,14 +600,17 @@ cudaError_t time_sinusoid(const float* t_steps, int n, int dim, float* out, cuda
 
 template <typename ActT>
 cudaError_t decoder_pack_input(const float* z_cf, const float* mu_cf, const float* spk, int B, int F, int S, int T,
-                               float temperature, RowMask mask, float* x_state, ActT* xin, long long xin_ld, cudaStream_t s) {
+                               float temperature, const float* temperatures, RowMask mask, float* x_state, ActT* xin,
+                               long long xin_ld, cudaStream_t s) {
   dim3 grid(ceil_div(T, 32), B);
   const size_t sh = (size_t)2 * F * 33 * sizeof(float);
-  decoder_pack_kernel<ActT><<<grid, 256, sh, s>>>(z_cf, mu_cf, spk, F, S, T, temperature, mask, x_state, xin, xin_ld);
+  decoder_pack_kernel<ActT><<<grid, 256, sh, s>>>(z_cf, mu_cf, spk, F, S, T, temperature, temperatures, mask, x_state, xin, xin_ld);
   return cudaGetLastError();
 }
-template cudaError_t decoder_pack_input<float>(const float*, const float*, const float*, int, int, int, int, float, RowMask, float*, float*, long long, cudaStream_t);
-template cudaError_t decoder_pack_input<bf16>(const float*, const float*, const float*, int, int, int, int, float, RowMask, float*, bf16*, long long, cudaStream_t);
+template cudaError_t decoder_pack_input<float>(const float*, const float*, const float*, int, int, int, int, float, const float*, RowMask, float*,
+                                               float*, long long, cudaStream_t);
+template cudaError_t decoder_pack_input<bf16>(const float*, const float*, const float*, int, int, int, int, float, const float*, RowMask, float*,
+                                              bf16*, long long, cudaStream_t);
 
 cudaError_t group_norm_stats(const float* x, int B, int T, int C, int groups, double* partial, int* n_chunks_out,
                              cudaStream_t s) {

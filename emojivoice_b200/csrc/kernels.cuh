@@ -16,6 +16,10 @@ cudaError_t cl_to_cf(const float* in, long long in_ld, long long in_bs, int B, i
 cudaError_t i64_to_i32(const long long* in, int* out, int n, cudaStream_t s);
 // dst[i] = vals[i], i < n <= 32: tiny host->device constant upload that is CUDA-graph capturable
 cudaError_t upload_floats(float* dst, const float* vals_host, int n, cudaStream_t s);
+// dst[i] = words[i], i < n: host->device upload of a table of 32-bit words through kernel parameters (graph capturable, no
+// pageable copy), kUploadWords words per launch
+constexpr int kUploadWords = 960;
+cudaError_t upload_words(void* dst, const void* words_host, int n, cudaStream_t s);
 
 // ---- text encoder --------------------------------------------------------------------------------------------
 // text_encoder.py:397: out[b,t,:] = emb[ids[b,t]] * scale, zero on padded rows
@@ -79,8 +83,9 @@ cudaError_t rope_tables(float* cos_t, float* sin_t, int T, int rope_dim, float b
 
 // ---- duration / alignment (integer, bit-exact) -------------------------------------------------------------------
 // y_max (nullable): atomicMax of the lengths (zeroed by the caller) -- the one scalar the host reads back (utils/model.py:18)
-cudaError_t durations(const float* logw, const int* x_lens, int B, int Tx, float length_scale, float* w_ceil,
-                      long long* y_lengths, long long* y_max, cudaStream_t s);
+// length_scales (device, B) or nullptr: item b's w_ceil = ceil(w) * length_scales[b], else * length_scale
+cudaError_t durations(const float* logw, const int* x_lens, int B, int Tx, float length_scale, const float* length_scales,
+                      float* w_ceil, long long* y_lengths, long long* y_max, cudaStream_t s);
 cudaError_t row_sum_aten(const float* x, int B, int Tx, float* out, cudaStream_t s);
 cudaError_t generate_path(const float* w_ceil, const int* x_lens, const int* y_lens, int B, int Tx, int T_pad,
                           float* attn, int* frame_token, cudaStream_t s);
@@ -91,9 +96,11 @@ cudaError_t gather_mu(const float* mu_x_cf, const int* frame_token, const int* y
 // sinusoidal timestep embedding (decoder.py:14-29): out[s, :] for the n Euler times
 cudaError_t time_sinusoid(const float* t_steps, int n, int dim, float* out, cudaStream_t s);
 // xin[b,t,:] = [x0 | mu | spk] * mask ; x_state = x0 = z*temperature      (decoder.py:384-388, flow_matching.py:51)
+// temperatures (device, B) or nullptr: item b's x0 = z * temperatures[b], else z * temperature
 template <typename ActT>
 cudaError_t decoder_pack_input(const float* z_cf, const float* mu_cf, const float* spk, int B, int F, int S, int T,
-                               float temperature, RowMask mask, float* x_state, ActT* xin, long long xin_ld, cudaStream_t s);
+                               float temperature, const float* temperatures, RowMask mask, float* x_state, ActT* xin,
+                               long long xin_ld, cudaStream_t s);
 // GroupNorm statistics over (channels-in-group x ALL padded frames) per batch item (decoder.py:37, SURVEY H1)
 cudaError_t group_norm_stats(const float* x, int B, int T, int C, int groups, double* partial, int* n_chunks_out,
                              cudaStream_t s);

@@ -5,6 +5,7 @@
 #include <algorithm>
 #include <cmath>
 #include <cstdlib>
+#include <cstring>
 
 #include "ctx.cuh"
 
@@ -199,10 +200,12 @@ extern "C" size_t ev_encode_workspace_bytes(const ev_ctx* ctx, int B, int Tx) {
   return w.off + 256;
 }
 
-extern "C" int ev_encode(ev_ctx* ctx, const int64_t* x, const int64_t* x_lengths, const int64_t* spks, int B, int Tx,
-                         float length_scale, float* spk_emb, float* mu_x, float* logw, float* w_ceil, int64_t* y_lengths,
-                         int64_t* summary, void* workspace, size_t workspace_bytes, void* stream) {
-  if (!ctx) return EV_ERR_INVALID;
+namespace {
+
+// ev_encode (length_scales == nullptr: length_scale for every item) and ev_encode_items (item b: length_scales[b])
+int encode_impl(ev_ctx* ctx, const int64_t* x, const int64_t* x_lengths, const int64_t* spks, int B, int Tx, float length_scale,
+                const float* length_scales, float* spk_emb, float* mu_x, float* logw, float* w_ceil, int64_t* y_lengths,
+                int64_t* summary, void* workspace, size_t workspace_bytes, void* stream) {
   if (!ctx->matcha.loaded) return fail(ctx, EV_ERR_STATE, "ev_encode: matcha weights not loaded");
   if (!x || !x_lengths || !mu_x || !logw || !w_ceil || !y_lengths || B <= 0 || Tx <= 0)
     return fail(ctx, EV_ERR_INVALID, "ev_encode: null argument or empty batch");
@@ -322,9 +325,29 @@ extern "C" int ev_encode(ev_ctx* ctx, const int64_t* x, const int64_t* x_lengths
     Epilogue el;
     el.mask = mask; el.mask_pre = 1; el.out_f32 = logw; el.f32_ld = 1; el.f32_bs = Tx;
     EV_TRY(run_conv_tf32(ctx, m.dp_proj, e.D2, Fd, bsF, B, Tx, el, e.split, s));
-    EV_LAUNCH(ctx, s, "durations", 0, R * 8.0, durations(logw, e.xlen32, B, Tx, length_scale, w_ceil, reinterpret_cast<long long*>(y_lengths), summ, s));
+    EV_LAUNCH(ctx, s, "durations", 0, R * 8.0,
+              durations(logw, e.xlen32, B, Tx, length_scale, length_scales, w_ceil, reinterpret_cast<long long*>(y_lengths), summ, s));
   }
   return 0;
+}
+
+}  // namespace
+
+extern "C" int ev_encode(ev_ctx* ctx, const int64_t* x, const int64_t* x_lengths, const int64_t* spks, int B, int Tx,
+                         float length_scale, float* spk_emb, float* mu_x, float* logw, float* w_ceil, int64_t* y_lengths,
+                         int64_t* summary, void* workspace, size_t workspace_bytes, void* stream) {
+  if (!ctx) return EV_ERR_INVALID;
+  return encode_impl(ctx, x, x_lengths, spks, B, Tx, length_scale, nullptr, spk_emb, mu_x, logw, w_ceil, y_lengths, summary,
+                     workspace, workspace_bytes, stream);
+}
+
+extern "C" int ev_encode_items(ev_ctx* ctx, const int64_t* x, const int64_t* x_lengths, const int64_t* spks, int B, int Tx,
+                               const float* length_scales, float* spk_emb, float* mu_x, float* logw, float* w_ceil,
+                               int64_t* y_lengths, int64_t* summary, void* workspace, size_t workspace_bytes, void* stream) {
+  if (!ctx) return EV_ERR_INVALID;
+  if (!length_scales) return fail(ctx, EV_ERR_INVALID, "ev_encode_items: null length_scales");
+  return encode_impl(ctx, x, x_lengths, spks, B, Tx, 1.0f, length_scales, spk_emb, mu_x, logw, w_ceil, y_lengths, summary,
+                     workspace, workspace_bytes, stream);
 }
 
 // ================================================================================================ alignment
@@ -360,6 +383,7 @@ namespace {
 template <typename ActT>
 struct DecBuffers {
   int* ylen32; float* t_steps; float* sinus; float* th1; float* th2; float* tproj;
+  float* item_dt; int* item_n;   // mixed step counts (ev_decode_items): [n_steps][B] Euler steps and [B] step counts after t_steps
   float* xstate; ActT* xin; ActT* cat0; ActT* cat1; ActT* din;
   float* h; float* r; float* xr; ActT* a; ActT* n; float* qkv; ActT* att; ActT* ff; double* gn_partial;
   double* gn_fused; size_t gn_fused_count;   // [n_steps][13][B][8][2] sums written by the conv epilogues (bf16 path)
@@ -367,17 +391,21 @@ struct DecBuffers {
   int* rag_arena; size_t rag_ints;           // tile lists of the convs whose padded output rows nobody reads (out-projection)
 };
 
+// n_steps Euler steps; n_rows rows of the time-embedding chain; items > 0: the per-item step tables of a batch of `items`
+// (one word table: [n_rows] times, [n_rows] steps, [items] step counts, uploaded at once)
 template <typename ActT>
-void plan_decode(const ev_matcha_cfg& c, int B, int T, int n_steps, Workspace& w, DecBuffers<ActT>* d) {
+void plan_decode(const ev_matcha_cfg& c, int B, int T, int n_steps, int n_rows, int items, Workspace& w, DecBuffers<ActT>* d) {
   const size_t R = (size_t)B * T, R2 = (size_t)B * (T / 2);
   const int D = c.dec_channels, inner = c.dec_heads * c.dec_head_dim;
   const int dec_in = 2 * c.n_feats + (c.n_spks > 1 ? c.spk_emb_dim : 0);
   d->ylen32 = w.take<int>(B);
-  d->t_steps = w.take<float>(n_steps);
-  d->sinus = w.take<float>((size_t)n_steps * dec_in);
-  d->th1 = w.take<float>((size_t)n_steps * 4 * D);
-  d->th2 = w.take<float>((size_t)n_steps * 4 * D);
-  d->tproj = w.take<float>((size_t)n_steps * 6 * D);
+  d->t_steps = w.take<float>(items > 0 ? 2 * (size_t)n_rows + items : (size_t)n_rows);
+  d->item_dt = d->t_steps ? d->t_steps + n_rows : nullptr;
+  d->item_n = d->item_dt ? reinterpret_cast<int*>(d->item_dt + n_rows) : nullptr;
+  d->sinus = w.take<float>((size_t)n_rows * dec_in);
+  d->th1 = w.take<float>((size_t)n_rows * 4 * D);
+  d->th2 = w.take<float>((size_t)n_rows * 4 * D);
+  d->tproj = w.take<float>((size_t)n_rows * 6 * D);
   d->xstate = w.take<float>(R * c.n_feats);
   d->xin = w.take<ActT>(R * dec_in);
   d->cat0 = w.take<ActT>(R * 2 * D);
@@ -426,6 +454,23 @@ void euler_schedule(int n, std::vector<float>* t_of_step, std::vector<float>* dt
   }
 }
 
+// The schedules of a batch whose item b takes n[b] steps, row-major [k][b] over k < max n: row k of item b is step k of
+// euler_schedule(n[b]); past its last step an item repeats its last time with a zero step (its state is held by a select, the
+// zero is never multiplied in).
+void euler_tables(const int* n, int B, std::vector<float>* t, std::vector<float>* dt) {
+  const int n_max = *std::max_element(n, n + B);
+  t->assign((size_t)n_max * B, 0.0f);
+  dt->assign((size_t)n_max * B, 0.0f);
+  std::vector<float> tb, dtb;
+  for (int b = 0; b < B; ++b) {
+    euler_schedule(n[b], &tb, &dtb);
+    for (int k = 0; k < n_max; ++k) {
+      (*t)[(size_t)k * B + b] = tb[std::min(k, n[b] - 1)];
+      (*dt)[(size_t)k * B + b] = k < n[b] ? dtb[k] : 0.0f;
+    }
+  }
+}
+
 template <typename ActT>
 struct Decoder {
   ev_ctx* ctx; const MatchaW& m; DecBuffers<ActT>& d; int B, T; cudaStream_t s; int D, inner;
@@ -438,6 +483,7 @@ struct Decoder {
   cudaEvent_t temb_event = nullptr;     // time embeddings are produced on another side branch: waited for at their first use
   long long temb_bs = 0;                // item stride of the time embeddings (0: one t for the batch; ev_estimator: one t per item)
   bool estimator_only = false;          // ev_estimator: the final projection writes v * mask instead of the Euler update
+  const int* item_n = nullptr;          // mixed step counts: this lane's [nb] step counts (device); step() then takes per-item steps
   // GroupNorm statistics: fused into the producing conv's epilogue on the tensor-core path (32 channels per group),
   // a separate reduction kernel otherwise.  Returns the (partial, n_chunks) pair gn_apply reads.
   bool fuse_gn() const { return std::is_same<ActT, bf16>::value && D == 256; }
@@ -625,7 +671,9 @@ struct Decoder {
     return 0;
   }
 
-  int step(const float* temb_step, float dt) {
+  // temb_step: this step's time embeddings (item b at + b * temb_bs); dt: the Euler step, or with item_n the lane's per-item
+  // steps item_dt[b] of step k
+  int step(const float* temb_step, float dt, const float* item_dt = nullptr, int k = 0) {
     const int T2 = T / 2;
     const int dec_in = (int)m.rn[0].c_in;
     const RowMask mask0{d.ylen32, 0}, mask1{d.ylen32, 1};
@@ -687,6 +735,7 @@ struct Decoder {
     if (!estimator_only) {     // Euler update x += dt * v * mask, and the next step's operand
       e.res = d.xstate; e.res_ld = F; e.res_bs = (long long)T * F;
       e.out_act = d.xin; e.act_ld = dec_in; e.act_bs = (long long)T * dec_in; e.mask_act = 1;
+      if (item_n) { e.item_dt = item_dt; e.item_n = item_n; e.item_k = k; }   // held items re-pack their unchanged state
     }
     EV_TRY(run_conv<ActT>(ctx, m.final_proj, d.a, D, (long long)T * D, B, T, e, s));
     return 0;
@@ -700,14 +749,24 @@ int decode_lane_count(const ev_ctx* ctx, int B) {
   return std::max(1, std::min(ctx->dec_lanes, B / 4));
 }
 
+// n_items (host, B) or nullptr: item b takes n_items[b] Euler steps (ev_decode_items), else every item n_steps.  temperatures
+// (device, B) or nullptr: item b's x0 = z * temperatures[b], else z * temperature.
 template <typename ActT>
 int decode_impl(ev_ctx* ctx, const float* mu_y, const int64_t* y_lengths, const float* z, const float* spk_emb, int B,
-                int T, int n_steps, float temperature, float* decoder_out, float* mel, void* workspace, size_t ws_bytes,
-                cudaStream_t s, const float* t_items = nullptr) {
+                int T, int n_steps, const int* n_items, float temperature, const float* temperatures, float* decoder_out, float* mel,
+                void* workspace, size_t ws_bytes, cudaStream_t s, const float* t_items = nullptr) {
   // t_items != nullptr (ev_estimator): ONE evaluation of the estimator with its own time t_items[b] per item; `z` is the point
   // it is evaluated at and decoder_out receives v * mask (decoder.py:363-443 as flow_matching.py:114 calls it)
   const bool est = t_items != nullptr;
-  const int n_rows = est ? B : n_steps;     // rows of the time-embedding chain
+  // mixed step counts: the decoder runs max n_items[b] steps; item b reads its own time embedding of step k (a B x n_steps table,
+  // item stride 6*D as for ev_estimator) and the final projection its own Euler step, and holds its state from step n_items[b] on.
+  // Equal counts are the scalar call (one n_steps-row table shared by the batch).
+  bool mixed = false;
+  if (n_items) {
+    n_steps = *std::max_element(n_items, n_items + B);
+    for (int b = 0; b < B; ++b) mixed |= n_items[b] != n_steps;
+  }
+  const int n_rows = est ? B : (mixed ? B * n_steps : n_steps);     // rows of the time-embedding chain
   const MatchaW& m = ctx->matcha;
   const ev_matcha_cfg& c = m.cfg;
   Workspace w(workspace, ws_bytes);
@@ -718,7 +777,7 @@ int decode_impl(ev_ctx* ctx, const float* mu_y, const int64_t* y_lengths, const 
     lane_b0[l] = b0;
     lane_nb[l] = B / n_lanes + (l < B % n_lanes ? 1 : 0);
     b0 += lane_nb[l];
-    plan_decode<ActT>(c, lane_nb[l], T, n_rows, w, &dl[l]);
+    plan_decode<ActT>(c, lane_nb[l], T, est ? 1 : n_steps, n_rows, mixed ? B : 0, w, &dl[l]);
   }
   if (w.overflow || !workspace) return fail(ctx, EV_ERR_STATE, "ev_decode: workspace too small");
   ctx->prof_tag = "/dec";
@@ -727,7 +786,8 @@ int decode_impl(ev_ctx* ctx, const float* mu_y, const int64_t* y_lengths, const 
   // time embeddings of all steps at once (they do not depend on the batch): sinusoid -> Linear -> SiLU -> Linear,
   // then Mish -> the six resnet mlp Linears stacked along N (decoder.py:381-382, :49,58)
   std::vector<float> ts, dts;
-  euler_schedule(n_steps, &ts, &dts);
+  if (mixed) euler_tables(n_items, B, &ts, &dts);
+  else euler_schedule(n_steps, &ts, &dts);
   // The time-embedding chain depends on nothing but n_steps: with one lane it runs as a side branch (second lane stream) next
   // to the input packing and the first ResNet conv, and is joined where the first time embedding is consumed.
   const bool temb_side = n_lanes == 1 && ctx->dec_side && !ctx->profiling && std::is_same<ActT, bf16>::value;
@@ -738,6 +798,13 @@ int decode_impl(ev_ctx* ctx, const float* mu_y, const int64_t* y_lengths, const 
   }
   if (est) {
     EV_CUDA(ctx, cudaMemcpyAsync(d.t_steps, t_items, (size_t)B * sizeof(float), cudaMemcpyDeviceToDevice, st));
+  } else if (mixed) {     // times, steps and step counts as one table through kernel parameters (no pageable copy: capturable)
+    std::vector<uint32_t> words((size_t)2 * n_rows + B);
+    std::memcpy(words.data(), ts.data(), (size_t)n_rows * 4);
+    std::memcpy(words.data() + n_rows, dts.data(), (size_t)n_rows * 4);
+    std::memcpy(words.data() + 2 * (size_t)n_rows, n_items, (size_t)B * 4);
+    EV_LAUNCH(ctx, st, "upload_words", 0, 4.0 * words.size(), upload_words(d.t_steps, words.data(), (int)words.size(), st));
+    ctx->launches += ceil_div((int)words.size(), kUploadWords) - 1;
   } else {
     EV_LAUNCH(ctx, st, "upload_floats", 0, 4.0 * n_steps, upload_floats(d.t_steps, ts.data(), n_steps, st));
     ctx->launches += ceil_div(n_steps, 32) - 1;
@@ -768,11 +835,12 @@ int decode_impl(ev_ctx* ctx, const float* mu_y, const int64_t* y_lengths, const 
     const RowMask mask0{q.ylen32, 0};
     EV_LAUNCH(ctx, ls[l], "decoder_pack_input", 0, (double)nb * T * (12.0 * F + sizeof(ActT) * dec_in),
               (decoder_pack_input<ActT>(z + b0 * item, mu_y + b0 * item, spk_emb ? spk_emb + (long long)b0 * S : nullptr, nb, F, S, T,
-                                        temperature, mask0, q.xstate, q.xin, dec_in, ls[l])));
+                                        temperature, temperatures ? temperatures + b0 : nullptr, mask0, q.xstate, q.xin, dec_in, ls[l])));
     dec.push_back(Decoder<ActT>{ctx, m, q, nb, T, ls[l], D, c.dec_heads * c.dec_head_dim});
     if (n_lanes == 1 && ctx->dec_side && std::is_same<ActT, bf16>::value) dec.back().side_stream = ctx->lane_stream[ev_ctx::kMaxLanes - 2];
     if (temb_side) dec.back().temb_event = ctx->lane_join[1];
     if (est) { dec.back().temb_bs = 6LL * D; dec.back().estimator_only = true; }
+    if (mixed) { dec.back().temb_bs = 6LL * D; dec.back().item_n = d.item_n + b0; }
     if (std::is_same<ActT, bf16>::value && nb <= kRaggedMaxB) {
       static const bool on = []() { const char* v = getenv("EV_FF_RAGGED"); return !(v && atoi(v) == 0); }();
       if (on) {
@@ -790,7 +858,14 @@ int decode_impl(ev_ctx* ctx, const float* mu_y, const int64_t* y_lengths, const 
   // launches interleave across lanes step by step so that eager (un-captured) calls overlap as well
   if (est) EV_TRY(dec[0].step(d.tproj, 1.0f));      // item b reads row b of tproj (temb_bs)
   for (int k = 0; k < n_steps && !est; ++k)
-    for (int l = 0; l < n_lanes; ++l) EV_TRY(dec[l].step(d.tproj + (size_t)k * 6 * D, dts[k]));
+    for (int l = 0; l < n_lanes; ++l) {
+      if (mixed) {      // row k*B + b of the tables belongs to item b (lane l starts at item lane_b0[l])
+        const size_t row = (size_t)k * B + lane_b0[l];
+        EV_TRY(dec[l].step(d.tproj + row * 6 * D, 1.0f, d.item_dt + row, k));
+      } else {
+        EV_TRY(dec[l].step(d.tproj + (size_t)k * 6 * D, dts[k]));
+      }
+    }
   for (int l = 0; l < n_lanes; ++l) {
     const int b0 = lane_b0[l], nb = lane_nb[l];
     DecBuffers<ActT>& q = dl[l];
@@ -806,16 +881,28 @@ int decode_impl(ev_ctx* ctx, const float* mu_y, const int64_t* y_lengths, const 
 
 }  // namespace
 
-extern "C" size_t ev_decode_workspace_bytes(const ev_ctx* ctx, int B, int T_pad, int n_timesteps) {
-  if (!ctx || !ctx->matcha.loaded || B <= 0 || T_pad <= 0 || n_timesteps <= 0) return 0;
+namespace {
+size_t decode_plan_bytes(const ev_ctx* ctx, int B, int T_pad, int n_steps, int n_rows, int items) {
   Workspace w(nullptr, 0);
   DecBuffers<float> d;  // fp32 operands are the larger plan; it also covers bf16
   const int n_lanes = std::min(std::max(ctx->dec_lanes, 1), std::max(1, B / 4));   // upper bound of decode_lane_count
-  for (int l = 0; l < n_lanes; ++l) plan_decode<float>(ctx->matcha.cfg, B / n_lanes + (l < B % n_lanes ? 1 : 0), T_pad, n_timesteps, w, &d);
+  for (int l = 0; l < n_lanes; ++l) plan_decode<float>(ctx->matcha.cfg, B / n_lanes + (l < B % n_lanes ? 1 : 0), T_pad, n_steps, n_rows, items, w, &d);
   size_t lanes_bytes = w.off;
   Workspace w1(nullptr, 0);                // the single-lane plan (profiling mode) must fit too
-  plan_decode<float>(ctx->matcha.cfg, B, T_pad, n_timesteps, w1, &d);
+  plan_decode<float>(ctx->matcha.cfg, B, T_pad, n_steps, n_rows, items, w1, &d);
   return std::max(lanes_bytes, w1.off) + 256;
+}
+constexpr long long kMaxItemSteps = 1LL << 20;   // B * max n_b of ev_decode_items (time-embedding rows)
+}  // namespace
+
+extern "C" size_t ev_decode_workspace_bytes(const ev_ctx* ctx, int B, int T_pad, int n_timesteps) {
+  if (!ctx || !ctx->matcha.loaded || B <= 0 || T_pad <= 0 || n_timesteps <= 0) return 0;
+  return decode_plan_bytes(ctx, B, T_pad, n_timesteps, n_timesteps, 0);
+}
+
+extern "C" size_t ev_decode_items_workspace_bytes(const ev_ctx* ctx, int B, int T_pad, int n_max) {
+  if (!ctx || !ctx->matcha.loaded || B <= 0 || T_pad <= 0 || n_max <= 0 || (long long)B * n_max > kMaxItemSteps) return 0;
+  return decode_plan_bytes(ctx, B, T_pad, n_max, B * n_max, B);   // covers the equal-counts plan (n_max rows, no tables)
 }
 
 extern "C" int ev_decode(ev_ctx* ctx, const float* mu_y, const int64_t* y_lengths, const float* z, const float* spk_emb,
@@ -830,10 +917,39 @@ extern "C" int ev_decode(ev_ctx* ctx, const float* mu_y, const int64_t* y_length
   EV_CUDA(ctx, cudaSetDevice(ctx->device));
   cudaStream_t s = as_stream(stream);
   if (precision == EV_PREC_FP32)
-    return decode_impl<float>(ctx, mu_y, y_lengths, z, spk_emb, B, T_pad, n_timesteps, temperature, decoder_out, mel, workspace, workspace_bytes, s);
+    return decode_impl<float>(ctx, mu_y, y_lengths, z, spk_emb, B, T_pad, n_timesteps, nullptr, temperature, nullptr, decoder_out, mel,
+                              workspace, workspace_bytes, s);
   if (precision == EV_PREC_BF16)
-    return decode_impl<bf16>(ctx, mu_y, y_lengths, z, spk_emb, B, T_pad, n_timesteps, temperature, decoder_out, mel, workspace, workspace_bytes, s);
+    return decode_impl<bf16>(ctx, mu_y, y_lengths, z, spk_emb, B, T_pad, n_timesteps, nullptr, temperature, nullptr, decoder_out, mel,
+                             workspace, workspace_bytes, s);
   return fail(ctx, EV_ERR_INVALID, "ev_decode: unknown precision");
+}
+
+extern "C" int ev_decode_items(ev_ctx* ctx, const float* mu_y, const int64_t* y_lengths, const float* z, const float* spk_emb,
+                               int B, int T_pad, const int32_t* n_steps_host, const float* temperatures, int precision,
+                               float* decoder_out, float* mel, void* workspace, size_t workspace_bytes, void* stream) {
+  if (!ctx) return EV_ERR_INVALID;
+  if (!ctx->matcha.loaded) return fail(ctx, EV_ERR_STATE, "ev_decode_items: matcha weights not loaded");
+  if (!mu_y || !y_lengths || !z || !decoder_out || !n_steps_host || !temperatures || B <= 0 || T_pad <= 0)
+    return fail(ctx, EV_ERR_INVALID, "ev_decode_items: null argument or empty shape");
+  int n_max = 0;
+  for (int b = 0; b < B; ++b) {
+    if (n_steps_host[b] < 1) return fail(ctx, EV_ERR_INVALID, "ev_decode_items: every item needs n_steps >= 1");
+    n_max = std::max(n_max, (int)n_steps_host[b]);
+  }
+  if ((long long)B * n_max > kMaxItemSteps) return fail(ctx, EV_ERR_INVALID, "ev_decode_items: B * max(n_steps) exceeds 2^20");
+  if (T_pad % 4) return fail(ctx, EV_ERR_INVALID, "ev_decode_items: T_pad must be a multiple of 4 (fix_len_compatibility)");
+  if (ctx->matcha.cfg.n_spks > 1 && !spk_emb) return fail(ctx, EV_ERR_INVALID, "ev_decode_items: spk_emb required");
+  EV_CUDA(ctx, cudaSetDevice(ctx->device));
+  cudaStream_t s = as_stream(stream);
+  const int* n_items = reinterpret_cast<const int*>(n_steps_host);
+  if (precision == EV_PREC_FP32)
+    return decode_impl<float>(ctx, mu_y, y_lengths, z, spk_emb, B, T_pad, n_max, n_items, 1.0f, temperatures, decoder_out, mel,
+                              workspace, workspace_bytes, s);
+  if (precision == EV_PREC_BF16)
+    return decode_impl<bf16>(ctx, mu_y, y_lengths, z, spk_emb, B, T_pad, n_max, n_items, 1.0f, temperatures, decoder_out, mel,
+                             workspace, workspace_bytes, s);
+  return fail(ctx, EV_ERR_INVALID, "ev_decode_items: unknown precision");
 }
 
 extern "C" size_t ev_estimator_workspace_bytes(const ev_ctx* ctx, int B, int T_pad) {
@@ -852,9 +968,9 @@ extern "C" int ev_estimator(ev_ctx* ctx, const float* y, const int64_t* y_length
   EV_CUDA(ctx, cudaSetDevice(ctx->device));
   cudaStream_t s = as_stream(stream);
   if (precision == EV_PREC_FP32)
-    return decode_impl<float>(ctx, mu, y_lengths, y, spk_emb, B, T_pad, 1, 1.0f, v_out, nullptr, workspace, workspace_bytes, s, t);
+    return decode_impl<float>(ctx, mu, y_lengths, y, spk_emb, B, T_pad, 1, nullptr, 1.0f, nullptr, v_out, nullptr, workspace, workspace_bytes, s, t);
   if (precision == EV_PREC_BF16)
-    return decode_impl<bf16>(ctx, mu, y_lengths, y, spk_emb, B, T_pad, 1, 1.0f, v_out, nullptr, workspace, workspace_bytes, s, t);
+    return decode_impl<bf16>(ctx, mu, y_lengths, y, spk_emb, B, T_pad, 1, nullptr, 1.0f, nullptr, v_out, nullptr, workspace, workspace_bytes, s, t);
   return fail(ctx, EV_ERR_INVALID, "ev_estimator: unknown precision");
 }
 
@@ -864,5 +980,17 @@ extern "C" int ev_test_euler_schedule(int n, float* t_host, float* dt_host) {
   std::vector<float> t, dt;
   euler_schedule(n, &t, &dt);
   for (int i = 0; i < n; ++i) { t_host[i] = t[i]; dt_host[i] = dt[i]; }
+  return 0;
+}
+
+// test hook: the per-item Euler tables of ev_decode_items with mixed step counts, [max n][B] each (pure host code)
+extern "C" int ev_test_euler_tables(const int32_t* n_steps_host, int B, float* t_host, float* dt_host) {
+  if (!n_steps_host || B <= 0 || !t_host || !dt_host) return EV_ERR_INVALID;
+  for (int b = 0; b < B; ++b)
+    if (n_steps_host[b] < 1) return EV_ERR_INVALID;
+  std::vector<float> t, dt;
+  euler_tables(reinterpret_cast<const int*>(n_steps_host), B, &t, &dt);
+  std::copy(t.begin(), t.end(), t_host);
+  std::copy(dt.begin(), dt.end(), dt_host);
   return 0;
 }

@@ -8,6 +8,8 @@ from __future__ import annotations
 
 import ctypes as C
 import datetime as dt
+import math
+import numbers
 
 import torch
 
@@ -102,7 +104,13 @@ class MatchaTTS:
     @torch.inference_mode()
     def synthesise(self, x, x_lengths, n_timesteps, temperature=1.0, spks=None, length_scale=1.0, z=None, dtype=None):
         """Same contract as matcha_tts.py:77-152.  Extras: `z` injects the prior noise (B, n_feats, T_pad) *before*
-        temperature scaling (the reference draws it at flow_matching.py:51); `dtype` picks "fp32" | "bf16"."""
+        temperature scaling (the reference draws it at flow_matching.py:51); `dtype` picks "fp32" | "bf16".
+
+        `n_timesteps`, `temperature` and `length_scale` each take a number (the whole batch) or a (B,) sequence / tensor (one
+        value per utterance).  Utterance b of a batch with per-utterance values gets the durations, alignment and lengths of
+        the batch called with length_scale[b], and the mel of the batch called with (n_timesteps[b], temperature[b]) at the
+        same padded length T_pad (ev_encode_items / ev_decode_items in include/emojivoice_b200.h); per-utterance values that
+        are all equal are the call with that number."""
         if not self._loaded:
             raise RuntimeError("load_state_dict() / load_from_checkpoint() first")
         t0 = dt.datetime.now()
@@ -113,6 +121,10 @@ class MatchaTTS:
             x = x.to(device=dev, dtype=torch.int64).contiguous()
             x_lengths = x_lengths.to(device=dev, dtype=torch.int64).contiguous()
             B, Tx = x.shape
+            n_timesteps = per_item_setting(n_timesteps, B, "n_timesteps")
+            temperature = per_item_setting(temperature, B, "temperature")
+            length_scale = per_item_setting(length_scale, B, "length_scale")
+            ls_items = isinstance(length_scale, tuple)
             if self.n_spks > 1:
                 if spks is None:
                     raise ValueError("multi-speaker model: `spks` (speaker / emoji ids) is required")
@@ -125,6 +137,13 @@ class MatchaTTS:
             S = self.spk_emb_dim if self.n_spks > 1 else 0
 
             def encode(i, o, ws):
+                if ls_items:
+                    ctx.check(L.ev_encode_items(ctx.handle, _lib.ptr(i["x"]), _lib.ptr(i["x_lengths"]), _lib.ptr(i["spks"]), B, Tx,
+                                                _lib.ptr(i["length_scales"]), _lib.ptr(o.get("spk_emb")), _lib.ptr(o["mu_x"]),
+                                                _lib.ptr(o["logw"]), _lib.ptr(o["w_ceil"]), _lib.ptr(o["y_lengths"]), _lib.ptr(o["summary"]),
+                                                _lib.ptr(ws), ws.numel(), _lib.stream_ptr()),
+                              "ev_encode_items")
+                    return
                 ctx.check(L.ev_encode(ctx.handle, _lib.ptr(i["x"]), _lib.ptr(i["x_lengths"]), _lib.ptr(i["spks"]), B, Tx,
                                       float(length_scale), _lib.ptr(o.get("spk_emb")), _lib.ptr(o["mu_x"]), _lib.ptr(o["logw"]),
                                       _lib.ptr(o["w_ceil"]), _lib.ptr(o["y_lengths"]), _lib.ptr(o["summary"]), _lib.ptr(ws), ws.numel(),
@@ -136,8 +155,11 @@ class MatchaTTS:
                        "summary": ((2,), i64)}
             if S:
                 enc_out["spk_emb"] = ((B, S), f32)
-            e = self._run("encode", (B, Tx, float(length_scale)), L.ev_encode_workspace_bytes(ctx.handle, B, Tx),
-                          {"x": x, "x_lengths": x_lengths, "spks": spks}, enc_out, encode)
+            enc_in = {"x": x, "x_lengths": x_lengths, "spks": spks}
+            if ls_items:    # a static input of the captured graph: a replay reads the values of its own call
+                enc_in["length_scales"] = torch.tensor(length_scale, dtype=torch.float32).to(dev)
+            e = self._run("encode", (B, Tx, "items" if ls_items else float(length_scale)), L.ev_encode_workspace_bytes(ctx.handle, B, Tx),
+                          enc_in, enc_out, encode)
             mu_x, logw, w_ceil, y_lengths, spk_emb = e["mu_x"], e["logw"], e["w_ceil"], e["y_lengths"], e.get("spk_emb")
             # the reference's one host sync (y_lengths.max(), utils/model.py:18): the library reduced it on the device, together
             # with the id-range flags (nn.Embedding raises IndexError where the kernels clamp)
@@ -152,19 +174,38 @@ class MatchaTTS:
                 z = z.to(device=dev, dtype=torch.float32).contiguous()
                 if tuple(z.shape) != (B, F, T_pad):
                     raise ValueError(f"z must have shape {(B, F, T_pad)}, got {tuple(z.shape)}")
-            n_steps, temp = int(n_timesteps), float(temperature)
+            dec_items = isinstance(n_timesteps, tuple) or isinstance(temperature, tuple)
+            dec_in = {"w_ceil": w_ceil, "x_lengths": x_lengths, "y_lengths": y_lengths, "mu_x": mu_x, "z": z, "spk_emb": spk_emb}
+            if dec_items:
+                # the step counts are read on the host while the launches are enqueued (part of the graph key); the temperatures
+                # are a static device input of the graph
+                n_list = n_timesteps if isinstance(n_timesteps, tuple) else (int(n_timesteps),) * B
+                n_host = (C.c_int32 * B)(*n_list)
+                temps = temperature if isinstance(temperature, tuple) else (float(temperature),) * B
+                dec_in["temperatures"] = torch.tensor(temps, dtype=torch.float32).to(dev)
+                dec_key = (B, Tx, T_pad, ("n",) + n_list, "items", prec)
+                dec_bytes = L.ev_decode_items_workspace_bytes(ctx.handle, B, T_pad, max(n_list))
+            else:
+                n_steps, temp = int(n_timesteps), float(temperature)
+                dec_key = (B, Tx, T_pad, n_steps, temp, prec)
+                dec_bytes = L.ev_decode_workspace_bytes(ctx.handle, B, T_pad, n_steps)
 
             def align_decode(i, o, ws):
                 ctx.check(L.ev_align(ctx.handle, _lib.ptr(i["w_ceil"]), _lib.ptr(i["x_lengths"]), _lib.ptr(i["y_lengths"]),
                                      _lib.ptr(i["mu_x"]), B, Tx, T_pad, _lib.ptr(o["attn"]), _lib.ptr(o["mu_y"]), _lib.ptr(o["y_mask"]),
                                      _lib.ptr(ws), ws.numel(), _lib.stream_ptr()), "ev_align")
+                if dec_items:
+                    ctx.check(L.ev_decode_items(ctx.handle, _lib.ptr(o["mu_y"]), _lib.ptr(i["y_lengths"]), _lib.ptr(i["z"]),
+                                                _lib.ptr(i["spk_emb"]), B, T_pad, n_host, _lib.ptr(i["temperatures"]), prec,
+                                                _lib.ptr(o["dec"]), _lib.ptr(o["mel"]), _lib.ptr(ws), ws.numel(), _lib.stream_ptr()),
+                              "ev_decode_items")
+                    return
                 ctx.check(L.ev_decode(ctx.handle, _lib.ptr(o["mu_y"]), _lib.ptr(i["y_lengths"]), _lib.ptr(i["z"]), _lib.ptr(i["spk_emb"]),
                                       B, T_pad, n_steps, temp, prec, _lib.ptr(o["dec"]), _lib.ptr(o["mel"]), _lib.ptr(ws), ws.numel(),
                                       _lib.stream_ptr()), "ev_decode")
 
-            nb = max(L.ev_align_workspace_bytes(ctx.handle, B, Tx, T_pad), L.ev_decode_workspace_bytes(ctx.handle, B, T_pad, n_steps))
-            d = self._run("decode", (B, Tx, T_pad, n_steps, temp, prec), nb,
-                          {"w_ceil": w_ceil, "x_lengths": x_lengths, "y_lengths": y_lengths, "mu_x": mu_x, "z": z, "spk_emb": spk_emb},
+            nb = max(L.ev_align_workspace_bytes(ctx.handle, B, Tx, T_pad), dec_bytes)
+            d = self._run("decode", dec_key, nb, dec_in,
                           {"attn": ((B, Tx, T_pad), f32), "mu_y": ((B, F, T_pad), f32), "y_mask": ((B, 1, T_pad), f32),
                            "dec": ((B, F, T_pad), f32), "mel": ((B, F, T_pad), f32)}, align_decode)
             attn, mu_y, y_mask, dec, mel = d["attn"], d["mu_y"], d["y_mask"], d["dec"], d["mel"]
@@ -302,6 +343,32 @@ class MatchaTTS:
         if reset:
             self._replayed_launches = 0
         return n
+
+
+def per_item_setting(value, B, name):
+    """One synthesis setting of a batch of B utterances: a number for the whole batch, or a (B,) sequence / tensor with one
+    value per utterance.  -> the number, or a tuple of B values when they differ (values that are all equal are the number).
+    Per-utterance values are checked here, since the library reads the length scales and temperatures on the device:
+    n_timesteps must be integers >= 1, length_scale finite and positive, temperature finite."""
+    if isinstance(value, numbers.Number) or (torch.is_tensor(value) and value.dim() == 0):
+        return value.item() if torch.is_tensor(value) else value
+    vals = value.detach().reshape(-1).tolist() if torch.is_tensor(value) else list(value)
+    if len(vals) != B:
+        raise ValueError(f"{name}: expected a number or {B} values (one per utterance), got {len(vals)}")
+    for v in vals:
+        if not isinstance(v, numbers.Real) or not math.isfinite(v):
+            raise ValueError(f"{name}: per-utterance values must be finite numbers, got {v!r}")
+    if name == "n_timesteps":
+        if any(v != int(v) or v < 1 for v in vals):
+            raise ValueError(f"n_timesteps: per-utterance step counts must be integers >= 1, got {vals}")
+        vals = [int(v) for v in vals]
+    elif name == "length_scale":
+        if any(v <= 0 for v in vals):
+            raise ValueError(f"length_scale: per-utterance values must be positive, got {vals}")
+        vals = [float(v) for v in vals]
+    else:
+        vals = [float(v) for v in vals]
+    return vals[0] if all(v == vals[0] for v in vals) else tuple(vals)
 
 
 class _CFMFacade:

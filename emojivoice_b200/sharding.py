@@ -9,6 +9,7 @@ runs unchanged under the `gloo` backend in the CPU test-suite.
 """
 from __future__ import annotations
 
+import numbers
 from dataclasses import dataclass, field
 
 SR, HOP = 22050, 256
@@ -28,22 +29,28 @@ class MicroBatch:
     rank: int = -1
 
 
-def microbatches(x_lengths, batch_size: int, n_timesteps: int = 10, frames_per_token: float = 2.9, sort: bool = True):
+def microbatches(x_lengths, batch_size: int, n_timesteps=10, frames_per_token: float = 2.9, sort: bool = True):
     """Cut the utterance list into micro-batches of `batch_size` (the last one may be smaller).
 
     sort=True orders utterances by text length first (stable), which bounds padding; sort=False keeps the caller's
-    order (what `matcha/cli.py:281-286`'s DataLoader does).  `frames_per_token` only feeds the cost estimate."""
+    order (what `matcha/cli.py:281-286`'s DataLoader does).  `frames_per_token` only feeds the cost estimate.
+    n_timesteps: the Euler steps of every utterance, or a sequence with each utterance's own count (indexed like
+    x_lengths); the cost of a batch sums each utterance's estimate at its own count.  The plan itself does not depend on it."""
     lens = [int(v) for v in x_lengths]
     if batch_size <= 0:
         raise ValueError("batch_size must be positive")
+    per_item = not isinstance(n_timesteps, numbers.Number)
+    if per_item and len(n_timesteps) != len(lens):
+        raise ValueError("n_timesteps: one step count per utterance expected")
     order = sorted(range(len(lens)), key=lambda i: lens[i]) if sort else list(range(len(lens)))
     out = []
     for k in range(0, len(order), batch_size):
         items = order[k:k + batch_size]
         tx_max = max(lens[i] for i in items)
         frames = int(round(tx_max * frames_per_token))
-        out.append(MicroBatch(index=len(out), items=items, tx_max=tx_max,
-                              cost=len(items) * estimate_flops(tx_max, frames, n_timesteps)))
+        cost = (sum(estimate_flops(tx_max, frames, int(n_timesteps[i])) for i in items) if per_item
+                else len(items) * estimate_flops(tx_max, frames, n_timesteps))
+        out.append(MicroBatch(index=len(out), items=items, tx_max=tx_max, cost=cost))
     return out
 
 
@@ -82,11 +89,13 @@ class ShardStats:
     extra: dict = field(default_factory=dict)
 
     def add(self, mel_lengths, tx_lengths, n_timesteps, seconds):
-        for t, f in zip(tx_lengths, mel_lengths):
+        """n_timesteps: the step count of every utterance, or a sequence with each one's own."""
+        steps = [n_timesteps] * len(tx_lengths) if isinstance(n_timesteps, numbers.Number) else list(n_timesteps)
+        for t, f, n in zip(tx_lengths, mel_lengths, steps):
             self.utterances += 1
             self.frames += int(f)
             self.audio_seconds += int(f) * HOP / SR
-            self.flops += estimate_flops(int(t), int(f), n_timesteps)
+            self.flops += estimate_flops(int(t), int(f), int(n))
         self.seconds += float(seconds)
 
 

@@ -101,6 +101,14 @@ EV_API size_t ev_encode_workspace_bytes(const ev_ctx* ctx, int B, int Tx);
 EV_API int ev_encode(ev_ctx* ctx, const int64_t* x, const int64_t* x_lengths, const int64_t* spks, int B, int Tx,
               float length_scale, float* spk_emb, float* mu_x, float* logw, float* w_ceil, int64_t* y_lengths,
               int64_t* summary, void* workspace, size_t workspace_bytes, void* stream);
+/* Per-item length scale: the same call with a speaking rate per utterance, length_scales (B) device fp32 (ev_encode is this
+ * call with length_scale in every entry).  Item b's w_ceil and y_lengths are bit-identical to those of ev_encode on the same
+ * batch with length_scale = length_scales[b]: the encoder does not read the length scale and the length stage is per row.
+ * The values stay on the device (no host synchronisation, capturable): a finite, positive scale per item is the caller's
+ * duty, as in the reference, which multiplies by whatever it is given.  Uses ev_encode_workspace_bytes. */
+EV_API int ev_encode_items(ev_ctx* ctx, const int64_t* x, const int64_t* x_lengths, const int64_t* spks, int B, int Tx,
+              const float* length_scales, float* spk_emb, float* mu_x, float* logw, float* w_ceil, int64_t* y_lengths,
+              int64_t* summary, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- alignment / length regulator (integer, bit-exact) -----------------------------------------------
  * Replaces matcha_tts.py:129-135: sequence_mask, generate_path (utils/model.py:29-41) and
@@ -120,6 +128,18 @@ EV_API int ev_align(ev_ctx* ctx, const float* w_ceil, const int64_t* x_lengths, 
 EV_API size_t ev_decode_workspace_bytes(const ev_ctx* ctx, int B, int T_pad, int n_timesteps);
 EV_API int ev_decode(ev_ctx* ctx, const float* mu_y, const int64_t* y_lengths, const float* z, const float* spk_emb,
               int B, int T_pad, int n_timesteps, float temperature, int precision, float* decoder_out,
+              float* mel, void* workspace, size_t workspace_bytes, void* stream);
+/* Per-item step count and temperature: item b takes n_steps_host[b] >= 1 Euler steps (host int32, B) from
+ * x0 = z * temperatures[b] (device fp32, B).  Item b's decoder_out and mel are bit-identical to those of ev_decode on the same
+ * batch (same mu_y, y_lengths, z, T_pad) called with (n_steps_host[b], temperatures[b]) for every item: items of a padded batch
+ * interact only through T_pad (GroupNorm, attention and masks are per item).  Item b integrates on its own schedule
+ * t_span = linspace(0, 1, n_b + 1); the call runs max n_b steps, and at steps k >= n_b item b's state is held by a select
+ * (not by a zero step: x + 0*v would change -0.0 and turn an infinite v into NaN) while the item still passes through the
+ * estimator.  Equal counts run the kernels and launches of ev_decode.  The step counts are read on the host; the
+ * temperatures stay on the device (capturable).  Rejects a null pointer or n_b < 1 with EV_ERR_INVALID. */
+EV_API size_t ev_decode_items_workspace_bytes(const ev_ctx* ctx, int B, int T_pad, int n_max);
+EV_API int ev_decode_items(ev_ctx* ctx, const float* mu_y, const int64_t* y_lengths, const float* z, const float* spk_emb,
+              int B, int T_pad, const int32_t* n_steps_host, const float* temperatures, int precision, float* decoder_out,
               float* mel, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- HiFi-GAN generator ----------------------------------------------------------------------------------
@@ -327,6 +347,9 @@ EV_API int ev_test_resnet_trace(ev_ctx* ctx, uint64_t* out_host, int n);
  * upsampler i (up[i]) and inside stage i (stage[i]), i < n_ups -- upper bounds of the generator's look-ahead. */
 EV_API int ev_test_vocoder_margins(const ev_hifigan_cfg* cfg, int32_t* stage, int32_t* up, int32_t* pre);
 EV_API int ev_test_euler_schedule(int n_timesteps, float* t_host, float* dt_host);
+/* The tables ev_decode_items uses for mixed step counts, (max n) x B row-major each (pure host code): row k of item b is step k
+ * of ev_test_euler_schedule(n_b); past its last step an item repeats its last time with a zero step. */
+EV_API int ev_test_euler_tables(const int32_t* n_steps_host, int B, float* t_host, float* dt_host);
 /* y_lengths of torch.sum order: sums (B,Tx) fp32 rows exactly as ATen's CPU float32 reduction does. */
 EV_API int ev_test_row_sum(ev_ctx* ctx, const float* x, int B, int Tx, float* out, void* stream);
 /* Diagnostic (EV_TC_TRACE=1): clock64 stamps [CTA][16] of the most recent tensor-core conv launch's pipeline milestones
