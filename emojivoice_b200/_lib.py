@@ -77,6 +77,10 @@ SIGNATURES = {
     "ev_denoise_ragged": (_I, [_P, _P, _P, _I, _I, _F, _P, _P, _SZ, _P]),
     "ev_to_waveform_ragged_workspace_bytes": (_SZ, [_P, _I, _I]),
     "ev_to_waveform_ragged": (_I, [_P, _P, _P, _I, _I, _I, _F, _P, _P, _SZ, _P]),
+    "ev_denoise_items_workspace_bytes": (_SZ, [_P, _I, _I]),
+    "ev_denoise_items": (_I, [_P, _P, _P, _I, _I, _P, _P, _P, _P, _SZ, _P]),
+    "ev_to_waveform_items_workspace_bytes": (_SZ, [_P, _I, _I]),
+    "ev_to_waveform_items": (_I, [_P, _P, _P, _I, _I, _I, _P, _P, _P, _P, _SZ, _P]),
     "ev_maximum_path_workspace_bytes": (_SZ, [_P, _I, _I, _I]),
     "ev_maximum_path": (_I, [_P, _P, _P, _P, _I, _I, _I, _F, _P, _P, _SZ, _P]),
     "ev_estimator_workspace_bytes": (_SZ, [_P, _I, _I]),

@@ -9,6 +9,7 @@ from . import sharding
 
 
 SETTINGS = ("length_scale", "temperature", "n_timesteps")
+VOCODER_SETTINGS = ("denoiser_strength",)      # per utterance too, but read after synthesis: the plan does not depend on them
 
 
 def collate(utterances, items):
@@ -59,20 +60,31 @@ def lanes_for(model, vocoder, n: int) -> Lanes:
 
 
 def utterance_settings(utterances, defaults):
-    """Each utterance's (length_scale, temperature, n_timesteps): an utterance is (ids, speaker_id) or (ids, speaker_id,
+    """Each utterance's settings (SETTINGS and VOCODER_SETTINGS): an utterance is (ids, speaker_id) or (ids, speaker_id,
     settings) with a dict holding any of those keys; a missing key takes its value from `defaults`.
-    -> (per-utterance dicts, True when some utterance has its own settings)"""
+    -> (per-utterance dicts, True when some utterance has its own synthesis settings (SETTINGS))"""
     out, own = [], False
     for u in utterances:
         s = dict(defaults)
         if len(u) > 2 and u[2]:
-            extra = set(u[2]) - set(SETTINGS)
+            extra = set(u[2]) - set(SETTINGS) - set(VOCODER_SETTINGS)
             if extra:
-                raise ValueError(f"unknown per-utterance settings {sorted(extra)}; expected keys among {SETTINGS}")
+                raise ValueError(f"unknown per-utterance settings {sorted(extra)}; expected keys among {SETTINGS + VOCODER_SETTINGS}")
             s.update(u[2])
-            own = True
+            own = own or any(k in SETTINGS for k in u[2])
         out.append(s)
     return out, own
+
+
+def denoiser_strengths(settings, denoiser):
+    """Each utterance's denoiser strength from its settings, None = not denoised; refuses a strength without a denoiser."""
+    from .hifigan import per_item_strength
+
+    dn = [s["denoiser_strength"] for s in settings]
+    if denoiser is None and any(v is not None for v in dn):
+        raise ValueError("a per-utterance denoiser_strength needs a denoiser: pass denoiser=Denoiser(vocoder)")
+    per_item_strength(dn, len(dn))          # the host-side checks, before any work is done
+    return dn
 
 
 @torch.inference_mode()
@@ -83,6 +95,10 @@ def synthesise_corpus(model, vocoder, utterances, batch_size=32, n_timesteps=10,
     where settings is a dict with any of "length_scale", "temperature", "n_timesteps" for that utterance (a missing key takes
     the keyword's value).  Utterances with different settings share micro-batches (MatchaTTS.synthesise with per-utterance
     values); the micro-batch plan does not depend on them, only its cost estimate uses each utterance's own step count.
+    settings may also hold "denoiser_strength": a number, or None for an utterance that is not denoised; a missing key takes
+    `denoiser_strength`, or None when `denoiser` is None (a strength without a denoiser is a ValueError).  The vocoder stage of
+    a micro-batch then denoises each utterance with its own strength (Generator.vocode_denoised, Denoiser with per-item
+    strengths), so an utterance's mel and waveform do not depend on what the other utterances asked of the denoiser.
 
     -> (results, stats): results maps utterance index -> dict(waveform (L,) cpu float32, mel_length, [mel]), stats is a
     sharding.ShardStats with this rank's device time.  `z_fn(mb, model, x, x_lengths, spks)` may supply the prior noise per
@@ -97,7 +113,9 @@ def synthesise_corpus(model, vocoder, utterances, batch_size=32, n_timesteps=10,
     caches one); the waveforms do not depend on it.  stats.seconds is the sum of the micro-batches' device times for one
     lane and the device span from the first launch to the last kernel's end for several."""
     lens = [len(u[0]) for u in utterances]
-    settings, own = utterance_settings(utterances, dict(length_scale=length_scale, temperature=temperature, n_timesteps=n_timesteps))
+    settings, own = utterance_settings(utterances, dict(length_scale=length_scale, temperature=temperature, n_timesteps=n_timesteps,
+                                                        denoiser_strength=denoiser_strength if denoiser is not None else None))
+    strengths = denoiser_strengths(settings, denoiser)
     steps = [int(s["n_timesteps"]) for s in settings] if own else n_timesteps
     plan = sharding.shard(lens, batch_size, rank, world_size, n_timesteps=steps, sort=sort)
     results, stats = {}, sharding.ShardStats()
@@ -154,12 +172,13 @@ def synthesise_corpus(model, vocoder, utterances, batch_size=32, n_timesteps=10,
                     n_b, temp_b, ls_b = n_timesteps, temperature, length_scale
                 out = m.synthesise(x, xl, n_b, temp_b, spks if m.n_spks > 1 else None, ls_b, **kw)
                 d = lanes.denoiser(lane, denoiser)
+                dn = [strengths[i] for i in mb.items]        # equal values are the scalar call (per_item_strength)
                 if ragged and d is not None and d.vocoder is v:
-                    wav = v.vocode_denoised(out["mel"], out["mel_lengths"], denoiser_strength)
+                    wav = v.vocode_denoised(out["mel"], out["mel_lengths"], dn)
                 else:
                     wav = v(out["mel"], lengths=out["mel_lengths"] if ragged and d is None else None).clamp(-1, 1)   # to_waveform, cli.py:121-126
                     if d is not None:
-                        wav = d(wav.squeeze(1), strength=denoiser_strength).unsqueeze(1)
+                        wav = d(wav.squeeze(1), strength=dn).unsqueeze(1)
                 e1.record()
                 # read-back on a copy stream into pinned memory (the `.cpu()` of to_waveform): the host crops an EARLIER micro-batch
                 # while this one's copy -- and the next ones' kernels -- are in flight

@@ -83,14 +83,9 @@ __global__ void spectral_subtract_kernel(float* __restrict__ spec, int frames, c
   }
 }
 
-// torch.istft: overlap-add of the windowed frames divided by the overlap-added squared window, centre padding trimmed.
-// lens (ragged batch, or nullptr): item b is written on [0, lens[b] * HOP) and zero beyond, where its frames were not computed
-__global__ void overlap_add_kernel(const float* __restrict__ y, int frames, const float* __restrict__ win_sq, int L_out,
-                                   const int* __restrict__ lens, float* __restrict__ out) {
-  const int b = blockIdx.y;
-  const int t = blockIdx.x * blockDim.x + threadIdx.x;
-  if (t >= L_out) return;
-  if (lens && t >= __ldg(lens + b) * HOP) { out[(long long)b * L_out + t] = 0.0f; return; }
+// torch.istft at output sample t of item b: overlap-add of the windowed frames divided by the overlap-added squared window,
+// centre padding trimmed
+__device__ __forceinline__ float overlap_add_at(const float* __restrict__ y, int frames, const float* __restrict__ win_sq, int b, int t) {
   const int tt = t + NFFT / 2;
   int f_lo = (tt - (NFFT - 1) + HOP - 1) / HOP;
   if (f_lo < 0) f_lo = 0;
@@ -102,7 +97,31 @@ __global__ void overlap_add_kernel(const float* __restrict__ y, int frames, cons
     acc += y[((long long)b * frames + f) * NFFT + n];
     env += win_sq[n];
   }
-  out[(long long)b * L_out + t] = acc / env;
+  return acc / env;
+}
+
+// lens (ragged batch, or nullptr): item b is written on [0, lens[b] * HOP) and zero beyond, where its frames were not computed
+__global__ void overlap_add_kernel(const float* __restrict__ y, int frames, const float* __restrict__ win_sq, int L_out,
+                                   const int* __restrict__ lens, float* __restrict__ out) {
+  const int b = blockIdx.y;
+  const int t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= L_out) return;
+  if (lens && t >= __ldg(lens + b) * HOP) { out[(long long)b * L_out + t] = 0.0f; return; }
+  out[(long long)b * L_out + t] = overlap_add_at(y, frames, win_sq, b, t);
+}
+
+// overlap_add_kernel of a batch with a strength per item: an item with on[b] == 0 (on != nullptr) was not transformed and gets
+// its input audio (B, L_in) unchanged, on [0, lens[b] * HOP) and zero beyond when lens != nullptr
+__global__ void overlap_add_items_kernel(const float* __restrict__ y, int frames, const float* __restrict__ win_sq, int L_out,
+                                         const int* __restrict__ lens, const float* __restrict__ audio, int L_in,
+                                         const unsigned char* __restrict__ on, float* __restrict__ out) {
+  const int b = blockIdx.y;
+  const int t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= L_out) return;
+  float v = 0.0f;
+  if (!lens || t < __ldg(lens + b) * HOP)
+    v = (on && !__ldg(on + b)) ? audio[(long long)b * L_in + t] : overlap_add_at(y, frames, win_sq, b, t);
+  out[(long long)b * L_out + t] = v;
 }
 
 // ---------------------------------------------------------------------------------------------- FFT path
@@ -146,15 +165,24 @@ __device__ __forceinline__ float2* fft1024(float2* a, float2* b, const float2* t
   return b;
 }
 
+// A strength per item (ev_denoise_items, ev_to_waveform_items): item b is denoised with s[b], or not at all when on != nullptr
+// and on[b] == 0.  The kernels take either this or one float for the batch; both give an item the same bits.
+struct ItemStrengths { const float* s; const unsigned char* on; };
+__device__ __forceinline__ float strength_of(float s, int) { return s; }
+__device__ __forceinline__ float strength_of(const ItemStrengths& s, int b) { return __ldg(s.s + b); }
+__device__ __forceinline__ bool denoised(float, int) { return true; }
+__device__ __forceinline__ bool denoised(const ItemStrengths& s, int b) { return !s.on || __ldg(s.on + b); }
+
 // One block per pair of frames (f0, f0 + 1), f0 even, 256 threads.  audio (B, L); y (B, frames, 1024) windowed inverse frames
 // (bias != nullptr); mag0_out (B, 513): magnitude of frame 0 (the bias spectrum of ev_denoiser_init).
-//   RAGGED = false: grid (ceil(frames / 2), B), every pair of every item.
+//   RAGGED = false: grid (ceil(frames / 2), B), every pair of every denoised item.
 //   RAGGED = true: grid B * ceil(frames / 2), block i computes entry i of the compact (item, pair) list of ragged_build_table
 //   (pairs[0] = its length, pairs[1 + i] = b << 16 | pair index) and blocks past its end exit.
 // Both variants run the same per-pair code, so a pair's result does not depend on which of them computed it.
-template <bool RAGGED>
+// S = float (one strength for the batch) or ItemStrengths; the scalar instantiations are the kernels of a single strength.
+template <bool RAGGED, typename S = float>
 __global__ void __launch_bounds__(256, RAGGED ? 3 : 0) denoise_fft_kernel(const float* __restrict__ audio, int L, int frames, const float2* __restrict__ tw,
-                                                          const float* __restrict__ bias, float strength, float* __restrict__ y,
+                                                          const float* __restrict__ bias, S strength, float* __restrict__ y,
                                                           float* __restrict__ mag0_out, const int* __restrict__ pairs) {
   __shared__ float2 buf0[NFFT], buf1[NFFT];
   int b = blockIdx.y, f0 = blockIdx.x * 2;
@@ -162,6 +190,8 @@ __global__ void __launch_bounds__(256, RAGGED ? 3 : 0) denoise_fft_kernel(const 
     if ((int)blockIdx.x >= __ldg(pairs)) return;
     const int e = __ldg(pairs + 1 + blockIdx.x);
     b = e >> 16; f0 = (e & 0xffff) * 2;
+  } else if (!denoised(strength, b)) {
+    return;                                                 // (the ragged list holds denoised items only)
   }
   const int f1 = f0 + 1, j = threadIdx.x;
   const float* xb = audio + (long long)b * L;
@@ -191,8 +221,10 @@ __global__ void __launch_bounds__(256, RAGGED ? 3 : 0) denoise_fft_kernel(const 
     const float ma = sqrtf(xa.x * xa.x + xa.y * xa.y), mc = sqrtf(xc.x * xc.x + xc.y * xc.y);   // denoiser.py:33
     if (mag0_out && f0 == 0) mag0_out[(long long)b * NBIN + k] = ma;
     if (bias) {
-      const float cut = __ldg(bias + k) * strength;
-      const float sa = ma > 0.0f ? fmaxf(ma - cut, 0.0f) / ma : 0.0f, sc = mc > 0.0f ? fmaxf(mc - cut, 0.0f) / mc : 0.0f;
+      // m - bias * strength in one rounding (a fused multiply-add), spelled out: the compiler contracts it so in the scalar
+      // kernels, and an instantiation that loads the strength must round the same way to give an item the same bits
+      const float nb = -__ldg(bias + k), st = strength_of(strength, b);
+      const float sa = ma > 0.0f ? fmaxf(__fmaf_rn(nb, st, ma), 0.0f) / ma : 0.0f, sc = mc > 0.0f ? fmaxf(__fmaf_rn(nb, st, mc), 0.0f) / mc : 0.0f;
       xa.x *= sa; xa.y *= sa; xc.x *= sc; xc.y *= sc;
       if (k == 0 || k == NFFT / 2) { xa.y = 0.0f; xc.y = 0.0f; }                  // c2r ignores the imaginary part of DC / Nyquist
       O[k] = make_float2(xa.x - xc.y, xa.y + xc.x);                               // xa + i xc
@@ -224,6 +256,25 @@ __global__ void ragged_lengths_kernel(const long long* __restrict__ lengths, int
   if (wide) wide[b] = min(n + extra, max_len);
 }
 
+// Mel frames past len_b that the denoised samples [0, len_b * HOP) depend on (DESIGN.md §4, ragged batches): sample t < len*HOP
+// is an overlap-add of frames f <= len + 1; frame f shares its FFT with its pair partner, so pairs (f0, f0 + 1), f0 <= len + 1,
+// are computed, and their windows read audio below (len + 2) * HOP + NFFT / 2 = (len + 4) * HOP.
+constexpr int kDenoiseReach = 4;
+
+// ragged_lengths_kernel of a batch with a strength per item.  lens32[b] = clamp(lengths[b], 0, max_len); table[b] = the STFT
+// frames whose pairs are listed: lens32[b] + 2 for a denoised item, 0 (no pairs) for one that is not; wide (optional) = the
+// frames the vocoder must get right: min(lens32[b] + kDenoiseReach, max_len) for a denoised item, lens32[b] for one that is not
+__global__ void item_lengths_kernel(const long long* __restrict__ lengths, const unsigned char* __restrict__ on, int B, int max_len,
+                                    int* __restrict__ lens32, int* __restrict__ table, long long* __restrict__ wide) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  const int n = (int)min(max(lengths[b], 0LL), (long long)max_len);
+  const bool dn = !on || on[b];
+  lens32[b] = n;
+  table[b] = dn ? n + kDenoiseReach - 2 : 0;
+  if (wide) wide[b] = dn ? min(n + kDenoiseReach, max_len) : n;
+}
+
 int ensure_basis(ev_ctx* ctx, cudaStream_t s) {
   DenoiseBasis& d = ctx->hifigan.dn;
   if (d.ready) return 0;
@@ -249,9 +300,10 @@ int ensure_basis(ev_ctx* ctx, cudaStream_t s) {
   return 0;
 }
 
-struct DnBuffers { float* padded; float* spec; float* frames_t; int* lens32; int* pairs; long long pad_ld; int frames; };
+// table (batches with a strength per item only): the frames item_lengths_kernel lists pairs for
+struct DnBuffers { float* padded; float* spec; float* frames_t; int* lens32; int* table; int* pairs; long long pad_ld; int frames; };
 
-void plan(int B, int L, Workspace& w, DnBuffers* d) {
+void plan(int B, int L, Workspace& w, DnBuffers* d, bool items = false) {
   d->frames = L / HOP + 1;
   d->pad_ld = (long long)(d->frames + 3) * HOP;                 // rows of 256 samples, 3 extra rows for the 4 taps
   d->padded = w.take<float>((size_t)B * d->pad_ld);
@@ -259,12 +311,25 @@ void plan(int B, int L, Workspace& w, DnBuffers* d) {
   d->frames_t = w.take<float>((size_t)B * d->frames * NFFT);
   d->lens32 = w.take<int>((size_t)B);                           // ragged batch: lengths and the compact pair list
   d->pairs = w.take<int>((size_t)B * ceil_div(d->frames, 2) + 1);
+  d->table = items ? w.take<int>((size_t)B) : nullptr;
 }
 
-// Mel frames past len_b that the denoised samples [0, len_b * HOP) depend on (DESIGN.md §4, ragged batches): sample t < len*HOP
-// is an overlap-add of frames f <= len + 1; frame f shares its FFT with its pair partner, so pairs (f0, f0 + 1), f0 <= len + 1,
-// are computed, and their windows read audio below (len + 2) * HOP + NFFT / 2 = (len + 4) * HOP.
-constexpr int kDenoiseReach = 4;
+bool use_fft() {
+  static const bool v = []() { const char* e = getenv("EV_DN_FFT"); return !(e && atoi(e) == 0); }();
+  return v;
+}
+
+constexpr double kPairFlops = 2.0 * 5.0 * NFFT * 10.0;
+
+// The length of the compact pair list (instrumented eager runs only, where a host copy is fine): the algorithmic work
+int listed_pairs(ev_ctx* ctx, const int* pairs, double* n_pairs, cudaStream_t s) {
+  if (!ctx->profiling) return 0;
+  int n = 0;
+  EV_CUDA(ctx, cudaMemcpyAsync(&n, pairs, sizeof(int), cudaMemcpyDeviceToHost, s));
+  EV_CUDA(ctx, cudaStreamSynchronize(s));
+  *n_pairs = n;
+  return 0;
+}
 
 // STFT of `audio` (B, L) into d.spec (re|im); when bias != nullptr also denoise + ISTFT into out (B, HOP*(L/HOP)).
 // lens32 (ragged batch, bias != nullptr, or nullptr): only the pairs that item b's samples [0, lens32[b] * HOP) read are
@@ -273,28 +338,22 @@ int stft_pipeline(ev_ctx* ctx, const float* audio, int B, int L, const float* bi
                   const int* lens32, DnBuffers& d, cudaStream_t s) {
   DenoiseBasis& bs = ctx->hifigan.dn;
   const int frames = d.frames;
-  static const bool use_fft = []() { const char* v = getenv("EV_DN_FFT"); return !(v && atoi(v) == 0); }();
-  const double pair_flops = 2.0 * 5.0 * NFFT * 10.0;
-  if (use_fft && lens32 && bias) {
+  const double pair_flops = kPairFlops;
+  if (use_fft() && lens32 && bias) {
     // frames [0, lens32[b] + 2) in pairs: ceil((len + 2) / 2) = floor((len + 1) / 2) + 1 pairs, all of them when len = frames - 1
     EV_LAUNCH(ctx, s, "ragged_table", 0, 8.0 * B, ragged_build_table(lens32, B, kDenoiseReach - 2, 1, 0, 2, frames, d.pairs, s));
     double n_pairs = (double)B * ceil_div(frames, 2);
-    if (ctx->profiling) {   // algorithmic work = the listed pairs (instrumented eager run: a host copy is fine here)
-      int n = 0;
-      EV_CUDA(ctx, cudaMemcpyAsync(&n, d.pairs, sizeof(int), cudaMemcpyDeviceToHost, s));
-      EV_CUDA(ctx, cudaStreamSynchronize(s));
-      n_pairs = n;
-    }
+    EV_TRY(listed_pairs(ctx, d.pairs, &n_pairs, s));
     EV_LAUNCH(ctx, s, "denoise_fft_ragged", pair_flops * n_pairs, 4.0 * n_pairs * 2.0 * (HOP + NFFT),
               (denoise_fft_kernel<true><<<B * ceil_div(frames, 2), 256, 0, s>>>(audio, L, frames, reinterpret_cast<const float2*>(bs.twiddle), bias,
                                                                                 strength, d.frames_t, nullptr, d.pairs), cudaGetLastError()));
-  } else if (use_fft) {
+  } else if (use_fft()) {
     const double fft_flops = pair_flops * ceil_div(frames, 2) * B;
     EV_LAUNCH(ctx, s, "denoise_fft", fft_flops, 4.0 * B * ((double)L + (bias ? (double)frames * NFFT : NBIN)),
               (denoise_fft_kernel<false><<<dim3(ceil_div(frames, 2), B), 256, 0, s>>>(audio, L, frames, reinterpret_cast<const float2*>(bs.twiddle), bias,
                                                                                      strength, d.frames_t, mag0, nullptr), cudaGetLastError()));
   }
-  if (use_fft) {
+  if (use_fft()) {
     if (!bias) return 0;
     const int L_out = HOP * (frames - 1);
     EV_LAUNCH(ctx, s, "overlap_add", 0, 4.0 * B * (4.0 * L_out + L_out),
@@ -330,18 +389,75 @@ int stft_pipeline(ev_ctx* ctx, const float* audio, int B, int L, const float* bi
   return 0;
 }
 
+// The FFT denoiser with a strength per item: `audio` (B, L) -> out (B, HOP*(L/HOP)).  lens32 (ragged batch, with d.table from
+// item_lengths_kernel, or nullptr): as stft_pipeline's, the listed pairs are those of the denoised items only.  An item that is
+// not denoised gets its audio (see overlap_add_items_kernel).  A denoised item's bits are those of stft_pipeline at its strength.
+int denoise_items(ev_ctx* ctx, const float* audio, int B, int L, ItemStrengths st, const int* lens32, const DnBuffers& d, float* out,
+                  cudaStream_t s) {
+  const DenoiseBasis& bs = ctx->hifigan.dn;
+  const float* bias = ctx->hifigan.denoise_bias;
+  const float2* tw = reinterpret_cast<const float2*>(bs.twiddle);
+  const int frames = d.frames, L_out = HOP * (frames - 1);
+  if (lens32) {
+    EV_LAUNCH(ctx, s, "ragged_table", 0, 8.0 * B, ragged_build_table(d.table, B, 0, 1, 0, 2, frames, d.pairs, s));
+    double n_pairs = (double)B * ceil_div(frames, 2);
+    EV_TRY(listed_pairs(ctx, d.pairs, &n_pairs, s));
+    EV_LAUNCH(ctx, s, "denoise_fft_ragged", kPairFlops * n_pairs, 4.0 * n_pairs * 2.0 * (HOP + NFFT),
+              (denoise_fft_kernel<true, ItemStrengths><<<B * ceil_div(frames, 2), 256, 0, s>>>(audio, L, frames, tw, bias, st, d.frames_t, nullptr,
+                                                                                               d.pairs), cudaGetLastError()));
+  } else {
+    EV_LAUNCH(ctx, s, "denoise_fft", kPairFlops * ceil_div(frames, 2) * B, 4.0 * B * ((double)L + (double)frames * NFFT),
+              (denoise_fft_kernel<false, ItemStrengths><<<dim3(ceil_div(frames, 2), B), 256, 0, s>>>(audio, L, frames, tw, bias, st, d.frames_t,
+                                                                                                     nullptr, nullptr), cudaGetLastError()));
+  }
+  EV_LAUNCH(ctx, s, "overlap_add", 0, 4.0 * B * (4.0 * L_out + L_out),
+            (overlap_add_items_kernel<<<dim3(ceil_div(L_out, 256), B), 256, 0, s>>>(d.frames_t, frames, bs.win_sq, L_out, lens32, audio, L, st.on, out),
+             cudaGetLastError()));
+  return 0;
+}
+
 // ev_to_waveform_ragged's workspace: widened lengths, the vocoded batch, the denoiser's buffers, the vocoder's workspace
 struct WavBuffers { long long* wide; float* audio; DnBuffers d; char* voc_ws; size_t voc_bytes; };
 
-void plan_to_waveform(const ev_ctx* ctx, int B, int T, Workspace& w, WavBuffers* t) {
+void plan_to_waveform(const ev_ctx* ctx, int B, int T, Workspace& w, WavBuffers* t, bool items = false) {
   t->wide = w.take<long long>((size_t)B);
   t->audio = w.take<float>((size_t)B * T * HOP);
-  plan(B, T * HOP, w, &t->d);
+  plan(B, T * HOP, w, &t->d, items);
   t->voc_bytes = ev_vocode_workspace_bytes(ctx, B, T);
   t->voc_ws = w.take<char>(t->voc_bytes);
 }
 
 bool ragged_lists_fit(int B, int frames) { return B <= kRaggedMaxB && ceil_div(frames, 2) < 65536; }
+
+// The argument checks of ev_denoise_ragged / ev_denoise_items (`name` prefixes the message)
+int check_denoise_args(ev_ctx* ctx, const char* name, const float* audio, const int64_t* lengths, int B, int L, const float* out) {
+  if (!ctx->hifigan.denoise_bias) return fail(ctx, EV_ERR_STATE, "ev_denoise: call ev_denoiser_init first");
+  if (!audio || !out || B <= 0 || L < NFFT / 2 + 1) return fail(ctx, EV_ERR_INVALID, "ev_denoise: null argument or audio shorter than the reflect padding");
+  if (lengths && !ragged_lists_fit(B, L / HOP + 1)) return fail(ctx, EV_ERR_INVALID, std::string(name) + ": batch or audio too long for the ragged pair list");
+  return 0;
+}
+
+// The argument checks of ev_to_waveform_ragged / ev_to_waveform_items
+int check_to_waveform_args(ev_ctx* ctx, const char* name, const float* mel, const int64_t* mel_lengths, int B, int T, int precision,
+                           const float* wav) {
+  const HifiganW& h = ctx->hifigan;
+  const std::string n(name);
+  if (!h.loaded) return fail(ctx, EV_ERR_STATE, n + ": hifigan weights not loaded");
+  if (!h.denoise_bias) return fail(ctx, EV_ERR_STATE, n + ": call ev_denoiser_init first");
+  if (!mel || !mel_lengths || !wav || B <= 0 || T <= 0) return fail(ctx, EV_ERR_INVALID, n + ": null argument or empty shape");
+  if (h.total_up != HOP) return fail(ctx, EV_ERR_INVALID, n + ": the generator's hop must equal the denoiser's (256)");
+  if (T * HOP < NFFT / 2 + 1) return fail(ctx, EV_ERR_INVALID, n + ": T < 3 frames is shorter than the reflect padding");
+  if (!ragged_lists_fit(B, T + 1)) return fail(ctx, EV_ERR_INVALID, n + ": batch or T too large for the ragged pair list");
+  if (precision != EV_PREC_FP32 && precision != EV_PREC_BF16) return fail(ctx, EV_ERR_INVALID, n + ": unknown precision");
+  return 0;
+}
+
+// Per-item strengths are an input of the FFT kernel only; the GEMM cross-check path (EV_DN_FFT=0) takes one strength per call
+int check_items_path(ev_ctx* ctx, const char* name, const float* strengths) {
+  if (!strengths) return fail(ctx, EV_ERR_INVALID, std::string(name) + ": null strengths");
+  if (!use_fft()) return fail(ctx, EV_ERR_INVALID, std::string(name) + ": per-item strengths need the FFT denoiser (EV_DN_FFT=0 selects the GEMM path, which takes one strength per call)");
+  return 0;
+}
 }  // namespace
 
 extern "C" size_t ev_denoise_workspace_bytes(const ev_ctx* ctx, int B, int L) {
@@ -383,9 +499,7 @@ extern "C" int ev_denoiser_init(ev_ctx* ctx, float* bias_spec_out, void* workspa
 extern "C" int ev_denoise_ragged(ev_ctx* ctx, const float* audio, const int64_t* lengths, int B, int L, float strength, float* out,
                                  void* workspace, size_t workspace_bytes, void* stream) {
   if (!ctx) return EV_ERR_INVALID;
-  if (!ctx->hifigan.denoise_bias) return fail(ctx, EV_ERR_STATE, "ev_denoise: call ev_denoiser_init first");
-  if (!audio || !out || B <= 0 || L < NFFT / 2 + 1) return fail(ctx, EV_ERR_INVALID, "ev_denoise: null argument or audio shorter than the reflect padding");
-  if (lengths && !ragged_lists_fit(B, L / HOP + 1)) return fail(ctx, EV_ERR_INVALID, "ev_denoise_ragged: batch or audio too long for the ragged pair list");
+  EV_TRY(check_denoise_args(ctx, "ev_denoise_ragged", audio, lengths, B, L, out));
   cudaStream_t s = as_stream(stream);
   EV_CUDA(ctx, cudaSetDevice(ctx->device));
   EV_TRY(ensure_basis(ctx, s));
@@ -405,6 +519,33 @@ extern "C" int ev_denoise(ev_ctx* ctx, const float* audio, int B, int L, float s
   return ev_denoise_ragged(ctx, audio, nullptr, B, L, strength, out, workspace, workspace_bytes, stream);
 }
 
+extern "C" size_t ev_denoise_items_workspace_bytes(const ev_ctx* ctx, int B, int L) {
+  if (!ctx || B <= 0 || L <= 0) return 0;
+  Workspace w(nullptr, 0);
+  DnBuffers d;
+  plan(B, L, w, &d, true);
+  return w.off + 256;
+}
+
+extern "C" int ev_denoise_items(ev_ctx* ctx, const float* audio, const int64_t* lengths, int B, int L, const float* strengths,
+                                const uint8_t* denoise, float* out, void* workspace, size_t workspace_bytes, void* stream) {
+  if (!ctx) return EV_ERR_INVALID;
+  EV_TRY(check_denoise_args(ctx, "ev_denoise_items", audio, lengths, B, L, out));
+  EV_TRY(check_items_path(ctx, "ev_denoise_items", strengths));
+  cudaStream_t s = as_stream(stream);
+  EV_CUDA(ctx, cudaSetDevice(ctx->device));
+  EV_TRY(ensure_basis(ctx, s));
+  Workspace w(workspace, workspace_bytes);
+  DnBuffers d;
+  plan(B, L, w, &d, true);
+  if (w.overflow || !workspace) return fail(ctx, EV_ERR_STATE, "ev_denoise_items: workspace too small");
+  if (lengths)
+    EV_LAUNCH(ctx, s, "ragged_lengths", 0, 13.0 * B,
+              (item_lengths_kernel<<<ceil_div(B, 256), 256, 0, s>>>(reinterpret_cast<const long long*>(lengths), denoise, B, L / HOP, d.lens32,
+                                                                   d.table, nullptr), cudaGetLastError()));
+  return denoise_items(ctx, audio, B, L, ItemStrengths{strengths, denoise}, lengths ? d.lens32 : nullptr, d, out, s);
+}
+
 extern "C" size_t ev_to_waveform_ragged_workspace_bytes(const ev_ctx* ctx, int B, int T) {
   if (!ctx || !ctx->hifigan.loaded || B <= 0 || T <= 0) return 0;
   Workspace w(nullptr, 0);
@@ -416,14 +557,8 @@ extern "C" size_t ev_to_waveform_ragged_workspace_bytes(const ev_ctx* ctx, int B
 extern "C" int ev_to_waveform_ragged(ev_ctx* ctx, const float* mel, const int64_t* mel_lengths, int B, int T, int precision, float strength,
                                      float* wav, void* workspace, size_t workspace_bytes, void* stream) {
   if (!ctx) return EV_ERR_INVALID;
+  EV_TRY(check_to_waveform_args(ctx, "ev_to_waveform_ragged", mel, mel_lengths, B, T, precision, wav));
   const HifiganW& h = ctx->hifigan;
-  if (!h.loaded) return fail(ctx, EV_ERR_STATE, "ev_to_waveform_ragged: hifigan weights not loaded");
-  if (!h.denoise_bias) return fail(ctx, EV_ERR_STATE, "ev_to_waveform_ragged: call ev_denoiser_init first");
-  if (!mel || !mel_lengths || !wav || B <= 0 || T <= 0) return fail(ctx, EV_ERR_INVALID, "ev_to_waveform_ragged: null argument or empty shape");
-  if (h.total_up != HOP) return fail(ctx, EV_ERR_INVALID, "ev_to_waveform_ragged: the generator's hop must equal the denoiser's (256)");
-  if (T * HOP < NFFT / 2 + 1) return fail(ctx, EV_ERR_INVALID, "ev_to_waveform_ragged: T < 3 frames is shorter than the reflect padding");
-  if (!ragged_lists_fit(B, T + 1)) return fail(ctx, EV_ERR_INVALID, "ev_to_waveform_ragged: batch or T too large for the ragged pair list");
-  if (precision != EV_PREC_FP32 && precision != EV_PREC_BF16) return fail(ctx, EV_ERR_INVALID, "ev_to_waveform_ragged: unknown precision");
   cudaStream_t s = as_stream(stream);
   EV_CUDA(ctx, cudaSetDevice(ctx->device));
   EV_TRY(ensure_basis(ctx, s));
@@ -437,4 +572,33 @@ extern "C" int ev_to_waveform_ragged(ev_ctx* ctx, const float* mel, const int64_
                                                                      t.d.lens32, t.wide), cudaGetLastError()));
   EV_TRY(ev_vocode_ragged(ctx, mel, reinterpret_cast<const int64_t*>(t.wide), B, T, precision, t.audio, t.voc_ws, t.voc_bytes, stream));
   return stft_pipeline(ctx, t.audio, B, T * HOP, h.denoise_bias, strength, nullptr, wav, t.d.lens32, t.d, s);
+}
+
+extern "C" size_t ev_to_waveform_items_workspace_bytes(const ev_ctx* ctx, int B, int T) {
+  if (!ctx || !ctx->hifigan.loaded || B <= 0 || T <= 0) return 0;
+  Workspace w(nullptr, 0);
+  WavBuffers t;
+  plan_to_waveform(ctx, B, T, w, &t, true);
+  return w.off + 256;
+}
+
+extern "C" int ev_to_waveform_items(ev_ctx* ctx, const float* mel, const int64_t* mel_lengths, int B, int T, int precision,
+                                    const float* strengths, const uint8_t* denoise, float* wav, void* workspace, size_t workspace_bytes,
+                                    void* stream) {
+  if (!ctx) return EV_ERR_INVALID;
+  EV_TRY(check_to_waveform_args(ctx, "ev_to_waveform_items", mel, mel_lengths, B, T, precision, wav));
+  EV_TRY(check_items_path(ctx, "ev_to_waveform_items", strengths));
+  cudaStream_t s = as_stream(stream);
+  EV_CUDA(ctx, cudaSetDevice(ctx->device));
+  EV_TRY(ensure_basis(ctx, s));
+  Workspace w(workspace, workspace_bytes);
+  WavBuffers t;
+  plan_to_waveform(ctx, B, T, w, &t, true);
+  if (w.overflow || !workspace) return fail(ctx, EV_ERR_STATE, "ev_to_waveform_items: workspace too small");
+  // a denoised item needs the vocoder exact on min(len + reach, T) frames, one that is not only on its own len
+  EV_LAUNCH(ctx, s, "ragged_lengths", 0, 25.0 * B,
+            (item_lengths_kernel<<<ceil_div(B, 256), 256, 0, s>>>(reinterpret_cast<const long long*>(mel_lengths), denoise, B, T, t.d.lens32,
+                                                                 t.d.table, t.wide), cudaGetLastError()));
+  EV_TRY(ev_vocode_ragged(ctx, mel, reinterpret_cast<const int64_t*>(t.wide), B, T, precision, t.audio, t.voc_ws, t.voc_bytes, stream));
+  return denoise_items(ctx, t.audio, B, T * HOP, ItemStrengths{strengths, denoise}, t.d.lens32, t.d, wav, s);
 }

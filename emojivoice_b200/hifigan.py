@@ -3,6 +3,7 @@
 from __future__ import annotations
 
 import ctypes as C
+import numbers
 
 import torch
 
@@ -108,30 +109,45 @@ class Generator:
         lengths[b] + 4 frames (all the denoised samples read) and the denoiser transforms only the STFT frames of each
         utterance's own samples (ev_to_waveform_ragged).  A Denoiser built on this generator must exist (it holds the bias
         spectrum).  lengths (B,) valid mel frames per item; lengths given on the host must lie in [1, T] (device tensors are
-        clamped to [0, T] on the device, as checking them would synchronise)."""
-        return self._run(mel, dtype, lengths, float(strength))
+        clamped to [0, T] on the device, as checking them would synchronise).
+
+        strength: a number for the whole batch, or a (B,) sequence / tensor with one per utterance, in which None means "not
+        denoised" (see `per_item_strength`).  Utterance b then gets, bit for bit, this call with its own strength, or
+        `self(mel, lengths=lengths)[b]` when it is not denoised (ev_to_waveform_items); strength 0 is not the same as None."""
+        s = per_item_strength(strength, mel.shape[0] if mel.dim() == 3 else 1)
+        if s is None:                     # no utterance is denoised: the ragged generator alone
+            check_lengths(lengths, mel.shape[-1])
+        return self._run(mel, dtype, lengths, s if s is None or isinstance(s, tuple) else float(s))
 
     def _run(self, mel, dtype, lengths, strength):
-        """ev_vocode_ragged (strength None) or ev_to_waveform_ragged, replayed as a CUDA graph once a call shape repeats."""
+        """ev_vocode_ragged (strength None), ev_to_waveform_ragged (a number) or ev_to_waveform_items (a tuple with None for the
+        items not denoised), replayed as a CUDA graph once a call shape repeats."""
         self._materialise()
         ctx, L = self._ctx, _lib.lib()
         dev = ctx.device
         denoise = strength is not None
+        items = isinstance(strength, tuple)
         if mel.dim() == 2:
             mel = mel.unsqueeze(0)
         with torch.cuda.device(dev):
             mel = mel.to(device=dev, dtype=torch.float32).contiguous()
             B, _, T = mel.shape
             prec = _lib.PREC[dtype if dtype is not None else self.precision]
-            nb = (L.ev_to_waveform_ragged_workspace_bytes if denoise else L.ev_vocode_workspace_bytes)(ctx.handle, B, T)
+            nb = (L.ev_to_waveform_items_workspace_bytes if items else L.ev_to_waveform_ragged_workspace_bytes if denoise
+                  else L.ev_vocode_workspace_bytes)(ctx.handle, B, T)
             if denoise:
                 check_lengths(lengths, T)
             if lengths is not None:
                 lengths = torch.as_tensor(lengths).reshape(-1).to(device=dev, dtype=torch.int64).contiguous()
                 if lengths.numel() != B:
                     raise ValueError(f"lengths has {lengths.numel()} entries for a batch of {B}")
+            st = strength_tensors(strength, dev) if items else (None, None)
 
-            def call(mel_, wav_, ws_, len_=None):
+            def call(mel_, wav_, ws_, len_=None, st_=(None, None)):
+                if items:
+                    ctx.check(L.ev_to_waveform_items(ctx.handle, _lib.ptr(mel_), _lib.ptr(len_), B, T, prec, _lib.ptr(st_[0]), _lib.ptr(st_[1]),
+                                                     _lib.ptr(wav_), _lib.ptr(ws_), ws_.numel(), _lib.stream_ptr()), "ev_to_waveform_items")
+                    return
                 if denoise:
                     ctx.check(L.ev_to_waveform_ragged(ctx.handle, _lib.ptr(mel_), _lib.ptr(len_), B, T, prec, strength, _lib.ptr(wav_),
                                                       _lib.ptr(ws_), ws_.numel(), _lib.stream_ptr()), "ev_to_waveform_ragged")
@@ -139,21 +155,25 @@ class Generator:
                 ctx.check(L.ev_vocode_ragged(ctx.handle, _lib.ptr(mel_), _lib.ptr(len_) if len_ is not None else None, B, T, prec,
                                              _lib.ptr(wav_), _lib.ptr(ws_), ws_.numel(), _lib.stream_ptr()), "ev_vocode")
 
-            key = (B, T, prec, lengths is not None) + ((strength,) if denoise else ())
+            # per-item strengths and flags are static inputs of the graph: a replay reads the values of its own call
+            key = (B, T, prec, lengths is not None) + (("items",) if items else (strength,) if denoise else ())
             ws_shared = ctx.workspace(nb)                   # (may grow the workspace: do it before looking graphs up)
             ent = self._graphs.get(key, ctx.ws_version) if self.cuda_graphs else None
             if ent is None and self.cuda_graphs and self._graphs.should_capture(key):
                 ent = dict(mel=mel.clone(), wav=torch.empty(B, 1, T * self.hop, device=dev), ws=ws_shared, ws_version=ctx.ws_version,
-                           len=lengths.clone() if lengths is not None else None)
-                ent["graph"], ent["launches"] = _lib.capture(ctx, lambda: call(ent["mel"], ent["wav"], ent["ws"], ent["len"]))
+                           len=lengths.clone() if lengths is not None else None, st=tuple(t.clone() if t is not None else None for t in st))
+                ent["graph"], ent["launches"] = _lib.capture(ctx, lambda: call(ent["mel"], ent["wav"], ent["ws"], ent["len"], ent["st"]))
                 self._graphs.put(key, ent)
             if ent is None:
                 wav = torch.empty(B, 1, T * self.hop, device=dev)
-                call(mel, wav, ws_shared, lengths)
+                call(mel, wav, ws_shared, lengths, st)
             else:
                 ent["mel"].copy_(mel)
                 if lengths is not None:
                     ent["len"].copy_(lengths)
+                if items:
+                    for dst, src in zip(ent["st"], st):
+                        dst.copy_(src)
                 ent["graph"].replay()
                 self._replayed_launches += ent["launches"]
                 wav = ent["wav"].clone()
@@ -176,6 +196,34 @@ def check_lengths(lengths, max_len):
     t = torch.as_tensor(lengths).reshape(-1)
     if t.numel() and (int(t.min()) < 1 or int(t.max()) > max_len):
         raise ValueError(f"lengths must lie in [1, {max_len}] frames, got [{int(t.min())}, {int(t.max())}]")
+
+
+def per_item_strength(value, B):
+    """The denoiser setting of a batch of B utterances: a number for the whole batch, None for "not denoised", or a (B,)
+    sequence / tensor with one of those per utterance.  -> the number, None when no utterance is denoised, or a tuple of B
+    floats and Nones; values that are all equal are the number, as MatchaTTS.synthesise does with its settings
+    (matcha.per_item_setting, whose rules the per-utterance strengths follow: finite numbers, since the library reads them on
+    the device)."""
+    from .matcha import per_item_setting
+
+    if value is None or isinstance(value, numbers.Number) or (torch.is_tensor(value) and value.dim() == 0):
+        return value.item() if torch.is_tensor(value) else value
+    vals = value.detach().reshape(-1).tolist() if torch.is_tensor(value) else list(value)
+    if len(vals) != B:
+        raise ValueError(f"strength: expected a number or {B} values (one per utterance), got {len(vals)}")
+    on = [v for v in vals if v is not None]
+    if not on:
+        return None
+    per_item_setting(on, len(on), "strength")
+    vals = [None if v is None else float(v) for v in vals]
+    return vals[0] if all(v == vals[0] for v in vals) else tuple(vals)
+
+
+def strength_tensors(strengths, device):
+    """A tuple of per_item_strength -> (strengths (B,) fp32, flags (B,) uint8: 0 = not denoised) on the device."""
+    s = torch.tensor([0.0 if v is None else v for v in strengths], dtype=torch.float32)
+    on = torch.tensor([v is not None for v in strengths], dtype=torch.uint8)
+    return s.to(device), on.to(device)
 
 
 class Denoiser:
@@ -201,11 +249,16 @@ class Denoiser:
     def __call__(self, audio, strength=0.0005, lengths=None):
         """lengths (B,) optional: valid mel frames per item of a padded batch, as `mel_lengths`.  Item b is then bit-identical
         to the call without lengths on [: lengths[b]*256] and zero beyond, and only the STFT frames those samples reach are
-        transformed (ev_denoise_ragged).  Lengths given on the host must lie in [1, n // 256]."""
+        transformed (ev_denoise_ragged).  Lengths given on the host must lie in [1, n // 256].
+
+        strength: a number, or a (B,) sequence / tensor with one per item in which None means "not denoised" (see
+        `per_item_strength`).  Item b then gets, bit for bit, this call with its own strength, or its input truncated to
+        (n // 256) * 256 samples (and zero past lengths[b]*256) when it is not denoised (ev_denoise_items)."""
         ctx, L = self.vocoder._ctx, _lib.lib()
         squeeze = audio.dim() == 1
         a = audio.reshape(-1, audio.shape[-1]).to(device=self.device, dtype=torch.float32).contiguous()
         B, n = a.shape
+        s = per_item_strength(strength, B)
         out = torch.empty(B, (n // 256) * 256, device=self.device)
         with torch.cuda.device(self.device):
             if lengths is not None:
@@ -213,9 +266,15 @@ class Denoiser:
                 lengths = torch.as_tensor(lengths).reshape(-1).to(device=self.device, dtype=torch.int64).contiguous()
                 if lengths.numel() != B:
                     raise ValueError(f"lengths has {lengths.numel()} entries for a batch of {B}")
-            ws = ctx.workspace(L.ev_denoise_workspace_bytes(ctx.handle, B, n))
-            ctx.check(L.ev_denoise_ragged(ctx.handle, _lib.ptr(a), _lib.ptr(lengths), B, n, float(strength), _lib.ptr(out), _lib.ptr(ws),
-                                          ws.numel(), _lib.stream_ptr()), "ev_denoise")
+            if s is not None and not isinstance(s, tuple):
+                ws = ctx.workspace(L.ev_denoise_workspace_bytes(ctx.handle, B, n))
+                ctx.check(L.ev_denoise_ragged(ctx.handle, _lib.ptr(a), _lib.ptr(lengths), B, n, float(s), _lib.ptr(out), _lib.ptr(ws),
+                                              ws.numel(), _lib.stream_ptr()), "ev_denoise")
+            else:
+                st, on = strength_tensors(s if s is not None else (None,) * B, self.device)
+                ws = ctx.workspace(L.ev_denoise_items_workspace_bytes(ctx.handle, B, n))
+                ctx.check(L.ev_denoise_items(ctx.handle, _lib.ptr(a), _lib.ptr(lengths), B, n, _lib.ptr(st), _lib.ptr(on), _lib.ptr(out),
+                                             _lib.ptr(ws), ws.numel(), _lib.stream_ptr()), "ev_denoise_items")
         return out[0] if squeeze else out
 
     forward = __call__

@@ -186,6 +186,25 @@ EV_API size_t ev_to_waveform_ragged_workspace_bytes(const ev_ctx* ctx, int B, in
 EV_API int ev_to_waveform_ragged(ev_ctx* ctx, const float* mel, const int64_t* mel_lengths, int B, int T, int precision,
               float strength, float* wav, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- vocoder + denoiser with a strength per item, or none -----------------------------------------------------
+ * The same calls with a denoiser setting per utterance: strengths (B) device fp32, denoise (B) device uint8 (0 = item b is
+ * not denoised; NULL = every item is).  Item b is, bit for bit,
+ *   denoised:     what ev_to_waveform_ragged / ev_denoise_ragged give it on the same batch with strength = strengths[b];
+ *   not denoised: ev_to_waveform_items: what ev_vocode_ragged gives it on the same batch and mel_lengths (the clamped generator
+ *                 output); ev_denoise_items: its audio truncated to L' = 256*(L/256) samples.
+ * Either way, on [0, lengths[b]*256) and ZERO beyond when lengths are given.  Strength 0 is not "not denoised": the STFT /
+ * ISTFT round trip changes low bits.  A not-denoised item adds no STFT frames, and ev_to_waveform_items vocodes it on
+ * mel_lengths[b] frames rather than mel_lengths[b] + 4.  Equal strengths with every item denoised are the scalar calls'
+ * results, with other kernels; callers that hold equal values pass the number.  Strengths and flags stay on the device (no
+ * host synchronisation, capturable; a finite strength is the caller's duty).  Other rules as the scalar calls.  The FFT
+ * denoiser only: with EV_DN_FFT=0 (the GEMM cross-check path, one strength per call) these return EV_ERR_INVALID. */
+EV_API size_t ev_denoise_items_workspace_bytes(const ev_ctx* ctx, int B, int L);
+EV_API int ev_denoise_items(ev_ctx* ctx, const float* audio, const int64_t* lengths, int B, int L, const float* strengths,
+              const uint8_t* denoise, float* out, void* workspace, size_t workspace_bytes, void* stream);
+EV_API size_t ev_to_waveform_items_workspace_bytes(const ev_ctx* ctx, int B, int T);
+EV_API int ev_to_waveform_items(ev_ctx* ctx, const float* mel, const int64_t* mel_lengths, int B, int T, int precision,
+              const float* strengths, const uint8_t* denoise, float* wav, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- monotonic alignment search (SURVEY 8 f4; training-side, the reference's only native component) ------------
  * replaces  maximum_path_c(paths, values, t_xs, t_ys, max_neg_val)   Matcha-TTS/matcha/utils/monotonic_align/core.pyx:42-47
  * (called through monotonic_align.maximum_path, __init__.py:7-22, from MatchaTTS.forward, models/matcha_tts.py:198).
