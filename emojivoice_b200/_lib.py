@@ -68,6 +68,7 @@ SIGNATURES = {
     "ev_decode": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _F, _I, _P, _P, _P, _SZ, _P]),
     "ev_decode_items_workspace_bytes": (_SZ, [_P, _I, _I, _I]),
     "ev_decode_items": (_I, [_P, _P, _P, _P, _P, _I, _I, _P, _P, _I, _P, _P, _P, _SZ, _P]),
+    "ev_prior_noise": (_I, [_P, _P, _I, _I, _I, _P, _P]),
     "ev_vocode_workspace_bytes": (_SZ, [_P, _I, _I]),
     "ev_vocode": (_I, [_P, _P, _I, _I, _I, _P, _P, _SZ, _P]),
     "ev_vocode_ragged": (_I, [_P, _P, _P, _I, _I, _I, _P, _P, _SZ, _P]),

@@ -10,6 +10,7 @@ from . import sharding
 
 SETTINGS = ("length_scale", "temperature", "n_timesteps")
 VOCODER_SETTINGS = ("denoiser_strength",)      # per utterance too, but read after synthesis: the plan does not depend on them
+NOISE_SETTINGS = ("seed",)                     # the prior noise's seed: the plan does not depend on it either
 
 
 def collate(utterances, items):
@@ -60,16 +61,17 @@ def lanes_for(model, vocoder, n: int) -> Lanes:
 
 
 def utterance_settings(utterances, defaults):
-    """Each utterance's settings (SETTINGS and VOCODER_SETTINGS): an utterance is (ids, speaker_id) or (ids, speaker_id,
-    settings) with a dict holding any of those keys; a missing key takes its value from `defaults`.
+    """Each utterance's settings (SETTINGS, VOCODER_SETTINGS and NOISE_SETTINGS): an utterance is (ids, speaker_id) or (ids,
+    speaker_id, settings) with a dict holding any of those keys; a missing key takes its value from `defaults`.
     -> (per-utterance dicts, True when some utterance has its own synthesis settings (SETTINGS))"""
     out, own = [], False
     for u in utterances:
         s = dict(defaults)
         if len(u) > 2 and u[2]:
-            extra = set(u[2]) - set(SETTINGS) - set(VOCODER_SETTINGS)
+            known = SETTINGS + VOCODER_SETTINGS + NOISE_SETTINGS
+            extra = set(u[2]) - set(known)
             if extra:
-                raise ValueError(f"unknown per-utterance settings {sorted(extra)}; expected keys among {SETTINGS + VOCODER_SETTINGS}")
+                raise ValueError(f"unknown per-utterance settings {sorted(extra)}; expected keys among {known}")
             s.update(u[2])
             own = own or any(k in SETTINGS for k in u[2])
         out.append(s)
@@ -87,10 +89,44 @@ def denoiser_strengths(settings, denoiser):
     return dn
 
 
+def splitmix64(seed, n):
+    """The first n outputs of splitmix64 seeded with `seed` mod 2^64 (Steele, Lea and Flood 2014).  Utterance i of a corpus
+    seeded with S draws its noise from output i: consecutive seeds S + i would give corpora S and S + 1 all but one noise in
+    common, while these streams share none."""
+    m = (1 << 64) - 1
+    x, out = seed & m, []
+    for _ in range(n):
+        x = (x + 0x9E3779B97F4A7C15) & m
+        v = ((x ^ (x >> 30)) * 0xBF58476D1CE4E5B9) & m
+        v = ((v ^ (v >> 27)) * 0x94D049BB133111EB) & m
+        out.append(v ^ (v >> 31))
+    return out
+
+
+def utterance_seeds(settings, seed, z_fn=None):
+    """Each utterance's noise seed (a uint64), or None when the corpus is not seeded.  Utterance i takes its settings' "seed",
+    else output i of splitmix64(seed) when `seed` is given.  Refuses, before any work is done, a corpus in which some utterances
+    are seeded and others are not, and seeds together with z_fn (which supplies the noise itself)."""
+    from .matcha import seed_value
+
+    derived = splitmix64(seed_value(seed), len(settings)) if seed is not None else None
+    seeds = []
+    for i, s in enumerate(settings):
+        v = s.get("seed", derived[i] if derived is not None else None)
+        seeds.append(None if v is None else seed_value(v, f"utterance {i}"))
+    if all(v is None for v in seeds):
+        return None
+    if any(v is None for v in seeds):
+        raise ValueError("some utterances have a noise seed and others do not: pass seed= or give every utterance a \"seed\"")
+    if z_fn is not None:
+        raise ValueError("z_fn supplies the prior noise itself: it cannot be combined with noise seeds")
+    return seeds
+
+
 @torch.inference_mode()
 def synthesise_corpus(model, vocoder, utterances, batch_size=32, n_timesteps=10, temperature=0.667, length_scale=1.0,
                       rank=0, world_size=1, denoiser=None, denoiser_strength=0.00025, sort=True, keep_mel=False, z_fn=None,
-                      ragged=True, cuda_graphs=False, in_flight=1, lanes=None):
+                      ragged=True, cuda_graphs=False, in_flight=1, lanes=None, seed=None):
     """Synthesise this rank's share of `utterances`: a list of (phoneme ids, speaker id) or (phoneme ids, speaker id, settings),
     where settings is a dict with any of "length_scale", "temperature", "n_timesteps" for that utterance (a missing key takes
     the keyword's value).  Utterances with different settings share micro-batches (MatchaTTS.synthesise with per-utterance
@@ -111,11 +147,19 @@ def synthesise_corpus(model, vocoder, utterances, batch_size=32, n_timesteps=10,
     whereas capturing costs ~250 ms per new shape (profiles/r02_host_cost.txt); True restores capture-on-second-sight.
     in_flight / lanes: micro-batches in flight at once (see `Lanes`; `lanes` passes a prebuilt set, else `lanes_for` builds and
     caches one); the waveforms do not depend on it.  stats.seconds is the sum of the micro-batches' device times for one
-    lane and the device span from the first launch to the last kernel's end for several."""
+    lane and the device span from the first launch to the last kernel's end for several.
+
+    seed: utterance i (its index in `utterances`) draws its prior noise on the GPU from output i of splitmix64(seed)
+    (MatchaTTS.synthesise(seed=...)); a "seed" in its settings overrides that value and does not change the plan.  The noise,
+    and so every waveform, is then the same for any rank / world_size split, in_flight, cuda_graphs and RNG history; without a
+    seed the noise comes from torch.randn as before.  The mel depends on the micro-batch (the decoder is not padding-invariant),
+    which the plan fixes independently of world_size.  Some utterances seeded and others not, or seeds with z_fn, are a
+    ValueError."""
     lens = [len(u[0]) for u in utterances]
     settings, own = utterance_settings(utterances, dict(length_scale=length_scale, temperature=temperature, n_timesteps=n_timesteps,
                                                         denoiser_strength=denoiser_strength if denoiser is not None else None))
     strengths = denoiser_strengths(settings, denoiser)
+    seeds = utterance_seeds(settings, seed, z_fn)
     steps = [int(s["n_timesteps"]) for s in settings] if own else n_timesteps
     plan = sharding.shard(lens, batch_size, rank, world_size, n_timesteps=steps, sort=sort)
     results, stats = {}, sharding.ShardStats()
@@ -166,6 +210,8 @@ def synthesise_corpus(model, vocoder, utterances, batch_size=32, n_timesteps=10,
                 kw = {}
                 if z_fn is not None:
                     kw["z"] = z_fn(mb, m, x, xl, spks)
+                if seeds is not None:
+                    kw["seed"] = [seeds[i] for i in mb.items]
                 if own:      # one value per utterance of the micro-batch
                     n_b, temp_b, ls_b = ([settings[i][k] for i in mb.items] for k in ("n_timesteps", "temperature", "length_scale"))
                 else:
@@ -222,7 +268,7 @@ def synthesise_corpus(model, vocoder, utterances, batch_size=32, n_timesteps=10,
 def synthesise_file(model, vocoder, script, out_dir, *, phonemizer=None, cleaner="english_cleaners2", spk=None, emoji_mapping=None,
                     default_spk: int = 12, batch_size: int = 32, n_timesteps: int = 10, temperature: float = 0.667,
                     length_scale: float = 1.0, denoiser=None, denoiser_strength: float = 0.00025, rank: int = 0,
-                    world_size: int = 1, in_flight: int = 1):
+                    world_size: int = 1, in_flight: int = 1, seed=None):
     """One call from a script file to audio on disk: the reference's batched file path composed end to end
     (`matcha/cli.py:226-250` get_texts / `:277-317` batched_synthesis / `:129-135` save_to_folder).
 
@@ -233,7 +279,8 @@ def synthesise_file(model, vocoder, script, out_dir, *, phonemizer=None, cleaner
     phonemizer : callable text -> phoneme string standing for espeak-ng (absent offline); the rule-based half of the cleaner
                  (`text_cleaners`) runs in front of it.  None: the line must already be a phoneme string of the symbol table.
     Writes `<out_dir>/utterance_{i:03d}_speaker_{spk:03d}.wav` (PCM_24, 22.05 kHz) + `.npy` (mel), i = line index, for the
-    lines this rank owns (`sharding.shard`); `in_flight` micro-batches at once (see `Lanes`).
+    lines this rank owns (`sharding.shard`); `in_flight` micro-batches at once (see `Lanes`).  seed: as synthesise_corpus, with
+    i the utterance's index among the script's non-empty lines, so every rank split writes the same files.
     -> (list of (index, wav_path, mel_length), ShardStats)"""
     from . import audio_io, text_cleaners, text_frontend
     from .emoji_frontend import emoji_to_spk
@@ -260,7 +307,7 @@ def synthesise_file(model, vocoder, script, out_dir, *, phonemizer=None, cleaner
         speakers.append(speaker)
     results, stats = synthesise_corpus(model, vocoder, utterances, batch_size=batch_size, n_timesteps=n_timesteps, temperature=temperature,
                                        length_scale=length_scale, rank=rank, world_size=world_size, denoiser=denoiser,
-                                       denoiser_strength=denoiser_strength, keep_mel=True, in_flight=in_flight)
+                                       denoiser_strength=denoiser_strength, keep_mel=True, in_flight=in_flight, seed=seed)
     written = []
     for i in sorted(results):
         name = f"utterance_{i:03d}_speaker_{speakers[i]:03d}"

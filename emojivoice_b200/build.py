@@ -18,7 +18,8 @@ OBJ = os.path.join(HERE, "build")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "libemojivoice_b200.so")
 SOURCES = ["api.cu", "weights.cu", "conv_simt.cu", "conv_tc.cu", "resblock_tc.cu", "elementwise.cu", "attention.cu", "attention_tc.cu", "attention_enc_tc.cu", "align.cu",
-           "matcha.cu", "hifigan.cu", "denoiser.cu", "mas.cu", "ragged.cu", "ff_tc.cu", "resnet_tc.cu", "train_forward.cu"]
+           "matcha.cu", "hifigan.cu", "denoiser.cu", "mas.cu", "ragged.cu", "ff_tc.cu", "resnet_tc.cu", "train_forward.cu",
+           "noise.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC",
               "-Xcompiler", "-fvisibility=hidden", "--expt-relaxed-constexpr"]
 

@@ -102,7 +102,7 @@ class MatchaTTS:
         return -(-int(length) // f) * f
 
     @torch.inference_mode()
-    def synthesise(self, x, x_lengths, n_timesteps, temperature=1.0, spks=None, length_scale=1.0, z=None, dtype=None):
+    def synthesise(self, x, x_lengths, n_timesteps, temperature=1.0, spks=None, length_scale=1.0, z=None, dtype=None, seed=None):
         """Same contract as matcha_tts.py:77-152.  Extras: `z` injects the prior noise (B, n_feats, T_pad) *before*
         temperature scaling (the reference draws it at flow_matching.py:51); `dtype` picks "fp32" | "bf16".
 
@@ -110,7 +110,15 @@ class MatchaTTS:
         value per utterance).  Utterance b of a batch with per-utterance values gets the durations, alignment and lengths of
         the batch called with length_scale[b], and the mel of the batch called with (n_timesteps[b], temperature[b]) at the
         same padded length T_pad (ev_encode_items / ev_decode_items in include/emojivoice_b200.h); per-utterance values that
-        are all equal are the call with that number."""
+        are all equal are the call with that number.
+
+        `seed` draws the prior noise on the GPU from a seed per utterance instead of torch.randn: a Python int (every
+        utterance; ints in [-2^63, 2^64) are taken mod 2^64), a (B,) sequence of ints or an int64 tensor (two's complement of
+        the uint64 seeds; never read back).  Utterance b's noise is then a function of (seed[b], feature, frame) only
+        (ev_prior_noise): it does not depend on B, T_pad, its row or the process's RNG state, and is returned in out["z"].
+        The mel still depends on the batch: the decoder is not padding-invariant (GroupNorm statistics and attention keys
+        cover T_pad), so a seeded utterance gets the same mel only in the same micro-batch.  None (the default) draws with
+        torch.randn as before; `z` and `seed` together are a ValueError."""
         if not self._loaded:
             raise RuntimeError("load_state_dict() / load_from_checkpoint() first")
         t0 = dt.datetime.now()
@@ -125,6 +133,9 @@ class MatchaTTS:
             temperature = per_item_setting(temperature, B, "temperature")
             length_scale = per_item_setting(length_scale, B, "length_scale")
             ls_items = isinstance(length_scale, tuple)
+            seeds = per_item_seed(seed, B)
+            if seeds is not None and z is not None:
+                raise ValueError("pass either `z` (the prior noise itself) or `seed` (to draw it), not both")
             if self.n_spks > 1:
                 if spks is None:
                     raise ValueError("multi-speaker model: `spks` (speaker / emoji ids) is required")
@@ -168,9 +179,10 @@ class MatchaTTS:
                 raise IndexError("index out of range in self: " + " and ".join(
                     n for bit, n in ((1, f"token id outside [0, {self.n_vocab})"), (2, f"speaker id outside [0, {self.n_spks})")) if bad_ids & bit))
             T_pad = self.fix_len_compatibility(y_max_length)
-            if z is None:
+            seeded = seeds is not None                                   # ev_prior_noise writes z inside the decode stage
+            if z is None and not seeded:
                 z = torch.randn(B, F, T_pad, device=dev)                 # flow_matching.py:51
-            else:
+            elif z is not None:
                 z = z.to(device=dev, dtype=torch.float32).contiguous()
                 if tuple(z.shape) != (B, F, T_pad):
                     raise ValueError(f"z must have shape {(B, F, T_pad)}, got {tuple(z.shape)}")
@@ -189,26 +201,36 @@ class MatchaTTS:
                 n_steps, temp = int(n_timesteps), float(temperature)
                 dec_key = (B, Tx, T_pad, n_steps, temp, prec)
                 dec_bytes = L.ev_decode_workspace_bytes(ctx.handle, B, T_pad, n_steps)
+            dec_out = {"attn": ((B, Tx, T_pad), f32), "mu_y": ((B, F, T_pad), f32), "y_mask": ((B, 1, T_pad), f32),
+                       "dec": ((B, F, T_pad), f32), "mel": ((B, F, T_pad), f32)}
+            if seeded:      # the seeds are a static device input of the graph, z one of its outputs
+                dec_in["seeds"] = seeds.to(dev)
+                dec_out["z"] = ((B, F, T_pad), f32)
+                dec_key += ("seeded",)
 
             def align_decode(i, o, ws):
+                if seeded:
+                    ctx.check(L.ev_prior_noise(ctx.handle, _lib.ptr(i["seeds"]), B, F, T_pad, _lib.ptr(o["z"]), _lib.stream_ptr()),
+                              "ev_prior_noise")
+                zp = _lib.ptr(o["z"] if seeded else i["z"])
                 ctx.check(L.ev_align(ctx.handle, _lib.ptr(i["w_ceil"]), _lib.ptr(i["x_lengths"]), _lib.ptr(i["y_lengths"]),
                                      _lib.ptr(i["mu_x"]), B, Tx, T_pad, _lib.ptr(o["attn"]), _lib.ptr(o["mu_y"]), _lib.ptr(o["y_mask"]),
                                      _lib.ptr(ws), ws.numel(), _lib.stream_ptr()), "ev_align")
                 if dec_items:
-                    ctx.check(L.ev_decode_items(ctx.handle, _lib.ptr(o["mu_y"]), _lib.ptr(i["y_lengths"]), _lib.ptr(i["z"]),
+                    ctx.check(L.ev_decode_items(ctx.handle, _lib.ptr(o["mu_y"]), _lib.ptr(i["y_lengths"]), zp,
                                                 _lib.ptr(i["spk_emb"]), B, T_pad, n_host, _lib.ptr(i["temperatures"]), prec,
                                                 _lib.ptr(o["dec"]), _lib.ptr(o["mel"]), _lib.ptr(ws), ws.numel(), _lib.stream_ptr()),
                               "ev_decode_items")
                     return
-                ctx.check(L.ev_decode(ctx.handle, _lib.ptr(o["mu_y"]), _lib.ptr(i["y_lengths"]), _lib.ptr(i["z"]), _lib.ptr(i["spk_emb"]),
+                ctx.check(L.ev_decode(ctx.handle, _lib.ptr(o["mu_y"]), _lib.ptr(i["y_lengths"]), zp, _lib.ptr(i["spk_emb"]),
                                       B, T_pad, n_steps, temp, prec, _lib.ptr(o["dec"]), _lib.ptr(o["mel"]), _lib.ptr(ws), ws.numel(),
                                       _lib.stream_ptr()), "ev_decode")
 
             nb = max(L.ev_align_workspace_bytes(ctx.handle, B, Tx, T_pad), dec_bytes)
-            d = self._run("decode", dec_key, nb, dec_in,
-                          {"attn": ((B, Tx, T_pad), f32), "mu_y": ((B, F, T_pad), f32), "y_mask": ((B, 1, T_pad), f32),
-                           "dec": ((B, F, T_pad), f32), "mel": ((B, F, T_pad), f32)}, align_decode)
+            d = self._run("decode", dec_key, nb, dec_in, dec_out, align_decode)
             attn, mu_y, y_mask, dec, mel = d["attn"], d["mu_y"], d["y_mask"], d["dec"], d["mel"]
+            if seeded:
+                z = d["z"]
         t = (dt.datetime.now() - t0).total_seconds()
         rtf = t * 22050 / (max(y_max_length, 1) * 256)                    # matcha_tts.py:142-143 (host clock, no sync)
         return {
@@ -369,6 +391,48 @@ def per_item_setting(value, B, name):
     else:
         vals = [float(v) for v in vals]
     return vals[0] if all(v == vals[0] for v in vals) else tuple(vals)
+
+
+_U64 = 1 << 64
+
+
+def seed_value(v, what="seed"):
+    """One noise seed as the uint64 it stands for: a Python (or numpy) int in [-2^63, 2^64), taken mod 2^64.  Bools and
+    non-integers are a ValueError."""
+    if isinstance(v, bool) or not isinstance(v, numbers.Integral):
+        raise ValueError(f"{what}: seeds must be integers, got {v!r}")
+    v = int(v)
+    if not -(1 << 63) <= v < _U64:
+        raise ValueError(f"{what}: seeds must lie in [-2^63, 2^64), got {v}")
+    return v % _U64
+
+
+def per_item_seed(seed, B):
+    """The noise seeds of a batch of B utterances: None, a number (every utterance), a (B,) sequence of ints or an integer
+    tensor with one seed per utterance.  -> None, or a (B,) int64 tensor holding the uint64 seeds in two's complement (on the
+    device of a tensor argument, else on the CPU).  An int64 tensor is taken as it is: every value is a valid seed, so it is
+    not read back."""
+    if seed is None:
+        return None
+    if torch.is_tensor(seed):
+        if seed.dtype == torch.int64:
+            if seed.dim() == 0:
+                return seed.reshape(1).expand(B).contiguous()
+            if seed.numel() != B:
+                raise ValueError(f"seed: expected a number or {B} seeds (one per utterance), got {seed.numel()}")
+            return seed.detach().reshape(B).contiguous()
+        if seed.dtype == torch.bool or seed.is_floating_point() or seed.is_complex():
+            raise ValueError(f"seed: seeds must be integers, got a {seed.dtype} tensor")
+        seed = seed.item() if seed.dim() == 0 else seed.detach().reshape(-1).tolist()
+    if isinstance(seed, numbers.Number):
+        vals = [seed_value(seed)] * B
+    else:
+        if isinstance(seed, (str, bytes)) or not hasattr(seed, "__iter__"):
+            raise ValueError(f"seed: seeds must be integers, got {seed!r}")
+        vals = [seed_value(v) for v in seed]
+        if len(vals) != B:
+            raise ValueError(f"seed: expected a number or {B} seeds (one per utterance), got {len(vals)}")
+    return torch.tensor([v - _U64 if v >= (1 << 63) else v for v in vals], dtype=torch.int64)
 
 
 class _CFMFacade:

@@ -142,6 +142,17 @@ EV_API int ev_decode_items(ev_ctx* ctx, const float* mu_y, const int64_t* y_leng
               int B, int T_pad, const int32_t* n_steps_host, const float* temperatures, int precision, float* decoder_out,
               float* mel, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- seeded prior noise ---------------------------------------------------------------------------------------
+ * The z of flow_matching.py:51 (randn_like(mu), before the temperature) as a function of a seed per utterance:
+ * seeds (B) device int64, read as uint64; z (B,n_feats,T) fp32.  Seed s keys Philox4x32-10 (Random123) with
+ * k = (s mod 2^32, s >> 32); feature f and frame group q = t >> 2 give (w0,w1,w2,w3) = Philox(counter = (q, f, 0, 0), k), and
+ *   u = (w0 + 0.5) 2^-32,  v = w1 2^-32,  z[f,4q] = sqrt(-2 ln u) cos(2 pi v),  z[f,4q+1] = sqrt(-2 ln u) sin(2 pi v),
+ * with (w2, w3) giving frames 4q+2 and 4q+3 the same way; float64 arithmetic rounded once to fp32, |z| <= 6.77, never inf or NaN.
+ * Row b depends on (seeds[b], f, t) only: not on B, T, the row's position or the other seeds, so frames [0, T) of a longer
+ * call are those of a shorter one, bit for bit.  Any T >= 1; no weights needed; one launch; no host synchronisation
+ * (capturable, a replay reads new seeds).  Null pointers or an empty shape: EV_ERR_INVALID. */
+EV_API int ev_prior_noise(ev_ctx* ctx, const int64_t* seeds, int B, int n_feats, int T, float* z, void* stream);
+
 /* ---- HiFi-GAN generator ----------------------------------------------------------------------------------
  * Replaces Generator.forward (hifigan/models.py:181-197) followed by the `.clamp(-1, 1)` of to_waveform
  * (feel_me.py:181-187; a no-op after tanh, kept for the contract).  mel (B,num_mels,T) -> wav (B,1,T*prod(rates)). */
