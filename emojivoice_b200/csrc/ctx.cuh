@@ -46,10 +46,9 @@ struct MatchaW {
   float *final_g = nullptr, *final_b = nullptr;
 };
 
-struct DenoiseBasis {          // windowed Fourier bases of the bias denoiser (denoiser.cu)
-  ConvWeights fwd, inv;
+struct DenoiseTables {         // tables of the bias denoiser's FFT (denoiser.cu)
   float* win_sq = nullptr;     // hann^2 [1024]
-  void* twiddle = nullptr;     // float2[1024] exp(-2 pi i n / 1024) for the FFT path
+  float2* twiddle = nullptr;   // [1024] exp(-2 pi i n / 1024)
   bool ready = false;
 };
 
@@ -65,7 +64,7 @@ struct HifiganW {
   float* post_b = nullptr;
   int c_last = 0, total_up = 1;
   float* denoise_bias = nullptr;  // (n_fft/2+1) once ev_denoiser_init ran
-  DenoiseBasis dn;
+  DenoiseTables dn;
 };
 
 }  // namespace ev

@@ -206,9 +206,8 @@ EV_API int ev_to_waveform_ragged(ev_ctx* ctx, const float* mel, const int64_t* m
  * Either way, on [0, lengths[b]*256) and ZERO beyond when lengths are given.  Strength 0 is not "not denoised": the STFT /
  * ISTFT round trip changes low bits.  A not-denoised item adds no STFT frames, and ev_to_waveform_items vocodes it on
  * mel_lengths[b] frames rather than mel_lengths[b] + 4.  Equal strengths with every item denoised are the scalar calls'
- * results, with other kernels; callers that hold equal values pass the number.  Strengths and flags stay on the device (no
- * host synchronisation, capturable; a finite strength is the caller's duty).  Other rules as the scalar calls.  The FFT
- * denoiser only: with EV_DN_FFT=0 (the GEMM cross-check path, one strength per call) these return EV_ERR_INVALID. */
+ * results; callers that hold equal values pass the number.  Strengths and flags stay on the device (no host
+ * synchronisation, capturable; a finite strength is the caller's duty).  Other rules as the scalar calls. */
 EV_API size_t ev_denoise_items_workspace_bytes(const ev_ctx* ctx, int B, int L);
 EV_API int ev_denoise_items(ev_ctx* ctx, const float* audio, const int64_t* lengths, int B, int L, const float* strengths,
               const uint8_t* denoise, float* out, void* workspace, size_t workspace_bytes, void* stream);

@@ -4,11 +4,7 @@ scalar call with its own strength gives it, or the vocoder's (Denoiser: its inpu
 
 CPU: argument parsing, the corpus settings and their refusals, the micro-batch plan.
 GPU: per-item calls against scalar calls and the oracle, launch counts, graph replay, device lengths, the work skipped, the
-corpus driver, the GEMM path's refusal, the C ABI's refusals."""
-import os
-import subprocess
-import sys
-
+corpus driver, the C ABI's refusals."""
 import pytest
 import torch
 
@@ -18,7 +14,6 @@ from emojivoice_b200.hifigan import per_item_strength
 from oracle import hifigan_oracle as ho
 
 HOP = 256
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 # ------------------------------------------------------------------------------------------------ CPU
@@ -317,41 +312,6 @@ def test_corpus_per_utterance_strengths(matcha_sd, gen_den, in_flight):
             assert got[i]["mel_length"] == refs[None][i]["mel_length"]
             assert torch.equal(got[i]["mel"], refs[None][i]["mel"]), i
             assert torch.equal(got[i]["waveform"], refs[s][i]["waveform"]), (i, s, ragged)
-
-
-_GEMM_PATH = """
-import sys
-sys.path.insert(0, {root!r})
-import torch
-import emojivoice_b200 as ev
-from emojivoice_b200 import synthetic
-from emojivoice_b200.config import HIFIGAN_V1
-g = ev.Generator(HIFIGAN_V1)
-g.load_state_dict(synthetic.hifigan_state_dict(HIFIGAN_V1, seed=4321, gain=1.0))
-g.remove_weight_norm()
-den = ev.Denoiser(g)
-mel = synthetic.synthetic_mel(2, 20, seed=1)
-wav = g(mel).clamp(-1, 1).squeeze(1)
-den(wav, 0.1)
-g.vocode_denoised(mel, [20, 7], 0.1)
-for call in (lambda: den(wav, [0.1, None]), lambda: g.vocode_denoised(mel, [20, 7], [0.1, None])):
-    try:
-        call()
-    except RuntimeError as e:
-        assert "FFT denoiser" in str(e), str(e)
-    else:
-        raise SystemExit("per-item strengths ran on the GEMM path")
-print("refused")
-"""
-
-
-@pytest.mark.gpu
-def test_gemm_path_refuses_per_item_strengths():
-    """EV_DN_FFT=0 (the GEMM cross-check path, one strength per call): the scalar calls run, the per-item calls are refused."""
-    env = dict(os.environ, EV_DN_FFT="0")
-    r = subprocess.run([sys.executable, "-c", _GEMM_PATH.format(root=ROOT)], env=env, cwd=ROOT, capture_output=True, text=True,
-                       timeout=600)
-    assert r.returncode == 0 and "refused" in r.stdout, r.stdout + r.stderr
 
 
 @pytest.mark.gpu
